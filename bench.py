@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: Mrays/s of the path-tracing hot path on BASELINE.json's million-triangle config.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload grid1m|bunny|cube] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload grid1m|bunny|cube] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -299,6 +299,24 @@ def parity_against_cpu_frame(drb, device, kind):
             "max_abs": float(np.abs(diff).max()), "rays_equal": bool(stats.rays == cpu_rays), "rays": int(stats.rays), "cpu_rays": int(cpu_rays)}
 
 
+DUMP_LIMIT_BYTES = 30 << 20          # per array; a dump holds at most two images, so it stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy.  An array larger than DUMP_LIMIT_BYTES is kept as every k-th row of its
+    flattening to (-1, last axis), i.e. every k-th pixel of an image in row-major order: the same pixels for the same
+    arguments, whichever build wrote them."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.nbytes > DUMP_LIMIT_BYTES:
+            a = a.reshape(-1, a.shape[-1])[::-(-a.nbytes // DUMP_LIMIT_BYTES)]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+        log("[bench] dumped %s %s %s to %s" % (name, a.dtype, a.shape, out_dir))
+
+
 def emit(line):
     """the ONE line on the real stdout"""
     os.write(REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -326,8 +344,15 @@ def main():
                     help="N > 1: shard sample indices (default) or interleaved 8x4-pixel tiles (bit-identical to the 1-GPU image)")
     ap.add_argument("--batch-paths", type=int, default=0, help="paths in flight per wavefront batch (0 = library default)")
     ap.add_argument("--spp", type=int, default=0, help="override samples per pixel (profiling runs only; invalidates the metric)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step of each timed loop computed as DIR/<name>.npy: "
+                         "resident_* for the scene-resident loop behind 'value', e2e_* for the host-buffer loop behind 'e2e' "
+                         "(--impl reference: the last CPU frame), so that two builds can be compared output for output (the "
+                         "inputs depend on the arguments only)")
     args = ap.parse_args()
-    K, W = max(args.steps, 1), max(args.warmup, 0)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    K, W = args.steps, args.warmup
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     objs, st, desc = workload(args.workload)
@@ -350,6 +375,9 @@ def main():
                 "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config,
                 "cpu_baseline": {"value": v, "unit": "Mrays/s", "cores": ncores, "kind": kind, "sample": sample},
                 "e2e": {"value": v, "unit": "Mrays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "rays_per_path": rpp, "gpu_launches": 0}
+        if args.dump_outputs:
+            # the last timed CPU frame (the reference's Kernel(), or its C restatement): 255 * mean radiance, indexed [x, y]
+            dump_outputs(args.dump_outputs, {"frame_255": LAST_CPU_FRAME["frame"], "rays": [float(LAST_CPU_FRAME["rays"])]})
         scene_file_cleanup()
         emit(line)
         return 0
@@ -415,6 +443,17 @@ def main():
     barrier()
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if clocks else None
+
+    def step_outputs(stats, img):
+        """what one step hands its caller: the radiance sums of the frame (rank 0, after the reduce) and the rays and
+        paths traced, summed over ranks"""
+        counts = torch.tensor([float(stats.rays), float(stats.paths)], device=dev, dtype=torch.float64)
+        if world > 1:
+            dist.all_reduce(counts)
+        return img.cpu().numpy() if rank == 0 else None, counts.cpu().numpy()
+
+    if args.dump_outputs:
+        resident_out = step_outputs(s, accum)          # the e2e steps below overwrite accum
     tot = torch.tensor([float(rays), float(paths), ms, trace_ms, float(launches), float(trace_launches)], device=dev, dtype=torch.float64)
     if world > 1:
         mx = tot.clone(); dist.all_reduce(mx, op=dist.ReduceOp.MAX)
@@ -482,9 +521,15 @@ def main():
         e2e_parts[k] = 0.0
     t_e = time.perf_counter(); e_rays = 0
     for _ in range(K):
-        e_rays += step_e2e().rays
+        last = step_e2e()
+        e_rays += last.rays
     barrier()
     e_ms = (time.perf_counter() - t_e) * 1e3
+    if args.dump_outputs:
+        e2e_out = step_outputs(last, host_img)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"resident_radiance_sum": resident_out[0], "resident_rays_paths": resident_out[1],
+                                             "e2e_radiance_sum": e2e_out[0], "e2e_rays_paths": e2e_out[1]})
     et = torch.tensor([float(e_rays), e_ms], device=dev, dtype=torch.float64)
     if world > 1:
         es = et.clone(); dist.all_reduce(es, op=dist.ReduceOp.SUM)

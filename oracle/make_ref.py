@@ -27,8 +27,9 @@ writes only binaries (and staged sample DATA files) into the git-ignored
     temporary file outside the repo for the duration of the compile; this build is never the one that is timed.
 
 ``samples/``
-    The reference's sample scenes and textures (DATA, not source), staged so the GPU
-    box (which has no /root/reference) can render the same inputs.
+    The reference's sample scenes and textures (DATA, not source), staged so that a
+    machine without a checkout of the reference can render the same inputs.  Beside them,
+    ``bolter2.blend.rts.bmp``: one of the reference's screenshots (SDL_SaveBMP output).
 
 Run:  python oracle/make_ref.py [--reference /root/reference] [--no-gpu]
 """
@@ -118,6 +119,10 @@ def stage_samples(ref_root):
     extra = os.path.join(ref_root, "raygpu", "scene.rts")
     if os.path.exists(extra):
         shutil.copyfile(extra, os.path.join(dst, "_raygpu_scene.rts"))
+        n += 1
+    shot = os.path.join(ref_root, "images", "bolter2.blend.rts.bmp")      # the BMP writer's byte-for-byte fixture
+    if os.path.exists(shot):
+        shutil.copyfile(shot, os.path.join(OUT, "bolter2.blend.rts.bmp"))
         n += 1
     return n
 

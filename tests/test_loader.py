@@ -258,10 +258,13 @@ def test_bmp_header_equals_the_reference_screenshots_byte_for_byte(tmp_path):
     assert (1280, 720) in done and len(done) >= 3
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/images"), reason="the reference's screenshots are not on this machine")
+SCREENSHOT = os.path.join(os.path.dirname(SAMPLES), "bolter2.blend.rts.bmp")
+
+
+@pytest.mark.skipif(not os.path.exists(SCREENSHOT), reason="the reference's screenshot is staged into oracle/_ref by oracle/make_ref.py")
 def test_bmp_writer_reproduces_a_reference_screenshot_file(tmp_path):
     """decode images/bolter2.blend.rts.bmp to top-down RGB and write it back: the file must come out byte-identical"""
-    ref = open("/root/reference/images/bolter2.blend.rts.bmp", "rb").read()
+    ref = open(SCREENSHOT, "rb").read()
     w, h = struct.unpack_from("<ii", ref, 18)
     px = np.frombuffer(ref[122:], np.uint8).reshape(h, w, 4)[::-1]            # bottom-up rows, B G R A
     rgb = np.ascontiguousarray(px[..., [2, 1, 0]])
