@@ -235,12 +235,11 @@ constexpr int kSentinel = (int)0x80000000;     // bottom of every traversal stac
 #define DRB_TRACE_MIN_BLOCKS 8
 #endif
 template <bool kSortedPush>
-__global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(DevScene sc, float scene_scale, Queues q, int cur, int refill, int leaf_batch, int step_min,
+__global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(DevScene sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
+                                               uint2* __restrict__ hit, uint32_t* counters, int cur, int refill, int leaf_batch, int step_min,
                                                const uint32_t* __restrict__ order)
 {
-    const uint32_t count = q.counters[cur];
-    const float4* __restrict__ ro = q.ray_o[cur];
-    const float4* __restrict__ rdv = q.ray_d[cur];
+    const uint32_t count = counters[cur];
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
 
@@ -249,8 +248,9 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
     uint32_t ray = 0xFFFFFFFFu;
     bool exhausted = false;                         // warp-uniform: the queue has been handed out completely
     f3 o = mk3(0.f), d = mk3(0.f);
-    // per-ray plane constants: t = fma(2^23 + q, s*, c*), near / far plane picked by the PRMT selectors
-    float sx = 0.f, sy = 0.f, sz = 0.f, cnx = 0.f, cny = 0.f, cnz = 0.f, cfx = 0.f, cfy = 0.f, cfz = 0.f;
+    // per-ray plane constants, per axis as (near, far) pairs: (t_near, t_far) = (2^23 + q_near, 2^23 + q_far) * (s, s) + (c_near, c_far),
+    // near / far plane picked by the PRMT selectors
+    float2 sxx = {}, syy = {}, szz = {}, cxx = {}, cyy = {}, czz = {};
     uint32_t snx = 0x7410u, sny = 0x7410u, snz = 0x7410u, sfx = 0x7432u, sfy = 0x7432u, sfz = 0x7432u;   // PRMT selectors of the near / far plane
     float best = kTMax; int bestp = -1;
     // traversal stack in dynamic shared memory, [level][thread], sized by the host to the tree height + 2: every
@@ -269,7 +269,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
         if (!exhausted && (midle == 0xffffffffu || 32 - __popc(midle) < refill)) {
             const int leader = __ffs(midle) - 1;
             uint32_t base = 0;
-            if ((int)lane == leader) base = atomicAdd(&q.counters[CNT_TICKET], (uint32_t)__popc(midle));
+            if ((int)lane == leader) base = atomicAdd(&counters[CNT_TICKET], (uint32_t)__popc(midle));
             base = __shfl_sync(0xffffffffu, base, leader);
             if (base + (uint32_t)__popc(midle) >= count) exhausted = true;
             if (idle) {
@@ -278,7 +278,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
                     const uint32_t i = order ? order[k] : k;        // queue position of the k-th ray in traversal order
                     const float4 o4 = ro[i], d4 = rdv[i];
                     if (__float_as_uint(o4.w) == kInvalidPid || sc.nprims == 0) {
-                        q.hit[i] = make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
+                        hit[i] = make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
                     } else {
                         ray = i;
                         o = xyz(o4); d = xyz(d4);
@@ -293,11 +293,12 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
                         // plane coordinate = qlo + q * qscale; t = (coordinate -/+ pad - o) * inv, folded into one FMA on
                         // the float 2^23 + q: t = (2^23 + q) * s + (c - 2^23 * s).  The near plane is the min plane for a
                         // positive direction component and the max plane for a negative one.
-                        sx = sc.qscale[0] * ix; sy = sc.qscale[1] * iy; sz = sc.qscale[2] * iz;
+                        const float sx = sc.qscale[0] * ix, sy = sc.qscale[1] * iy, sz = sc.qscale[2] * iz;
                         const float px = copysignf(pad, ix), py = copysignf(pad, iy), pz = copysignf(pad, iz);
-                        cnx = fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x - px) * ix); cfx = fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x + px) * ix);
-                        cny = fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y - py) * iy); cfy = fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y + py) * iy);
-                        cnz = fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z - pz) * iz); cfz = fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z + pz) * iz);
+                        sxx = make_float2(sx, sx); syy = make_float2(sy, sy); szz = make_float2(sz, sz);
+                        cxx = make_float2(fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x - px) * ix), fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x + px) * ix));
+                        cyy = make_float2(fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y - py) * iy), fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y + py) * iy));
+                        czz = make_float2(fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z - pz) * iz), fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z + pz) * iz));
                         snx = ix >= 0.f ? 0x7410u : 0x7432u; sny = iy >= 0.f ? 0x7410u : 0x7432u; snz = iz >= 0.f ? 0x7410u : 0x7432u;
                         sfx = snx ^ 0x22u; sfy = sny ^ 0x22u; sfz = snz ^ 0x22u;
                         best = kTMax; bestp = -1;
@@ -313,17 +314,21 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
         if (node >= 0) {
             const WideNode* np = sc.wnodes + node;
             const f8 nA = ldg256(np->bx), nB = ldg256(np->bz);          // the whole node: two 256-bit loads
-#define DRB_PLANE(w, sel, s_, c_) fmaf(prmt_exp23(__float_as_uint(w), (sel)), (s_), (c_))
+            // (near, far) distance of one axis: both planes come from the same word and share the scale, so they go through
+            // one packed FFMA2.  Each half is one IEEE fma rounded like fmaf.  (Only explicit fmas are packed: ptxas contracts
+            // a packed mul followed by a packed add into FFMA2 even under -fmad=false.)
+#define DRB_PLANES(w, sn, sf, s_, c_) __ffma2_rn(make_float2(prmt_exp23(__float_as_uint(w), (sn)), prmt_exp23(__float_as_uint(w), (sf))), (s_), (c_))
 #define DRB_CHILD(c, wx, wy, wz)                                                                                              \
-            const float tn##c = fmaxf(fmaxf(DRB_PLANE(wx, snx, sx, cnx), DRB_PLANE(wy, sny, sy, cny)), fmaxf(DRB_PLANE(wz, snz, sz, cnz), 0.0f)); \
-            const float tf##c = fminf(fminf(DRB_PLANE(wx, sfx, sx, cfx), DRB_PLANE(wy, sfy, sy, cfy)), fminf(DRB_PLANE(wz, sfz, sz, cfz), best)); \
+            const float2 x##c = DRB_PLANES(wx, snx, sfx, sxx, cxx), y##c = DRB_PLANES(wy, sny, sfy, syy, cyy), z##c = DRB_PLANES(wz, snz, sfz, szz, czz); \
+            const float tn##c = fmaxf(fmaxf(x##c.x, y##c.x), fmaxf(z##c.x, 0.0f));                                            \
+            const float tf##c = fminf(fminf(x##c.y, y##c.y), fminf(z##c.y, best));                                            \
             const uint32_t k##c = (tn##c <= tf##c) ? ((__float_as_uint(tn##c) & 0xFFFFFFFCu) | c##u) : 0xFFFFFFFFu;
             DRB_CHILD(0, nA.lo.x, nA.hi.x, nB.lo.x)
             DRB_CHILD(1, nA.lo.y, nA.hi.y, nB.lo.y)
             DRB_CHILD(2, nA.lo.z, nA.hi.z, nB.lo.z)
             DRB_CHILD(3, nA.lo.w, nA.hi.w, nB.lo.w)
 #undef DRB_CHILD
-#undef DRB_PLANE
+#undef DRB_PLANES
             // t_near >= 0, so its bits order like unsigned integers; the two low bits carry the slot
             if constexpr (kSortedPush) {
             // sort the four keys (5 compare-exchanges), push the hits far-to-near, continue with the nearest
@@ -333,7 +338,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
             if (s0 == 0xFFFFFFFFu) node = DRB_POP();
             else {
                 const int c0 = __float_as_int(nB.hi.x), c1 = __float_as_int(nB.hi.y), c2 = __float_as_int(nB.hi.z), c3 = __float_as_int(nB.hi.w);
-#define DRB_LINK(k) (((k) & 3u) == 0u ? c0 : (((k) & 3u) == 1u ? c1 : (((k) & 3u) == 2u ? c2 : c3)))
+#define DRB_LINK(k) (((k) & 2u) ? (((k) & 1u) ? c3 : c2) : (((k) & 1u) ? c1 : c0))
                 if (s3 != 0xFFFFFFFFu) DRB_PUSH(DRB_LINK(s3));
                 if (s2 != 0xFFFFFFFFu) DRB_PUSH(DRB_LINK(s2));
                 if (s1 != 0xFFFFFFFFu) DRB_PUSH(DRB_LINK(s1));
@@ -349,8 +354,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
                 if (k2 != kmin && k2 != 0xFFFFFFFFu) DRB_PUSH(c2);
                 if (k1 != kmin && k1 != 0xFFFFFFFFu) DRB_PUSH(c1);
                 if (k0 != kmin && k0 != 0xFFFFFFFFu) DRB_PUSH(c0);
-                const uint32_t near = kmin & 3u;
-                node = near == 0u ? c0 : (near == 1u ? c1 : (near == 2u ? c2 : c3));
+                node = (kmin & 2u) ? ((kmin & 1u) ? c3 : c2) : ((kmin & 1u) ? c1 : c0);
             }
             }
         }
@@ -369,7 +373,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
         }
         // ---- retire -----------------------------------------------------------------------------------
         if (node == kSentinel && leaf == 0 && ray != 0xFFFFFFFFu) {
-            q.hit[ray] = bestp >= 0 ? make_uint2(__float_as_uint(best), (uint32_t)bestp) : make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
+            hit[ray] = bestp >= 0 ? make_uint2(__float_as_uint(best), (uint32_t)bestp) : make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
             ray = 0xFFFFFFFFu;
         }
     }
@@ -467,22 +471,25 @@ enum { MODE_DEAD = 0, MODE_FINAL = 1, MODE_DIFFUSE = 2, MODE_DIFFUSE_UNIT = 3, M
 #ifndef DRB_SHADE_MIN_BLOCKS
 #define DRB_SHADE_MIN_BLOCKS 8
 #endif
-__global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc, FrameParams fp, Queues q, int cur, int last_bounce)
+__global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc, FrameParams fp, const float4* __restrict__ ro, const float4* __restrict__ rdv,
+                                                                           const float4* __restrict__ thr, const uint2* __restrict__ hit,
+                                                                           float4* __restrict__ ro_next, float4* __restrict__ rdv_next,
+                                                                           float4* __restrict__ thr_next, float4* __restrict__ contrib,
+                                                                           uint32_t* counters, int cur, int last_bounce)
 {
     __shared__ float s_rec[4][REC_WORDS][kShadeRays];           // [warp][field][slot]: conflict-free for slot = lane + 32 g
     __shared__ uint8_t s_req[4][kShadeRays];                    // slots that wait for a unit-sphere sample, in ray order
-    const uint32_t count = q.counters[cur];
-    const int nxt = cur ^ 1;
+    const uint32_t count = counters[cur];
     const unsigned lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const unsigned lt_mask = (1u << lane) - 1u;
     float (*rec)[kShadeRays] = s_rec[warp];
     uint8_t* req = s_req[warp];
-    uint64_t local_rays = 0;
+    uint32_t local_rays = 0;                                    // a warp shades rays of one queue (< 2^32): 32 bits hold its sum
     for (;;) {
         // the next kShadeRays rays of the queue: a ticket rather than a grid stride, so that warps whose groups are cheap
         // (all misses, no sampling) simply take more of them (frame 412 -> 404 ms)
         uint32_t base = 0;
-        if (lane == 0) base = atomicAdd(&q.counters[CNT_SHADE_TICKET], (uint32_t)kShadeRays);
+        if (lane == 0) base = atomicAdd(&counters[CNT_SHADE_TICKET], (uint32_t)kShadeRays);
         base = __shfl_sync(0xffffffffu, base, 0);
         if (base >= count) break;
         // ---- stage 1 ----------------------------------------------------------------------------------------------------
@@ -493,20 +500,20 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
             const int slot = g * 32 + (int)lane;
             int mode = MODE_DEAD;
             if (i < count) {
-                const float4 o4 = q.ray_o[cur][i];
+                const float4 o4 = __ldg(&ro[i]);
                 const uint32_t pid = __float_as_uint(o4.w);
                 if (pid != kInvalidPid) {
                     local_rays++;
-                    const float4 d4 = q.ray_d[cur][i];
-                    const float4 a4 = q.thr[cur][i];
-                    const uint2 h = q.hit[i];
+                    const float4 d4 = __ldg(&rdv[i]);
+                    const float4 a4 = __ldg(&thr[i]);
+                    const uint2 h = __ldg(&hit[i]);
                     const f3 rayo = xyz(o4), raydir = xyz(d4);
                     f3 atten = xyz(a4);
                     const float t = __uint_as_float(h.x);
                     const int prim = (int)h.y;
                     if (!(prim >= 0 && t > 0.0f)) {
                         const f3 c = atten * environment(sc, fp, raydir) * mk3(fp.bg_intensity);
-                        q.contrib[pid] = make_float4(c.x, c.y, c.z, 0.f);
+                        contrib[pid] = make_float4(c.x, c.y, c.z, 0.f);
                     } else {
                         const ShadeRec* srec = sc.recs + prim;
                         const float4 r0 = __ldg(&srec->r[0]), r1 = __ldg(&srec->r[1]), r2 = __ldg(&srec->r[2]);
@@ -561,9 +568,9 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
                         }
                         if (!(mat == 0 || mat == 2 || mat == 3 || mat == 4 || mat == 5)) {
                             const f3 c = ocolor * atten;                            // emissive, kernel.cu:941-944
-                            q.contrib[pid] = make_float4(c.x, c.y, c.z, 0.f);
+                            contrib[pid] = make_float4(c.x, c.y, c.z, 0.f);
                         } else if (last_bounce) {
-                            q.contrib[pid] = make_float4(0.f, 0.f, 0.f, 0.f);       // depth exhausted: black (kernel.cu:981), nothing to scatter
+                            contrib[pid] = make_float4(0.f, 0.f, 0.f, 0.f);       // depth exhausted: black (kernel.cu:981), nothing to scatter
                         } else {
                             uint32_t draws = __float_as_uint(d4.w);
                             f3 vec;                                                 // successor direction (FINAL), normal (diffuse lobe) or mirror direction (metal lobe)
@@ -713,7 +720,7 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
         }
         // ---- stage 3: finish and append in ray order ---------------------------------------------------------------------------
         uint32_t dst0 = 0;
-        if (lane == 0) dst0 = atomicAdd(&q.counters[nxt], (uint32_t)nalive);
+        if (lane == 0) dst0 = atomicAdd(&counters[cur ^ 1], (uint32_t)nalive);
         dst0 = __shfl_sync(0xffffffffu, dst0, 0);
 #pragma unroll 1
         for (int g = 0; g < kShadeGroups; ++g) {
@@ -734,9 +741,9 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
                     }
                 }
                 const uint32_t dst = dst0 + (uint32_t)__popc(malive & lt_mask);
-                q.ray_o[nxt][dst] = make_float4(hp.x, hp.y, hp.z, rec[REC_PID][slot]);
-                q.ray_d[nxt][dst] = make_float4(ndir.x, ndir.y, ndir.z, rec[REC_DRAWS][slot]);
-                q.thr[nxt][dst] = make_float4(rec[REC_AR][slot], rec[REC_AG][slot], rec[REC_AB][slot], rec[REC_XY][slot]);
+                ro_next[dst] = make_float4(hp.x, hp.y, hp.z, rec[REC_PID][slot]);
+                rdv_next[dst] = make_float4(ndir.x, ndir.y, ndir.z, rec[REC_DRAWS][slot]);
+                thr_next[dst] = make_float4(rec[REC_AR][slot], rec[REC_AG][slot], rec[REC_AB][slot], rec[REC_XY][slot]);
             }
             dst0 += (uint32_t)__popc(malive);
         }
@@ -745,7 +752,7 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
     // ray statistics: one 64-bit atomic per warp
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) local_rays += __shfl_xor_sync(0xffffffffu, local_rays, off);
-    if (lane == 0 && local_rays) atomicAdd(reinterpret_cast<unsigned long long*>(&q.counters[CNT_RAYS]), (unsigned long long)local_rays);
+    if (lane == 0 && local_rays) atomicAdd(reinterpret_cast<unsigned long long*>(&counters[CNT_RAYS]), (unsigned long long)local_rays);
 }
 
 // Sort key of a queued ray: direction octant (3 bits) above the 21-bit Morton code of the origin's cell in a
@@ -1047,10 +1054,9 @@ int g_step_min = []() { const char* e = getenv("DOGERAY_B200_STEP_MIN"); int v =
 // the closest-hit kernel for this scene: large scenes push the other hit children far-to-near (see DRB_SORTED_PUSH_FROM)
 void launch_trace(const drb_scene* s, const RenderBuffers* rb, cudaStream_t stream, const DevScene& sc, float scale, const Queues& q, int cur, const uint32_t* order)
 {
-    if (s->nprims >= (int64_t)DRB_SORTED_PUSH_FROM)
-        k_trace<true><<<rb->trace_blocks, kTraceThreads, rb->trace_smem, stream>>>(sc, scale, q, cur, g_refill, g_leaf_batch, g_step_min, order);
-    else
-        k_trace<false><<<rb->trace_blocks, kTraceThreads, rb->trace_smem, stream>>>(sc, scale, q, cur, g_refill, g_leaf_batch, g_step_min, order);
+    auto kernel = s->nprims >= (int64_t)DRB_SORTED_PUSH_FROM ? k_trace<true> : k_trace<false>;
+    kernel<<<rb->trace_blocks, kTraceThreads, rb->trace_smem, stream>>>(sc, scale, q.ray_o[cur], q.ray_d[cur], q.hit, q.counters, cur,
+                                                                      g_refill, g_leaf_batch, g_step_min, order);
 }
 
 
@@ -1190,7 +1196,9 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
             if (stats) { auto e0 = pool.get(), e1 = pool.get(); trace_ev.push_back({ e0, e1 }); DRB_CUDA(cudaEventRecord(e0, stream)); }
             launch_trace(s, rb, stream, sc, fp.scene_scale, q, cur, order);
             if (stats) DRB_CUDA(cudaEventRecord(trace_ev.back().second, stream));
-            k_shade<<<std::min<uint32_t>((uint32_t)rb->shade_blocks, (live + 4u * kShadeRays - 1u) / (4u * kShadeRays)), 128, 0, stream>>>(sc, fp, q, cur, b == st->max_depth - 1 ? 1 : 0);
+            k_shade<<<std::min<uint32_t>((uint32_t)rb->shade_blocks, (live + 4u * kShadeRays - 1u) / (4u * kShadeRays)), 128, 0, stream>>>(
+                sc, fp, q.ray_o[cur], q.ray_d[cur], q.thr[cur], q.hit, q.ray_o[cur ^ 1], q.ray_d[cur ^ 1], q.thr[cur ^ 1], q.contrib, q.counters, cur,
+                b == st->max_depth - 1 ? 1 : 0);
             k_prepare<<<1, 32, 0, stream>>>(q.counters, cur, -1, 0u);
             launches += 3; trace_launches += 1;
             cur ^= 1;
