@@ -154,6 +154,8 @@ _sig("drb_render_multi_times", _i, C.POINTER(C.c_float), _i)
 _sig("drb_scene_create_multi", _i, _vp, C.POINTER(C.c_int), _i, _u32, C.POINTER(C.c_void_p))
 _sig("drb_frame_i3", _i, _vp, C.POINTER(Settings), C.POINTER(Opts), _i, _vp)
 _sig("drb_trace_ids", _i, _vp, _vp, _vp, _i64, _vp, _vp)
+_sig("drb_trace_device", _i, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp)
+_sig("drb_occluded_device", _i, _vp, _vp, _vp, _vp, _i64, _vp, _vp)
 _sig("drb_primary_rays", _i, _vp, C.POINTER(Settings), C.POINTER(Opts), _u32, _vp, _vp)
 _sig("drb_tonemap", _i, _vp, _i, _i, C.c_double, _vp)
 _sig("drb_tonemap_device", _i, _vp, _i, _i, C.c_double, _vp, _vp)
@@ -176,7 +178,7 @@ EXPORTED_SYMBOLS = [
     "drb_rts_write", "drb_settings_default", "drb_scene_create", "drb_scene_create_ex", "drb_scene_tree", "drb_scene_wide", "drb_scene_load", "drb_scene_free",
     "drb_scene_settings", "drb_scene_num_prims", "drb_scene_num_objects", "drb_scene_build_info",
     "drb_scene_lbvh", "drb_opts_default", "drb_render_device", "drb_render", "drb_render_multi", "drb_frame_i3",
-    "drb_trace_ids", "drb_primary_rays", "drb_tonemap", "drb_tonemap_device", "drb_write_bmp",
+    "drb_trace_ids", "drb_trace_device", "drb_occluded_device", "drb_primary_rays", "drb_tonemap", "drb_tonemap_device", "drb_write_bmp",
     "drb_write_ppm", "drb_read_ppm", "drb_free", "drb_last_error", "drb_abi_version",
     "drb_device_count", "drb_trim", "drb_philox_word",
 ]
@@ -193,6 +195,22 @@ def _check(rc: int):
 
 def _b(s: Optional[str]):
     return None if s is None else os.fsencode(s)
+
+
+def _stream_handle(stream: Optional[int]):
+    """None -> the scene's own (non-blocking) stream.  0 is how torch names the legacy default stream
+    (torch.cuda.current_stream().cuda_stream outside a stream context); the C ABI reads a NULL stream as "the scene's own",
+    so the legacy default stream travels as its CUDA handle cudaStreamLegacy (0x1)."""
+    return None if stream is None else (1 if stream == 0 else stream)
+
+
+def _record(stream, *tensors):
+    """keeps tensors that work on `stream` reads or writes alive until it is done when they belong to another stream"""
+    import torch
+    if stream != torch.cuda.current_stream(stream.device):
+        for x in tensors:
+            if x is not None:
+                x.record_stream(stream)
 
 
 def default_settings() -> Settings:
@@ -240,7 +258,7 @@ def create_multi(hs: "HostScene", devices: Sequence[int], build_flags: int = 0) 
     devs = (C.c_int * len(devices))(*devices)
     out = (C.c_void_p * len(devices))()
     _check(_lib.drb_scene_create_multi(hs.handle, devs, len(devices), build_flags, out))
-    return [Scene(C.c_void_p(out[k])) for k in range(len(devices))]
+    return [Scene(C.c_void_p(out[k]), devices[k]) for k in range(len(devices))]
 
 
 def hash_bytes(data: bytes) -> int:
@@ -366,30 +384,29 @@ def make_objects(n: int) -> np.ndarray:
 class Scene:
     """Device-resident scene: textures uploaded, LBVH built on the GPU, everything kept in HBM."""
 
-    def __init__(self, handle):
+    def __init__(self, handle, device: int = 0):
         self._h = handle
+        self.device = device                         # the CUDA device the scene lives on
 
     @classmethod
     def load(cls, rts_path: str, tex_dir: Optional[str] = None, device: int = 0) -> "Scene":
         h = C.c_void_p()
         _check(_lib.drb_scene_load(_b(rts_path), _b(tex_dir), device, C.byref(h)))
-        return cls(h)
+        return cls(h, device)
 
     @classmethod
     def from_host(cls, hs: HostScene, device: int = 0, build_flags: int = 0) -> "Scene":
         h = C.c_void_p()
         _check(_lib.drb_scene_create_ex(hs.handle, device, build_flags, C.byref(h)))
-        return cls(h)
+        return cls(h, device)
 
     @classmethod
     def from_device_objects(cls, hs: HostScene, objects_ptr: int, device: int = 0, build_flags: int = 0, stream: Optional[int] = None) -> "Scene":
         """The object lines are already in device memory (hs.num_objects records of OBJECT_DTYPE at `objects_ptr`, e.g.
         all-gathered over NVLink from per-rank partial uploads); `stream` is the stream that produced them."""
         h = C.c_void_p()
-        if stream == 0:
-            stream = 1                                # cudaStreamLegacy, see Scene._opts
-        _check(_lib.drb_scene_create_from_device(hs.handle, device, build_flags, objects_ptr, stream, C.byref(h)))
-        return cls(h)
+        _check(_lib.drb_scene_create_from_device(hs.handle, device, build_flags, objects_ptr, _stream_handle(stream), C.byref(h)))
+        return cls(h, device)
 
     def close(self):
         if self._h and _lib is not None:             # _lib is None while the interpreter shuts down
@@ -457,10 +474,7 @@ class Scene:
         if sample_count is not None:
             flags |= FLAG_EXACT_SAMPLES
         o.seed, o.sample_base, o.sample_count, o.batch_paths, o.flags = seed, sample_base, int(sample_count or 0), batch_paths, flags
-        # None -> the scene's own (non-blocking) stream.  0 is how torch names the legacy default stream
-        # (torch.cuda.current_stream().cuda_stream outside a stream context); the C ABI reads a NULL stream as "the scene's
-        # own", so the legacy default stream travels as its CUDA handle cudaStreamLegacy (0x1).
-        o.stream = None if stream is None else (1 if stream == 0 else stream)
+        o.stream = _stream_handle(stream)
         o.tile_rank, o.tile_count = tile_rank, tile_count
         return o
 
@@ -508,6 +522,64 @@ class Scene:
         ids = np.empty(len(o), np.int32); t = np.empty(len(o), np.float32)
         _check(_lib.drb_trace_ids(self._h, o.ctypes.data, d.ctypes.data, len(o), ids.ctypes.data, t.ctypes.data))
         return ids, t
+
+    def trace_device(self, o_ptr: int, d_ptr: int, n: int, ids_ptr: int, t_ptr: Optional[int] = None, uv_ptr: Optional[int] = None,
+                     stream: Optional[int] = None):
+        """Closest hit for n rays in DEVICE arrays (n*3 float32 each): ids int32 (-1 = miss), optionally t float32 (-1 on a miss)
+        and (u, v) float32 pairs of the hit triangle.  Enqueued on `stream` (a raw handle; None -> the scene's own), asynchronous."""
+        _check(_lib.drb_trace_device(self._h, o_ptr, d_ptr, n, ids_ptr, t_ptr, uv_ptr, _stream_handle(stream)))
+
+    def occluded_device(self, o_ptr: int, d_ptr: int, n: int, out_ptr: int, tmax_ptr: Optional[int] = None, stream: Optional[int] = None):
+        """Any hit below tmax (n float32 in device memory; None -> 10000) for n rays in DEVICE arrays: n bytes 0 / 1 at
+        `out_ptr`.  Enqueued on `stream` (a raw handle; None -> the scene's own), asynchronous."""
+        _check(_lib.drb_occluded_device(self._h, o_ptr, d_ptr, tmax_ptr, n, out_ptr, _stream_handle(stream)))
+
+    def _query_args(self, stream, *tensors):
+        """(torch, stream, contiguous inputs): float32 CUDA tensors on the scene's device, the stream defaulting to the
+        caller's current torch stream"""
+        import torch
+        dev = torch.device("cuda", self.device)
+        out = []
+        for x in tensors:
+            if not isinstance(x, torch.Tensor):
+                raise ValueError("ray queries take torch tensors, got %s" % type(x).__name__)
+            if x.dtype != torch.float32 or x.device != dev:
+                raise ValueError("ray queries take float32 tensors on %s, got %s on %s" % (dev, x.dtype, x.device))
+            out.append(x.contiguous())
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        return torch, stream, out
+
+    def trace(self, origins, dirs, *, with_uv: bool = True, stream=None):
+        """Closest hit for torch rays: origins and dirs float32 (..., 3) on the scene's device.  Returns (ids int32 (...),
+        t float32 (...), uv float32 (..., 2) or None), allocated on that device and enqueued on `stream` (a torch.cuda.Stream,
+        default the current one) without synchronising."""
+        torch, stream, (o, d) = self._query_args(stream, origins, dirs)
+        if o.shape != d.shape or o.shape[-1:] != (3,):
+            raise ValueError("origins and dirs must have the same shape (..., 3), got %s and %s" % (tuple(o.shape), tuple(d.shape)))
+        lead = o.shape[:-1]
+        ids = torch.empty(lead, dtype=torch.int32, device=o.device)
+        t = torch.empty(lead, dtype=torch.float32, device=o.device)
+        uv = torch.empty(lead + (2,), dtype=torch.float32, device=o.device) if with_uv else None
+        self.trace_device(o.data_ptr(), d.data_ptr(), o.numel() // 3, ids.data_ptr(), t.data_ptr(), uv.data_ptr() if with_uv else None,
+                          stream.cuda_stream)
+        _record(stream, o, d, ids, t, uv)
+        return ids, t, uv
+
+    def occluded(self, origins, dirs, tmax=None, *, stream=None):
+        """Any hit at t < tmax for torch rays: origins and dirs float32 (..., 3), tmax float32 (...) or None (10000), all on
+        the scene's device.  Returns bool (...), enqueued on `stream` (a torch.cuda.Stream, default the current one) without
+        synchronising."""
+        torch, stream, xs = self._query_args(stream, origins, dirs, *(() if tmax is None else (tmax,)))
+        o, d = xs[0], xs[1]
+        tm = xs[2] if tmax is not None else None
+        if o.shape != d.shape or o.shape[-1:] != (3,) or (tm is not None and tm.shape != o.shape[:-1]):
+            raise ValueError("origins and dirs must have the same shape (..., 3) and tmax their leading shape")
+        out = torch.empty(o.shape[:-1], dtype=torch.bool, device=o.device)
+        self.occluded_device(o.data_ptr(), d.data_ptr(), o.numel() // 3, out.data_ptr(), tm.data_ptr() if tm is not None else None,
+                             stream.cuda_stream)
+        _record(stream, o, d, tm, out)
+        return out
 
     def primary_rays(self, settings: Optional[Settings] = None, sample: int = 0, seed: int = 0) -> Tuple[np.ndarray, np.ndarray]:
         """Camera rays of one sample index, (H, W, 3) each: kernel.cu:1067-1076."""

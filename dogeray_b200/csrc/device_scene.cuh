@@ -122,6 +122,8 @@ struct drb_scene {
     cudaStream_t stream = nullptr;
     // render work buffers, grown on demand (render.cu)
     struct RenderBuffers* rb = nullptr;
+    // ray-query scratch, separate from the render's queues (render.cu)
+    struct QueryBuffers* qb = nullptr;
 };
 
 #define DRB_CUDA(call)                                                                                     \
@@ -134,6 +136,7 @@ struct drb_scene {
     } while (0)
 
 void drb_render_buffers_free(drb_scene* s);
+void drb_query_buffers_free(drb_scene* s);
 // Lets kernels and copies running on device `accessor` address pool memory of device `owner` (NVLink peers); granted once
 // per pair and process.  False when the devices cannot reach each other.
 bool drb_peer_access(int owner, int accessor);

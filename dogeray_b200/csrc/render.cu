@@ -381,6 +381,145 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
 #undef DRB_POP
 }
 
+// ---- any hit ---------------------------------------------------------------------------------------
+// Occlusion query: does hit()'s test accept some primitive at t < tmax?  The traversal of k_trace<false> (persistent warps
+// with per-lane refill, packed slab test, shared-memory stack, nearest child next, the other hits pushed) with three
+// changes: the far bound of the slab test is the ray's own tmax for the whole ray (there is no shrinking `best`), the first
+// accepted primitive ends the ray, and the answer is one byte.  The primitive test is intersect_prim itself started from
+// best = tmax, so the two kernels accept the same primitives below that bound and occluded == (closest id >= 0 && closest
+// t < tmax) exactly: the padded boxes never cull an accepted hit (§4 of DESIGN.md), and a box holding a hit at t < tmax
+// still passes with its far bound lowered to tmax.  tmax (already clamped to 10000, > 0) rides in the w component of the
+// direction stream.
+// Leaves: with DRB_OCCLUDED_LEAF_NOW a lane tests each leaf as soon as it reaches it; by default it stashes the leaf and
+// the warp tests stashed leaves together, as k_trace does (DESIGN.md §5 has both measured).
+#ifndef DRB_OCCLUDED_LEAF_NOW
+#define DRB_OCCLUDED_LEAF_NOW 0
+#endif
+__global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_occluded(DevScene sc, float scene_scale, const float4* __restrict__ ro,
+                                                                                 const float4* __restrict__ rdv, uint8_t* __restrict__ occluded,
+                                                                                 uint32_t* counters, int refill, int leaf_batch, int step_min)
+{
+    const uint32_t count = counters[0];
+    const unsigned lane = threadIdx.x & 31u;
+    const unsigned lt_mask = (1u << lane) - 1u;
+
+    int node = kSentinel;
+    int leaf = 0;                                   // stashed leaf (~primitive slot, always < 0), 0 = none
+    uint32_t ray = 0xFFFFFFFFu;
+    bool exhausted = false;                         // warp-uniform: the queue has been handed out completely
+    bool hit_any = false;
+    f3 o = mk3(0.f), d = mk3(0.f);
+    float2 sxx = {}, syy = {}, szz = {}, cxx = {}, cyy = {}, czz = {};
+    uint32_t snx = 0x7410u, sny = 0x7410u, snz = 0x7410u, sfx = 0x7432u, sfy = 0x7432u, sfz = 0x7432u;
+    float tmax = 0.f;
+    extern __shared__ int s_stack[];
+    int* sp = s_stack + threadIdx.x;
+#define DRB_PUSH(v) do { *sp = (v); sp += 128; } while (0)
+#define DRB_POP() (sp -= 128, *sp)
+
+    for (;;) {
+        // ---- refill idle lanes (as k_trace) -----------------------------------------------------------
+        const bool idle = (node == kSentinel && leaf == 0);
+        const unsigned midle = __ballot_sync(0xffffffffu, idle);
+        if (midle == 0xffffffffu && exhausted) break;
+        if (!exhausted && (midle == 0xffffffffu || 32 - __popc(midle) < refill)) {
+            const int leader = __ffs(midle) - 1;
+            uint32_t base = 0;
+            if ((int)lane == leader) base = atomicAdd(&counters[CNT_TICKET], (uint32_t)__popc(midle));
+            base = __shfl_sync(0xffffffffu, base, leader);
+            if (base + (uint32_t)__popc(midle) >= count) exhausted = true;
+            if (idle) {
+                const uint32_t i = base + (uint32_t)__popc(midle & lt_mask);
+                if (i < count) {
+                    const float4 o4 = ro[i], d4 = rdv[i];
+                    if (!(d4.w > 0.0f) || sc.nprims == 0) {
+                        occluded[i] = 0;                    // nothing is accepted at t < tmax <= 0 (t > 1e-4 / t > 0)
+                    } else {
+                        ray = i;
+                        o = xyz(o4); d = xyz(d4);
+                        tmax = d4.w;
+                        hit_any = false;
+                        // the per-ray constants of k_trace, operation for operation
+                        const float ix = safe_inv(d.x), iy = safe_inv(d.y), iz = safe_inv(d.z);
+                        const float pad = fminf((fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fabsf(o.z)) + scene_scale) * 1.9073486e-6f, sc.pad_cap);
+                        const float sx = sc.qscale[0] * ix, sy = sc.qscale[1] * iy, sz = sc.qscale[2] * iz;
+                        const float px = copysignf(pad, ix), py = copysignf(pad, iy), pz = copysignf(pad, iz);
+                        sxx = make_float2(sx, sx); syy = make_float2(sy, sy); szz = make_float2(sz, sz);
+                        cxx = make_float2(fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x - px) * ix), fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x + px) * ix));
+                        cyy = make_float2(fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y - py) * iy), fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y + py) * iy));
+                        czz = make_float2(fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z - pz) * iz), fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z + pz) * iz));
+                        snx = ix >= 0.f ? 0x7410u : 0x7432u; sny = iy >= 0.f ? 0x7410u : 0x7432u; snz = iz >= 0.f ? 0x7410u : 0x7432u;
+                        sfx = snx ^ 0x22u; sfy = sny ^ 0x22u; sfz = snz ^ 0x22u;
+                        sp = s_stack + threadIdx.x; DRB_PUSH(kSentinel);
+                        node = 0;
+                    }
+                }
+            }
+        }
+        // ---- kSteps descent steps per lane between warp votes ----------------------------------------------
+#pragma unroll
+        for (int step = 0; step < kSteps; ++step) {
+        if (node >= 0) {
+            const WideNode* np = sc.wnodes + node;
+            const f8 nA = ldg256(np->bx), nB = ldg256(np->bz);
+#define DRB_PLANES(w, sn, sf, s_, c_) __ffma2_rn(make_float2(prmt_exp23(__float_as_uint(w), (sn)), prmt_exp23(__float_as_uint(w), (sf))), (s_), (c_))
+#define DRB_CHILD(c, wx, wy, wz)                                                                                              \
+            const float2 x##c = DRB_PLANES(wx, snx, sfx, sxx, cxx), y##c = DRB_PLANES(wy, sny, sfy, syy, cyy), z##c = DRB_PLANES(wz, snz, sfz, szz, czz); \
+            const float tn##c = fmaxf(fmaxf(x##c.x, y##c.x), fmaxf(z##c.x, 0.0f));                                            \
+            const float tf##c = fminf(fminf(x##c.y, y##c.y), fminf(z##c.y, tmax));                                            \
+            const uint32_t k##c = (tn##c <= tf##c) ? ((__float_as_uint(tn##c) & 0xFFFFFFFCu) | c##u) : 0xFFFFFFFFu;
+            DRB_CHILD(0, nA.lo.x, nA.hi.x, nB.lo.x)
+            DRB_CHILD(1, nA.lo.y, nA.hi.y, nB.lo.y)
+            DRB_CHILD(2, nA.lo.z, nA.hi.z, nB.lo.z)
+            DRB_CHILD(3, nA.lo.w, nA.hi.w, nB.lo.w)
+#undef DRB_CHILD
+#undef DRB_PLANES
+            const uint32_t kmin = min(min(k0, k1), min(k2, k3));
+            if (kmin == 0xFFFFFFFFu) node = DRB_POP();
+            else {
+                const int c0 = __float_as_int(nB.hi.x), c1 = __float_as_int(nB.hi.y), c2 = __float_as_int(nB.hi.z), c3 = __float_as_int(nB.hi.w);
+                if (k3 != kmin && k3 != 0xFFFFFFFFu) DRB_PUSH(c3);
+                if (k2 != kmin && k2 != 0xFFFFFFFFu) DRB_PUSH(c2);
+                if (k1 != kmin && k1 != 0xFFFFFFFFu) DRB_PUSH(c1);
+                if (k0 != kmin && k0 != 0xFFFFFFFFu) DRB_PUSH(c0);
+                node = (kmin & 2u) ? ((kmin & 1u) ? c3 : c2) : ((kmin & 1u) ? c1 : c0);
+            }
+        }
+#if DRB_OCCLUDED_LEAF_NOW
+        if (node < 0 && node != kSentinel) {
+            float b = tmax; int bp = -1;
+            intersect_prim(sc.prims, ~node, o, d, b, bp);
+            if (bp >= 0) { hit_any = true; node = kSentinel; } else node = DRB_POP();
+        }
+#else
+        if (node < 0 && node != kSentinel && leaf == 0) { leaf = node; node = DRB_POP(); }
+#endif
+        }
+#if !DRB_OCCLUDED_LEAF_NOW
+        // ---- postponed leaves: an accepted primitive ends the ray, whatever the lane holds next -------------
+        const unsigned mpend = __ballot_sync(0xffffffffu, leaf != 0);
+        if (mpend) {
+            const unsigned mstep = __ballot_sync(0xffffffffu, node >= 0);
+            if (__popc(mpend) >= leaf_batch || __popc(mstep) < step_min) {
+                if (leaf != 0) {
+                    float b = tmax; int bp = -1;
+                    intersect_prim(sc.prims, ~leaf, o, d, b, bp);
+                    leaf = 0;
+                    if (bp >= 0) { hit_any = true; node = kSentinel; }
+                }
+            }
+        }
+#endif
+        // ---- retire -----------------------------------------------------------------------------------
+        if (node == kSentinel && leaf == 0 && ray != 0xFFFFFFFFu) {
+            occluded[ray] = hit_any ? 1 : 0;
+            ray = 0xFFFFFFFFu;
+        }
+    }
+#undef DRB_PUSH
+#undef DRB_POP
+}
+
 // ---- shading ---------------------------------------------------------------------------------------
 // tex2D<uchar4> with the reference's descriptor (kernel.cu:1959-1964): normalised coordinates, wrap,
 // point filter; rows top-down
@@ -831,6 +970,50 @@ __global__ void k_store_ids(const uint2* __restrict__ hit, const int32_t* __rest
     ids[i] = p >= 0 ? orig[p] : -1;
     t[i] = __uint_as_float(h.x);
 }
+// one chunk of a ray query: caller's float3 arrays -> query streams (index in chunk; tmax of an occlusion query in d.w,
+// clamped to hit()'s 10000 -- a NaN stays NaN and is never occluded)
+__global__ void __launch_bounds__(256) k_load_query(const float* __restrict__ o3, const float* __restrict__ d3, const float* __restrict__ tmax,
+                                                     uint32_t n, float4* __restrict__ ro, float4* __restrict__ rdv)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const size_t k = (size_t)i * 3;
+    const float tm = tmax ? tmax[i] : kTMax;
+    ro[i] = make_float4(o3[k], o3[k + 1], o3[k + 2], __uint_as_float(i));
+    rdv[i] = make_float4(d3[k], d3[k + 1], d3[k + 2], tm > kTMax ? kTMax : tm);
+}
+// closest-hit results of one chunk -> caller's arrays.  (u, v) of a triangle hit is recomputed with intersect_prim's
+// operations in its order (same __frcp_rn, same left-associated dot / cross, no contraction in this TU): the values the
+// acceptance test used, bit for bit.
+__global__ void __launch_bounds__(256) k_store_query(const Prim* __restrict__ prims, const float4* __restrict__ ro, const float4* __restrict__ rdv,
+                                                      const uint2* __restrict__ hit, const int32_t* __restrict__ orig, uint32_t n,
+                                                      int32_t* __restrict__ ids, float* __restrict__ t, float* __restrict__ uv)
+{
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint2 h = hit[i];
+    const int p = (int)h.y;
+    ids[i] = p >= 0 ? orig[p] : -1;
+    if (t) t[i] = __uint_as_float(h.x);
+    if (!uv) return;
+    float u = 0.0f, v = 0.0f;
+    if (p >= 0) {
+        const float4 pa = prims[p].a;
+        if (__float_as_int(pa.w) == DRB_KIND_TRI) {
+            const f3 o = xyz(ro[i]), d = xyz(rdv[i]);
+            const f3 v0 = xyz(pa), e1 = xyz(prims[p].b), e2 = xyz(prims[p].c);
+            const f3 hv = cross(d, e2);
+            const float a = dot(e1, hv);
+            const float f = __frcp_rn(a);
+            const f3 sv = o - v0;
+            u = f * dot(sv, hv);
+            const f3 qv = cross(sv, e1);
+            v = f * dot(d, qv);
+        }
+    }
+    uv[2 * (size_t)i] = u;
+    uv[2 * (size_t)i + 1] = v;
+}
 // camera rays of queue 0 (slot order) -> row-major arrays
 __global__ void k_store_rays(FrameParams fp, uint32_t nslots, Queues q, float* __restrict__ o3, float* __restrict__ d3)
 {
@@ -881,6 +1064,15 @@ struct RenderBuffers {
     uint32_t* sort_vals[2] = { nullptr, nullptr };
     void* sort_tmp = nullptr;
     size_t sort_tmp_bytes = 0;
+};
+
+// Scratch of the ray-query entry points (drb_trace_device, drb_occluded_device), apart from the render's queues: a query
+// never reallocates or overwrites what the next frame uses.  Sized to one chunk of rays (40 B each).
+struct QueryBuffers {
+    size_t capacity = 0;                // rays per chunk
+    Queues q{};                         // ray_o[0], ray_d[0], hit and counters only
+    int trace_blocks = 0, occluded_blocks = 0;
+    size_t trace_smem = 0;              // stack of k_trace / k_occluded: (tree height + 2) levels x 128 lanes
 };
 
 namespace {
@@ -938,7 +1130,28 @@ struct DeviceFacts {
     int shade_blocks[64] = { 0 };
     std::map<std::pair<int, size_t>, int> trace_blocks;        // (device, dynamic smem) -> grid
     size_t max_smem_set[64] = { 0 };
+    std::map<std::pair<int, size_t>, int> occluded_blocks;     // the same for k_occluded
+    size_t occluded_smem_set[64] = { 0 };
 } g_facts;
+
+int occluded_shape(int device, size_t smem, int* blocks)
+{
+    std::lock_guard<std::mutex> g(g_facts.mu);
+    const int d = device & 63;
+    auto it = g_facts.occluded_blocks.find({ device, smem });
+    if (it == g_facts.occluded_blocks.end()) {
+        int sms = 148, per_sm = 1;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+        if (smem > g_facts.occluded_smem_set[d]) {
+            DRB_CUDA(cudaFuncSetAttribute(k_occluded, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            g_facts.occluded_smem_set[d] = smem;
+        }
+        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_occluded, kTraceThreads, smem));
+        it = g_facts.occluded_blocks.emplace(std::make_pair(device, smem), sms * std::max(per_sm, 1)).first;
+    }
+    *blocks = it->second;
+    return DRB_OK;
+}
 
 int launch_shape(int device, size_t trace_smem, int* trace_blocks, int* shade_blocks)
 {
@@ -1052,11 +1265,68 @@ int g_leaf_batch = []() { const char* e = getenv("DOGERAY_B200_LEAF_BATCH"); int
 int g_step_min = []() { const char* e = getenv("DOGERAY_B200_STEP_MIN"); int v = e ? atoi(e) : 20; return v < 1 ? 1 : v; }();
 
 // the closest-hit kernel for this scene: large scenes push the other hit children far-to-near (see DRB_SORTED_PUSH_FROM)
-void launch_trace(const drb_scene* s, const RenderBuffers* rb, cudaStream_t stream, const DevScene& sc, float scale, const Queues& q, int cur, const uint32_t* order)
+void launch_trace(const drb_scene* s, int blocks, size_t smem, cudaStream_t stream, const DevScene& sc, float scale, const Queues& q, int cur,
+                  const uint32_t* order)
 {
     auto kernel = s->nprims >= (int64_t)DRB_SORTED_PUSH_FROM ? k_trace<true> : k_trace<false>;
-    kernel<<<rb->trace_blocks, kTraceThreads, rb->trace_smem, stream>>>(sc, scale, q.ray_o[cur], q.ray_d[cur], q.hit, q.counters, cur,
-                                                                      g_refill, g_leaf_batch, g_step_min, order);
+    kernel<<<blocks, kTraceThreads, smem, stream>>>(sc, scale, q.ray_o[cur], q.ray_d[cur], q.hit, q.counters, cur, g_refill, g_leaf_batch, g_step_min, order);
+}
+
+// rays per chunk of a ray query (DOGERAY_B200_QUERY_CHUNK, default 64 Mi: 2.6 GB of query scratch)
+size_t g_query_chunk = []() { const char* e = getenv("DOGERAY_B200_QUERY_CHUNK"); long v = e ? atol(e) : (64L << 20); return (size_t)std::min(std::max(v, 1L), 1L << 30); }();
+
+int ensure_query_buffers(drb_scene* s, size_t rays)
+{
+    if (s->qb && s->qb->capacity >= rays) return DRB_OK;
+    drb_query_buffers_free(s);
+    s->qb = new QueryBuffers();
+    QueryBuffers* qb = s->qb;
+    Queues& q = qb->q;
+    cudaStream_t st = s->stream;
+    DRB_CUDA(drb_dev_alloc((void**)&q.ray_o[0], rays * sizeof(float4), st));
+    DRB_CUDA(drb_dev_alloc((void**)&q.ray_d[0], rays * sizeof(float4), st));
+    DRB_CUDA(drb_dev_alloc((void**)&q.hit, rays * sizeof(uint2), st));
+    DRB_CUDA(drb_dev_alloc((void**)&q.counters, CNT_WORDS * sizeof(uint32_t), st));
+    DRB_CUDA(cudaMemsetAsync(q.counters, 0, CNT_WORDS * sizeof(uint32_t), st));
+    DRB_CUDA(cudaStreamSynchronize(st));             // the buffers are used from the caller's stream next
+    qb->trace_smem = (size_t)std::max(s->stack_levels, 3) * kTraceThreads * sizeof(int);
+    int shade_blocks = 0;
+    if (int rc = launch_shape(s->device, qb->trace_smem, &qb->trace_blocks, &shade_blocks)) return rc;
+    if (int rc = occluded_shape(s->device, qb->trace_smem, &qb->occluded_blocks)) return rc;
+    qb->capacity = rays;
+    return DRB_OK;
+}
+
+// Both ray queries, chunk by chunk on one stream without a host synchronisation: load, set the counters, traverse, store.
+// tmax == nullptr with occluded != nullptr: 10000 for every ray.
+int run_query(drb_scene* s, const float* o3, const float* d3, const float* tmax, int64_t n, int32_t* ids, float* t, float* uv,
+              uint8_t* occluded, void* stream)
+{
+    DRB_CUDA(cudaSetDevice(s->device));
+    const size_t chunk = std::min<size_t>((size_t)n, g_query_chunk);
+    if (int rc = ensure_query_buffers(s, chunk)) return rc;
+    const QueryBuffers* qb = s->qb;
+    const Queues& q = qb->q;
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    const DevScene sc = dev_scene(s);
+    const float scale = scene_scale(s);
+    for (int64_t done = 0; done < n; done += (int64_t)chunk) {
+        const uint32_t m = (uint32_t)std::min<int64_t>((int64_t)chunk, n - done);
+        const unsigned grid = (m + 255u) / 256u;
+        k_load_query<<<grid, 256, 0, st>>>(o3 + 3 * done, d3 + 3 * done, tmax ? tmax + done : nullptr, m, q.ray_o[0], q.ray_d[0]);
+        k_prepare<<<1, 32, 0, st>>>(q.counters, -1, 0, m);
+        if (occluded) {
+            // one byte per ray, written by the traversal itself: there is nothing to map back
+            k_occluded<<<qb->occluded_blocks, kTraceThreads, qb->trace_smem, st>>>(sc, scale, q.ray_o[0], q.ray_d[0], occluded + done, q.counters,
+                                                                                  g_refill, g_leaf_batch, g_step_min);
+        } else {
+            launch_trace(s, qb->trace_blocks, qb->trace_smem, st, sc, scale, q, 0, nullptr);
+            k_store_query<<<grid, 256, 0, st>>>(s->prims, q.ray_o[0], q.ray_d[0], q.hit, s->orig_id, m, ids + done, t ? t + done : nullptr,
+                                                uv ? uv + 2 * done : nullptr);
+        }
+    }
+    DRB_CUDA(cudaGetLastError());
+    return DRB_OK;
 }
 
 
@@ -1194,7 +1464,7 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
                 }
             }
             if (stats) { auto e0 = pool.get(), e1 = pool.get(); trace_ev.push_back({ e0, e1 }); DRB_CUDA(cudaEventRecord(e0, stream)); }
-            launch_trace(s, rb, stream, sc, fp.scene_scale, q, cur, order);
+            launch_trace(s, rb->trace_blocks, rb->trace_smem, stream, sc, fp.scene_scale, q, cur, order);
             if (stats) DRB_CUDA(cudaEventRecord(trace_ev.back().second, stream));
             k_shade<<<std::min<uint32_t>((uint32_t)rb->shade_blocks, (live + 4u * kShadeRays - 1u) / (4u * kShadeRays)), 128, 0, stream>>>(
                 sc, fp, q.ray_o[cur], q.ray_d[cur], q.thr[cur], q.hit, q.ray_o[cur ^ 1], q.ray_d[cur ^ 1], q.thr[cur ^ 1], q.contrib, q.counters, cur,
@@ -1254,6 +1524,17 @@ void drb_render_buffers_free(drb_scene* s)
     drb_dev_free(s->rb->sort_tmp, st);
     delete s->rb;
     s->rb = nullptr;
+}
+
+void drb_query_buffers_free(drb_scene* s)
+{
+    if (!s || !s->qb) return;
+    Queues& q = s->qb->q;
+    cudaStream_t st = s->stream;
+    cudaDeviceSynchronize();                          // queries run on caller streams
+    drb_dev_free(q.ray_o[0], st); drb_dev_free(q.ray_d[0], st); drb_dev_free(q.hit, st); drb_dev_free(q.counters, st);
+    delete s->qb;
+    s->qb = nullptr;
 }
 
 extern "C" {
@@ -1537,13 +1818,27 @@ int drb_trace_ids(drb_scene* s, const float* o3, const float* d3, int64_t n, int
     const uint32_t nn = (uint32_t)n;
     k_load_rays<<<(nn + 255) / 256, 256, 0, stream>>>(d_o, d_d, nn, q);
     k_prepare<<<1, 32, 0, stream>>>(q.counters, -1, 0, nn);
-    launch_trace(s, rb, stream, dev_scene(s), scene_scale(s), q, 0, nullptr);
+    launch_trace(s, rb->trace_blocks, rb->trace_smem, stream, dev_scene(s), scene_scale(s), q, 0, nullptr);
     k_store_ids<<<(nn + 255) / 256, 256, 0, stream>>>(q.hit, s->orig_id, nn, d_ids, d_t);
     DRB_CUDA(cudaGetLastError());
     DRB_CUDA(cudaMemcpyAsync(ids, d_ids, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
     if (t) DRB_CUDA(cudaMemcpyAsync(t, d_t, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
     DRB_CUDA(cudaStreamSynchronize(stream));
     return DRB_OK;
+}
+
+int drb_trace_device(drb_scene* s, const float* o3_dev, const float* d3_dev, int64_t n, int32_t* ids_dev, float* t_dev, float* uv_dev, void* stream)
+{
+    if (!s || n < 0 || (n && (!o3_dev || !d3_dev || !ids_dev))) { drb_set_error("drb_trace_device: bad argument"); return DRB_ERR_ARG; }
+    if (n == 0) return DRB_OK;
+    return run_query(s, o3_dev, d3_dev, nullptr, n, ids_dev, t_dev, uv_dev, nullptr, stream);
+}
+
+int drb_occluded_device(drb_scene* s, const float* o3_dev, const float* d3_dev, const float* tmax_dev, int64_t n, uint8_t* occluded_dev, void* stream)
+{
+    if (!s || n < 0 || (n && (!o3_dev || !d3_dev || !occluded_dev))) { drb_set_error("drb_occluded_device: bad argument"); return DRB_ERR_ARG; }
+    if (n == 0) return DRB_OK;
+    return run_query(s, o3_dev, d3_dev, tmax_dev, n, nullptr, nullptr, nullptr, occluded_dev, stream);
 }
 
 int drb_primary_rays(drb_scene* s, const drb_settings* settings, const drb_opts* opts, uint32_t sample, float* o3, float* d3)

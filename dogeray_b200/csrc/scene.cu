@@ -1030,6 +1030,7 @@ void drb_scene_free(drb_scene* s)
     if (!s) return;
     cudaSetDevice(s->device);
     drb_render_buffers_free(s);
+    drb_query_buffers_free(s);
     cudaStream_t st = s->stream;
     if (st) cudaStreamSynchronize(st);
     for (void* p : { (void*)s->prims, (void*)s->recs, (void*)s->orig_id, (void*)s->textures, (void*)s->dbg.keys,

@@ -246,6 +246,26 @@ int drb_frame_i3(drb_scene* s, const drb_settings* settings, const drb_opts* opt
 /* Closest-hit object ids (index of the object line, -1 = miss) and distances for explicit rays:
  * the same query as hit() (kernel.cu:468-512).  o3/d3: n*3 floats on the host. */
 int drb_trace_ids(drb_scene* s, const float* o3, const float* d3, int64_t n, int32_t* ids, float* t);
+
+/* ---- ray queries on device arrays ----------------------------------------------------------
+ * Both calls take DEVICE arrays on the scene's device, enqueue their work on `stream` (a cudaStream_t; NULL -> the scene's
+ * own stream; for the legacy default stream pass cudaStreamLegacy, not 0) and return without synchronising: synchronise
+ * the stream before reading the results.  Rays are processed in chunks of DOGERAY_B200_QUERY_CHUNK (default 64 Mi) through
+ * query buffers of the scene's own, 40 B per ray of a chunk, kept until drb_scene_free; the render's buffers and results
+ * are not touched.  Like drb_render_device: one call at a time per handle, and successive calls on a handle ordered on ONE
+ * stream (the buffers are reused by the next call).  n == 0 does nothing; n < 0 or a NULL required pointer -> DRB_ERR_ARG. */
+
+/* Closest hit for n rays, o3_dev / d3_dev n*3 float32: exactly the query of drb_trace_ids / hit() (kernel.cu:468-512),
+ * t in (1e-4, 1e4) for triangles, (0, 1e4) for spheres.  ids_dev: object-line index or -1; t_dev (may be NULL): distance,
+ * -1 on a miss; uv_dev (may be NULL): n*2 float32, the (u, v) of hit_tri for a triangle hit (hit point =
+ * (1-u-v)*v0 + u*v1 + v*v2), (0, 0) for a sphere or a miss. */
+int drb_trace_device(drb_scene* s, const float* o3_dev, const float* d3_dev, int64_t n,
+                     int32_t* ids_dev, float* t_dev, float* uv_dev, void* stream);
+/* Any hit: occluded_dev[i] = 1 if some primitive is accepted by hit()'s test at a distance t < min(tmax_dev[i], 1e4), else 0
+ * (so exactly (closest id >= 0) && (closest t < tmax)); tmax <= 0 or NaN gives 0.  tmax_dev == NULL -> 1e4 for every ray.
+ * occluded_dev: n bytes (viewable as torch.bool).  Stops at the first accepted primitive. */
+int drb_occluded_device(drb_scene* s, const float* o3_dev, const float* d3_dev, const float* tmax_dev, int64_t n,
+                        uint8_t* occluded_dev, void* stream);
 /* The camera rays of sample `sample` for every pixel, row-major (y*W + x): what Kernel computes at
  * kernel.cu:1067-1076.  o3/d3: W*H*3 floats on the host. */
 int drb_primary_rays(drb_scene* s, const drb_settings* settings, const drb_opts* opts, uint32_t sample, float* o3, float* d3);
