@@ -139,6 +139,8 @@ _sig("drb_scene_create_ex", _i, _vp, _i, _u32, _pp)
 _sig("drb_scene_create_from_device", _i, _vp, _i, _u32, _vp, _vp, _pp)
 _sig("drb_scene_tree", _i, _vp, _vp, _vp, _vp, _vp)
 _sig("drb_scene_wide", _i, _vp, _vp, _vp)
+_sig("drb_scene_refit_device", _i, _vp, _vp, _i64, _vp)
+_sig("drb_scene_refit", _i, _vp, _vp, _i64)
 _sig("drb_scene_load", _i, _cp, _cp, _i, _pp)
 _sig("drb_scene_free", None, _vp)
 _sig("drb_scene_settings", _i, _vp, C.POINTER(Settings))
@@ -175,7 +177,7 @@ EXPORTED_SYMBOLS = [
     "drb_host_scene_num_objects", "drb_host_scene_objects", "drb_host_scene_settings",
     "drb_host_scene_num_textures", "drb_host_scene_texture_path", "drb_host_scene_num_skipped", "drb_host_scene_num_renderable",
     "drb_scene_create_from_device", "drb_scene_create_multi", "drb_render_multi_times",
-    "drb_rts_write", "drb_settings_default", "drb_scene_create", "drb_scene_create_ex", "drb_scene_tree", "drb_scene_wide", "drb_scene_load", "drb_scene_free",
+    "drb_rts_write", "drb_settings_default", "drb_scene_create", "drb_scene_create_ex", "drb_scene_tree", "drb_scene_wide", "drb_scene_refit_device", "drb_scene_refit", "drb_scene_load", "drb_scene_free",
     "drb_scene_settings", "drb_scene_num_prims", "drb_scene_num_objects", "drb_scene_build_info",
     "drb_scene_lbvh", "drb_opts_default", "drb_render_device", "drb_render", "drb_render_multi", "drb_frame_i3",
     "drb_trace_ids", "drb_trace_device", "drb_occluded_device", "drb_primary_rays", "drb_tonemap", "drb_tonemap_device", "drb_write_bmp",
@@ -464,6 +466,33 @@ class Scene:
         child = np.zeros((n, 4), np.int32); boxes = np.zeros((n, 4, 3), np.uint32)
         _check(_lib.drb_scene_wide(self._h, child.ctypes.data, boxes.ctypes.data))
         return dict(child=child, boxes=boxes)
+
+    def refit_device(self, objects_ptr: int, n: int, stream: Optional[int] = None):
+        """New object lines for the same tree: n (== num_objects) records of OBJECT_DTYPE in DEVICE memory at `objects_ptr`,
+        produced on `stream` (a raw handle; None -> the scene's own).  Synchronous: the scene is updated when it returns."""
+        _check(_lib.drb_scene_refit_device(self._h, objects_ptr, n, _stream_handle(stream)))
+
+    def refit(self, objects, *, stream=None):
+        """Update the resident scene in place from new object lines, keeping its tree (drb_scene_refit): a host OBJECT_DTYPE
+        array of num_objects records, or a contiguous CUDA tensor on the scene's device holding them (nbytes ==
+        num_objects * 156, e.g. float32 (n, 39)) written on `stream` (a torch.cuda.Stream, default the current one)."""
+        n = self.num_objects
+        if isinstance(objects, np.ndarray):
+            if objects.dtype != OBJECT_DTYPE or objects.ndim != 1 or len(objects) != n:
+                raise ValueError("refit takes %d records of OBJECT_DTYPE, got %s %s" % (n, objects.dtype, objects.shape))
+            a = np.ascontiguousarray(objects)
+            _check(_lib.drb_scene_refit(self._h, a.ctypes.data, n))
+            return
+        import torch
+        if not isinstance(objects, torch.Tensor):
+            raise ValueError("refit takes a numpy OBJECT_DTYPE array or a CUDA tensor, got %s" % type(objects).__name__)
+        dev = torch.device("cuda", self.device)
+        if objects.device != dev or not objects.is_contiguous() or objects.nbytes != n * OBJECT_DTYPE.itemsize:
+            raise ValueError("refit takes a contiguous tensor of %d bytes on %s, got %d bytes on %s" %
+                             (n * OBJECT_DTYPE.itemsize, dev, objects.nbytes, objects.device))
+        if stream is None:
+            stream = torch.cuda.current_stream(dev)
+        self.refit_device(objects.data_ptr(), n, stream.cuda_stream)
 
     @staticmethod
     def _opts(seed=0, sample_base=0, sample_count=None, batch_paths=0, flags=0, stream=None, tile_rank=0, tile_count=0) -> Opts:

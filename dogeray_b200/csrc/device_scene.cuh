@@ -110,6 +110,8 @@ struct drb_scene {
     WideNode* wnodes = nullptr; // the traversal structure
     int64_t nwnodes = 0;
     int wide_levels = 0;        // height of the wide tree (levels of the breadth-first collapse)
+    int* wide_level_start = nullptr; // first node of every level, wide_levels + 1 entries (the refit's bottom-up order)
+    uint32_t* refit_inv = nullptr;   // object line -> slot << 1 | sphere, or ~0u; made by the first refit
     int stack_levels = 3;       // traversal stack entries a lane can need (exact bound from the collapse + sentinel + 1)
     Prim* prims = nullptr;
     ShadeRec* recs = nullptr;

@@ -68,6 +68,66 @@ __global__ void k_init_bounds(int* b)
     else if (threadIdx.x < 6) b[threadIdx.x] = (int)0x80000000;  // max
 }
 
+// One renderable object line -> its primitive and float box (from the vertices, or centre +- |radius|) and the flags of its
+// shading record (or-ed into `flags`); pack_rec then makes the record.  The build (k_pack) and the refit (k_refit_check, k_refit_pack) share
+// both, so a refitted primitive is bit for bit what a fresh build packs from the same line.
+__device__ __forceinline__ void pack_prim(const drb_object& o, Prim& p, uint32_t& flags, float lo[3], float hi[3])
+{
+    if (o.type == 0) {
+        const float r = fabsf(o.dim[0]);
+        p.a = make_float4(o.pos[0], o.pos[1], o.pos[2], __int_as_float(DRB_KIND_SPHERE));
+        p.b = make_float4(o.dim[0], 0.f, 0.f, 0.f);
+        p.c = make_float4(0.f, 0.f, 0.f, 0.f);
+        p.d = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int a = 0; a < 3; ++a) { lo[a] = o.pos[a] - r; hi[a] = o.pos[a] + r; }
+        flags |= DRB_SF_SPHERE;
+    } else {
+        p.a = make_float4(o.pos[0], o.pos[1], o.pos[2], __int_as_float(DRB_KIND_TRI));
+        p.b = make_float4(o.dim[0] - o.pos[0], o.dim[1] - o.pos[1], o.dim[2] - o.pos[2], 0.f);
+        p.c = make_float4(o.rot[0] - o.pos[0], o.rot[1] - o.pos[1], o.rot[2] - o.pos[2], 0.f);
+        p.d = make_float4(0.f, 0.f, 0.f, 0.f);
+        for (int a = 0; a < 3; ++a) {
+            lo[a] = fminf(o.pos[a], fminf(o.dim[a], o.rot[a]));
+            hi[a] = fmaxf(o.pos[a], fmaxf(o.dim[a], o.rot[a]));
+        }
+        const bool face = o.norm[2] != -20.0f;
+        const bool smooth = face && o.n1[2] != -20.0f && o.smooth;
+        if (face) flags |= DRB_SF_FACE_NORMAL;
+        if (smooth) flags |= DRB_SF_SMOOTH;
+        if (o.checker) flags |= DRB_SF_CHECKER;
+        if (smooth || o.checker || o.texnum >= 0 || o.rtexnum >= 0) flags |= DRB_SF_NEEDS_UV;
+    }
+}
+__device__ __forceinline__ void pack_rec(const drb_object& o, uint32_t flags, ShadeRec& r)
+{
+    r.r[0] = make_float4(o.norm[0], o.norm[1], o.norm[2], __uint_as_float(flags));
+    r.r[1] = make_float4(o.col[0], o.col[1], o.col[2], o.add_y);
+    r.r[2] = make_float4(o.add_x, __int_as_float(o.mat), __int_as_float(o.texnum), __int_as_float(o.rtexnum));
+    r.r[3] = make_float4(o.n1[0], o.n1[1], o.n1[2], o.t1[0]);
+    r.r[4] = make_float4(o.n2[0], o.n2[1], o.n2[2], o.t2[0]);
+    r.r[5] = make_float4(o.n3[0], o.n3[1], o.n3[2], o.t3[0]);
+    r.r[6] = make_float4(o.t1[1], o.t2[1], o.t3[1], 0.f);
+    r.r[7] = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+// warp-reduce per-lane boxes into the ordered-int scene bounds, one atomic per warp and component
+__device__ __forceinline__ void reduce_bounds(const float lo[3], const float hi[3], int* __restrict__ scene_bounds)
+{
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        float l = lo[a], h = hi[a];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            l = fminf(l, __shfl_xor_sync(0xffffffffu, l, off));
+            h = fmaxf(h, __shfl_xor_sync(0xffffffffu, h, off));
+        }
+        if ((threadIdx.x & 31) == 0 && l <= h) {
+            atomicMin(&scene_bounds[a], float_to_ordered(l));
+            atomicMax(&scene_bounds[3 + a], float_to_ordered(h));
+        }
+    }
+}
+
 // one thread per object line
 __global__ void k_pack(const drb_object* __restrict__ objs, int64_t n, const int* __restrict__ flag, const int* __restrict__ slot, int nprims,
                        Prim* __restrict__ prims, ShadeRec* __restrict__ recs, int32_t* __restrict__ orig,
@@ -84,61 +144,18 @@ __global__ void k_pack(const drb_object* __restrict__ objs, int64_t n, const int
     if (live) {
         const drb_object o = objs[i];
         const int k = slot[i];
-        Prim p;
         uint32_t flags = 0;
-        if (o.type == 0) {
-            const float r = fabsf(o.dim[0]);
-            p.a = make_float4(o.pos[0], o.pos[1], o.pos[2], __int_as_float(DRB_KIND_SPHERE));
-            p.b = make_float4(o.dim[0], 0.f, 0.f, 0.f);
-            p.c = make_float4(0.f, 0.f, 0.f, 0.f);
-            p.d = make_float4(0.f, 0.f, 0.f, 0.f);
-            for (int a = 0; a < 3; ++a) { lo[a] = o.pos[a] - r; hi[a] = o.pos[a] + r; }
-            flags |= DRB_SF_SPHERE;
-        } else {
-            p.a = make_float4(o.pos[0], o.pos[1], o.pos[2], __int_as_float(DRB_KIND_TRI));
-            p.b = make_float4(o.dim[0] - o.pos[0], o.dim[1] - o.pos[1], o.dim[2] - o.pos[2], 0.f);
-            p.c = make_float4(o.rot[0] - o.pos[0], o.rot[1] - o.pos[1], o.rot[2] - o.pos[2], 0.f);
-            p.d = make_float4(0.f, 0.f, 0.f, 0.f);
-            for (int a = 0; a < 3; ++a) {
-                lo[a] = fminf(o.pos[a], fminf(o.dim[a], o.rot[a]));
-                hi[a] = fmaxf(o.pos[a], fmaxf(o.dim[a], o.rot[a]));
-            }
-            const bool face = o.norm[2] != -20.0f;
-            const bool smooth = face && o.n1[2] != -20.0f && o.smooth;
-            if (face) flags |= DRB_SF_FACE_NORMAL;
-            if (smooth) flags |= DRB_SF_SMOOTH;
-            if (o.checker) flags |= DRB_SF_CHECKER;
-            if (smooth || o.checker || o.texnum >= 0 || o.rtexnum >= 0) flags |= DRB_SF_NEEDS_UV;
-        }
+        Prim p;
+        pack_prim(o, p, flags, lo, hi);
         prims[k] = p;
         ShadeRec r;
-        r.r[0] = make_float4(o.norm[0], o.norm[1], o.norm[2], __uint_as_float(flags));
-        r.r[1] = make_float4(o.col[0], o.col[1], o.col[2], o.add_y);
-        r.r[2] = make_float4(o.add_x, __int_as_float(o.mat), __int_as_float(o.texnum), __int_as_float(o.rtexnum));
-        r.r[3] = make_float4(o.n1[0], o.n1[1], o.n1[2], o.t1[0]);
-        r.r[4] = make_float4(o.n2[0], o.n2[1], o.n2[2], o.t2[0]);
-        r.r[5] = make_float4(o.n3[0], o.n3[1], o.n3[2], o.t3[0]);
-        r.r[6] = make_float4(o.t1[1], o.t2[1], o.t3[1], 0.f);
-        r.r[7] = make_float4(0.f, 0.f, 0.f, 0.f);
+        pack_rec(o, flags, r);
         recs[k] = r;
         orig[k] = (int32_t)i;
         bmin[k] = make_float4(lo[0], lo[1], lo[2], 0.f);
         bmax[k] = make_float4(hi[0], hi[1], hi[2], 0.f);
     }
-    // warp-reduce the bounds, one atomic per warp and component
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        float l = lo[a], h = hi[a];
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            l = fminf(l, __shfl_xor_sync(0xffffffffu, l, off));
-            h = fmaxf(h, __shfl_xor_sync(0xffffffffu, h, off));
-        }
-        if ((threadIdx.x & 31) == 0 && l <= h) {
-            atomicMin(&scene_bounds[a], float_to_ordered(l));
-            atomicMax(&scene_bounds[3 + a], float_to_ordered(h));
-        }
-    }
+    reduce_bounds(lo, hi, scene_bounds);
 }
 
 __device__ __forceinline__ uint64_t spread21(uint32_t v)
@@ -479,7 +496,7 @@ __global__ void __launch_bounds__(kBuildThreads) k_wide_all(const int32_t* __res
                                                             const float4* __restrict__ lmin, const float4* __restrict__ lmax,
                                                             const int* __restrict__ scene_bounds, int max_nodes,
                                                             int32_t* wq0, int32_t* wq1, int4* slots, int* counts, unsigned long long* blk_tot,
-                                                            WideNode* out, int* need, BuildCtl* ctl)
+                                                            WideNode* out, int* need, int* level_start, BuildCtl* ctl)
 {
     cg::grid_group grid = cg::this_grid();
     __shared__ int s_level_start[kMaxWideLevels + 1];
@@ -561,6 +578,8 @@ __global__ void __launch_bounds__(kBuildThreads) k_wide_all(const int32_t* __res
     }
     if (t == 0) s_level_start[min(levels, kMaxWideLevels)] = level_base;
     __syncthreads();
+    if (b == 0)                                                     // the level boundaries stay with the scene for refits
+        for (int L = t; L <= min(levels, kMaxWideLevels); L += kBuildThreads) level_start[L] = s_level_start[L];
     // exact stack bound, deepest level first (children live on the next level, so they are done)
     if (!err)
         for (int L = levels - 1; L >= 0; --L) {
@@ -585,14 +604,135 @@ __global__ void __launch_bounds__(kBuildThreads) k_wide_all(const int32_t* __res
     }
 }
 
-__global__ void k_wide_single(const float4* __restrict__ lmin, const float4* __restrict__ lmax, const int* __restrict__ scene_bounds, WideNode* __restrict__ out)
+__global__ void k_wide_single(const float4* __restrict__ lmin, const float4* __restrict__ lmax, const int* __restrict__ scene_bounds, WideNode* __restrict__ out,
+                              int* __restrict__ level_start)
 {
+    level_start[0] = 0; level_start[1] = 1;
     WideNode nd;
     uint32_t q[3];
     quant_child(lmin[0], lmax[0], scene_bounds, q);
     for (int k = 0; k < 4; ++k) { nd.bx[k] = nd.by[k] = nd.bz[k] = 0x0000FFFFu; nd.child[k] = DRB_WIDE_EMPTY; }
     nd.bx[0] = q[0]; nd.by[0] = q[1]; nd.bz[0] = q[2]; nd.child[0] = ~0;
     out[0] = nd;
+}
+
+// ---- refit: new object lines, same tree ----------------------------------------------------------------
+// quant_axis is monotone (float subtract, divide by a positive scale, floor / ceil and the clamp each are), so the
+// quantised box of a union is the integer union of the quantised boxes: min of the low halves, max of the high halves,
+// with an empty slot (min 65535, max 0) neutral.  An internal child's box is therefore the integer union of the four
+// boxes of the wide node it links to -- bit for bit what k_wide_all quantises from the float union of the same leaves --
+// and the refit never needs the binary tree: leaf boxes on the new grid, then the integer union level by level, deepest
+// first.
+struct RefitCtl {
+    int bounds[6];                      // scene bounds of the new leaf boxes (ordered ints, as in the build)
+    unsigned long long bad;             // (first offending line << 2) | reason, ~0 when every line passed
+};
+constexpr unsigned kRefitKindChanged = 1u, kRefitNonFinite = 2u;
+constexpr uint32_t kRefitNoSlot = 0xFFFFFFFFu;
+
+__global__ void k_refit_init(RefitCtl* ctl)
+{
+    if (threadIdx.x < 3) ctl->bounds[threadIdx.x] = 0x7FFFFFFF;
+    else if (threadIdx.x < 6) ctl->bounds[threadIdx.x] = (int)0x80000000;
+    else if (threadIdx.x == 6) ctl->bad = ~0ull;
+}
+
+// object line -> slot << 1 | (sphere) of its primitive, kRefitNoSlot for lines outside the tree; built once per scene
+__global__ void k_refit_inverse(const int32_t* __restrict__ orig, const Prim* __restrict__ prims, int nprims, uint32_t* __restrict__ inv)
+{
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < nprims) inv[orig[k]] = ((uint32_t)k << 1) | (__float_as_int(prims[k].a.w) == DRB_KIND_SPHERE ? 1u : 0u);
+}
+
+__device__ __forceinline__ bool finite3(const float v[3]) { return isfinite(v[0]) && isfinite(v[1]) && isfinite(v[2]); }
+
+// one thread per object line: validate, leaf box (k_pack's operations) into scratch, scene bounds.  Writes nothing of the
+// scene, so a refused refit leaves it as it was.
+__global__ void k_refit_check(const drb_object* __restrict__ objs, int64_t n, const uint32_t* __restrict__ inv,
+                              float4* __restrict__ lmin, float4* __restrict__ lmax, RefitCtl* __restrict__ ctl)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    float lo[3] = { 3.0e38f, 3.0e38f, 3.0e38f }, hi[3] = { -3.0e38f, -3.0e38f, -3.0e38f };
+    if (i < n) {
+        const drb_object& o = objs[i];
+        const uint32_t e = inv[i];
+        unsigned bad = 0;
+        if (drb_object_renderable(o) != (e != kRefitNoSlot) || (e != kRefitNoSlot && (o.type == 0) != ((e & 1u) != 0)))
+            bad = kRefitKindChanged;
+        else if (e != kRefitNoSlot) {
+            Prim p;
+            uint32_t flags = 0;
+            pack_prim(o, p, flags, lo, hi);
+            const bool ok = o.type == 0 ? finite3(o.pos) && isfinite(o.dim[0]) && finite3(lo) && finite3(hi)
+                                        : finite3(o.pos) && finite3(o.dim) && finite3(o.rot);
+            if (ok) {
+                lmin[e >> 1] = make_float4(lo[0], lo[1], lo[2], 0.f);
+                lmax[e >> 1] = make_float4(hi[0], hi[1], hi[2], 0.f);
+            } else bad = kRefitNonFinite;
+        }
+        if (bad) {
+            atomicMin(&ctl->bad, ((unsigned long long)i << 2) | bad);
+            for (int a = 0; a < 3; ++a) { lo[a] = 3.0e38f; hi[a] = -3.0e38f; }
+        }
+    }
+    reduce_bounds(lo, hi, ctl->bounds);
+}
+
+// one thread per object line: primitive and shading record of every line in the tree, once k_refit_check passed them all
+__global__ void k_refit_pack(const drb_object* __restrict__ objs, int64_t n, const uint32_t* __restrict__ inv, const RefitCtl* __restrict__ ctl,
+                             Prim* __restrict__ prims, ShadeRec* __restrict__ recs)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || ctl->bad != ~0ull) return;
+    const uint32_t e = inv[i];
+    if (e == kRefitNoSlot) return;
+    const drb_object o = objs[i];
+    const int k = (int)(e >> 1);
+    float lo[3], hi[3];
+    uint32_t flags = 0;
+    Prim p;
+    pack_prim(o, p, flags, lo, hi);
+    prims[k] = p;
+    ShadeRec r;
+    pack_rec(o, flags, r);
+    recs[k] = r;
+}
+
+// The node boxes in ONE cooperative launch, deepest level first (the shape of k_wide_all's stack-bound pass): a leaf child
+// is quantised on the new grid, an internal child is the integer union of its node's four boxes, finished one level down.
+__global__ void __launch_bounds__(kBuildThreads) k_refit_wide(const int* __restrict__ level_start, int levels, const float4* __restrict__ lmin,
+                                                              const float4* __restrict__ lmax, const RefitCtl* ctl, WideNode* nodes)
+{
+    cg::grid_group grid = cg::this_grid();
+    if (ctl->bad != ~0ull) return;                                  // the same in every block: nobody waits at a barrier
+    const int nb = (int)gridDim.x, b = (int)blockIdx.x, t = (int)threadIdx.x;
+    for (int L = levels - 1; L >= 0; --L) {
+        const int l0 = level_start[L], l1 = level_start[L + 1];
+        for (int i = l0 + b * kBuildThreads + t; i < l1; i += nb * kBuildThreads) {
+            WideNode nd = nodes[i];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int c = nd.child[k];
+                if (c == DRB_WIDE_EMPTY) continue;
+                uint32_t q[3];
+                if (c < 0) quant_child(lmin[~c], lmax[~c], ctl->bounds, q);
+                else {
+                    const WideNode& ch = nodes[c];
+                    const uint32_t* w[3] = { ch.bx, ch.by, ch.bz };
+#pragma unroll
+                    for (int a = 0; a < 3; ++a) {
+                        uint32_t mn = 0xFFFFu, mx = 0u;
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) { mn = min(mn, w[a][j] & 0xFFFFu); mx = max(mx, w[a][j] >> 16); }
+                        q[a] = mn | (mx << 16);
+                    }
+                }
+                nd.bx[k] = q[0]; nd.by[k] = q[1]; nd.bz[k] = q[2];
+            }
+            nodes[i] = nd;
+        }
+        grid.sync();
+    }
 }
 
 template <typename T> int dev_alloc(T** p, size_t count, cudaStream_t st)
@@ -809,7 +949,7 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
     const bool lbvh_only = (s->build_flags & DRB_BUILD_LBVH_ONLY) != 0;
     const int nprims = (int)drb_host_scene_num_renderable(hs);
     const drb_object* d_objs = objs_dev;
-    int* d_flag = nullptr; int* d_slot = nullptr; int* d_bounds = nullptr; BuildCtl* d_ctl = nullptr;
+    int* d_flag = nullptr; int* d_slot = nullptr; int* d_bounds = nullptr; BuildCtl* d_ctl = nullptr; int* d_levels = nullptr;
     if (!d_objs) {
         drb_object* up = nullptr;
         if (int rc = tmp.alloc(&up, (size_t)nobj)) return rc;
@@ -820,6 +960,7 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
     if (int rc = tmp.alloc(&d_slot, (size_t)nobj + 1)) return rc;
     if (int rc = tmp.alloc(&d_bounds, 8)) return rc;
     if (int rc = tmp.alloc(&d_ctl, 1)) return rc;
+    if (int rc = tmp.alloc(&d_levels, (size_t)kMaxWideLevels + 1)) return rc;
     DRB_CUDA(cudaMemsetAsync(d_ctl, 0, sizeof(BuildCtl), st));
     DRB_CUDA(cudaEventRecord(ev.e[1], st));
     clk.mark("upload-enqueue");
@@ -945,10 +1086,10 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
             const float4* c_lmin = lmin; const float4* c_lmax = lmax; const int* c_bounds = d_bounds;
             int max_nodes = (int)nint;
             void* args[] = { &c_left, &c_right, &c_nmin, &c_nmax, &c_lmin, &c_lmax, &c_bounds, &max_nodes, &wq[0], &wq[1], &wslots, &wcounts, &wtot,
-                             &s->wnodes, &wneed, &d_ctl };
+                             &s->wnodes, &wneed, &d_levels, &d_ctl };
             DRB_CUDA(cudaLaunchCooperativeKernel((const void*)k_wide_all, dim3(blocks), dim3(kBuildThreads), args, 0, st));
         } else {
-            k_wide_single<<<1, 1, 0, st>>>(lmin, lmax, d_bounds, s->wnodes);
+            k_wide_single<<<1, 1, 0, st>>>(lmin, lmax, d_bounds, s->wnodes, d_levels);
         }
         DRB_CUDA(cudaMemcpyAsync(hb, d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
         DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl, sizeof ctl, cudaMemcpyDeviceToHost, st));
@@ -967,6 +1108,8 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
         else { s->nwnodes = 1; s->wide_levels = 1; s->stack_levels = 3; s->info.max_depth = 1; }
         s->info.rebuild_iterations = ctl.rounds;
         s->info.nwide = s->nwnodes; s->info.wide_levels = s->wide_levels; s->info.stack_levels = s->stack_levels;
+        if (int rc = dev_alloc(&s->wide_level_start, (size_t)s->wide_levels + 1, st)) return rc;
+        DRB_CUDA(cudaMemcpyAsync(s->wide_level_start, d_levels, ((size_t)s->wide_levels + 1) * sizeof(int), cudaMemcpyDeviceToDevice, st));
     }
     float ms = 0;
     cudaEventElapsedTime(&ms, ev.e[0], ev.e[1]); s->info.upload_ms = ms;
@@ -1009,6 +1152,63 @@ int upload_textures(drb_scene* s, const drb_host_scene* hs)
     return DRB_OK;
 }
 
+// New object lines into an existing tree, enqueued on `st` (already ordered after the caller's producer and the scene's
+// own stream) with ONE host synchronisation, for the validation result and the new bounds.  Scratch comes from the block
+// cache, so repeated refits make no allocator call after the first.
+int refit_tree(drb_scene* s, const drb_object* d_objs, cudaStream_t st)
+{
+    const int64_t nobj = s->nobjects;
+    const int nprims = (int)s->nprims;
+    const int T = 256;
+    Scratch tmp(st);
+    RefitCtl* d_ctl = nullptr; float4* lmin = nullptr; float4* lmax = nullptr;
+    if (int rc = tmp.alloc(&d_ctl, 1)) return rc;
+    if (int rc = tmp.alloc(&lmin, (size_t)nprims)) return rc;
+    if (int rc = tmp.alloc(&lmax, (size_t)nprims)) return rc;
+    if (!s->refit_inv) {
+        if (int rc = dev_alloc(&s->refit_inv, (size_t)nobj, st)) return rc;
+        DRB_CUDA(cudaMemsetAsync(s->refit_inv, 0xFF, (size_t)nobj * sizeof(uint32_t), st));
+        if (nprims > 0) k_refit_inverse<<<(nprims + T - 1) / T, T, 0, st>>>(s->orig_id, s->prims, nprims, s->refit_inv);
+    }
+    const unsigned grid_lines = (unsigned)((nobj + T - 1) / T);
+    k_refit_init<<<1, 32, 0, st>>>(d_ctl);
+    k_refit_check<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv, lmin, lmax, d_ctl);
+    if (nprims > 0) {
+        k_refit_pack<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv, d_ctl, s->prims, s->recs);
+        int blocks = 1;
+        if (int rc = coop_grid(s->device, (const void*)k_refit_wide, (int)((s->nwnodes + kBuildThreads - 1) / kBuildThreads), 2, &blocks)) return rc;
+        const int* c_levels = s->wide_level_start; int levels = s->wide_levels;
+        const float4* c_lmin = lmin; const float4* c_lmax = lmax; const RefitCtl* c_ctl = d_ctl;
+        void* args[] = { &c_levels, &levels, &c_lmin, &c_lmax, &c_ctl, &s->wnodes };
+        DRB_CUDA(cudaLaunchCooperativeKernel((const void*)k_refit_wide, dim3(blocks), dim3(kBuildThreads), args, 0, st));
+    }
+    DRB_CUDA(cudaGetLastError());
+    RefitCtl ctl;
+    DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl, sizeof ctl, cudaMemcpyDeviceToHost, st));
+    DRB_CUDA(cudaStreamSynchronize(st));                     // the one synchronisation of the refit
+    if (ctl.bad != ~0ull) {
+        const long long line = (long long)(ctl.bad >> 2);
+        if ((ctl.bad & 3ull) == kRefitKindChanged)
+            drb_set_error("drb_scene_refit: object line %lld changed whether it is rendered, or its kind (sphere / triangle)", line);
+        else
+            drb_set_error("drb_scene_refit: object line %lld has a non-finite vertex, centre or radius", line);
+        return DRB_ERR_ARG;
+    }
+    if (nprims > 0)
+        for (int a = 0; a < 3; ++a) { s->info.bounds_min[a] = ordered_to_float(ctl.bounds[a]); s->info.bounds_max[a] = ordered_to_float(ctl.bounds[3 + a]); }
+    return DRB_OK;
+}
+
+int refit_args(const drb_scene* s, const void* objects, int64_t nobjects)
+{
+    if (!s || nobjects < 0 || (nobjects > 0 && !objects)) { drb_set_error("drb_scene_refit: bad argument"); return DRB_ERR_ARG; }
+    if (nobjects != s->nobjects) {
+        drb_set_error("drb_scene_refit: %lld object lines given, the scene has %lld", (long long)nobjects, (long long)s->nobjects);
+        return DRB_ERR_ARG;
+    }
+    return DRB_OK;
+}
+
 } // namespace
 
 void drb_host_scene_unpin(drb_host_scene* hs)
@@ -1035,7 +1235,8 @@ void drb_scene_free(drb_scene* s)
     if (st) cudaStreamSynchronize(st);
     for (void* p : { (void*)s->prims, (void*)s->recs, (void*)s->orig_id, (void*)s->textures, (void*)s->dbg.keys,
                      (void*)s->dbg.order, (void*)s->dbg.parent, (void*)s->dbg.left, (void*)s->dbg.right, (void*)s->dbg.node_min,
-                     (void*)s->dbg.node_max, (void*)s->tree.left, (void*)s->tree.right, (void*)s->tree.node_min, (void*)s->tree.node_max, (void*)s->wnodes })
+                     (void*)s->dbg.node_max, (void*)s->tree.left, (void*)s->tree.right, (void*)s->tree.node_min, (void*)s->tree.node_max, (void*)s->wnodes,
+                     (void*)s->wide_level_start, (void*)s->refit_inv })
         if (p) drb_dev_free(p, st);
     for (void* p : s->texture_storage) drb_dev_free(p, st);
     if (st) cudaStreamDestroy(st);
@@ -1213,6 +1414,36 @@ int drb_scene_build_info(const drb_scene* s, drb_build_info* out)
     if (!s || !out) { drb_set_error("drb_scene_build_info: null argument"); return DRB_ERR_ARG; }
     *out = s->info;
     return DRB_OK;
+}
+
+int drb_scene_refit_device(drb_scene* s, const void* objects_dev, int64_t nobjects, void* stream)
+{
+    if (int rc = refit_args(s, objects_dev, nobjects)) return rc;
+    if (nobjects == 0) return DRB_OK;
+    DRB_CUDA(cudaSetDevice(s->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    if (st != s->stream) {
+        // the refit runs on the caller's stream, after what is already enqueued on the scene's own
+        cudaEvent_t done = nullptr;
+        DRB_CUDA(cudaEventCreateWithFlags(&done, cudaEventDisableTiming));
+        const cudaError_t e1 = cudaEventRecord(done, s->stream);
+        const cudaError_t e2 = e1 == cudaSuccess ? cudaStreamWaitEvent(st, done, 0) : e1;
+        cudaEventDestroy(done);
+        DRB_CUDA(e2);
+    }
+    return refit_tree(s, (const drb_object*)objects_dev, st);
+}
+
+int drb_scene_refit(drb_scene* s, const drb_object* objects_host, int64_t nobjects)
+{
+    if (int rc = refit_args(s, objects_host, nobjects)) return rc;
+    if (nobjects == 0) return DRB_OK;
+    DRB_CUDA(cudaSetDevice(s->device));
+    Scratch up(s->stream);
+    drb_object* d = nullptr;
+    if (int rc = up.alloc(&d, (size_t)nobjects)) return rc;
+    DRB_CUDA(cudaMemcpyAsync(d, objects_host, (size_t)nobjects * sizeof(drb_object), cudaMemcpyHostToDevice, s->stream));
+    return refit_tree(s, d, s->stream);
 }
 
 int drb_scene_lbvh(const drb_scene* s, uint64_t* keys, int32_t* order, int32_t* parent, int32_t* left, int32_t* right,

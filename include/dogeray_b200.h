@@ -177,6 +177,29 @@ int drb_scene_tree(const drb_scene* s, int32_t* left, int32_t* right, float* nod
  * that child on axis a (16-bit scene grid).  nwide entries each (drb_build_info.nwide). */
 int drb_scene_wide(const drb_scene* s, int32_t* child, uint32_t* boxes);
 
+/* Refit: replace the object lines of a resident scene and update its traversal tree in place.  The tree keeps its
+ * topology; only primitives, shading records and node boxes change (no Morton sort, no rebuild, same handle, and the
+ * query and render buffers stay).  The traversal cost of the tree grows as the geometry moves away from the arrangement
+ * it was built for; rebuild with drb_scene_create_from_device when it has moved far.
+ *   objects_dev  `nobjects` records of drb_object in file order, on the scene's device; nobjects must equal
+ *                drb_scene_num_objects(s).  Only read during the call.
+ *   stream       the stream that produced the array (a cudaStream_t; NULL -> the scene's own).  The refit runs on it,
+ *                after that stream's earlier work and after work already enqueued on the scene's own stream.  Work on
+ *                other streams that reads the scene must be finished by the caller before the call.
+ * Every line that was a renderable triangle or sphere at creation must still be one, of the same kind, no other line may
+ * become renderable, and the vertex, centre and radius values of renderable lines must be finite.  Otherwise the call
+ * returns DRB_ERR_ARG, drb_last_error() names the first offending line, and the scene is unchanged (every line is checked
+ * before anything is written).  Everything else in a line may change: vertices, normals, UVs, colour, roughness,
+ * material, texture ids (still indexing the textures uploaded at creation) and flags.  The camera is not part of a refit.
+ * One host synchronisation (for the validation result and the new bounds): when the call returns the refit is complete
+ * and later work on any stream sees the new scene.  drb_build_info then has the new bounds; every other field keeps its
+ * build-time value.  drb_scene_lbvh / drb_scene_tree (DRB_BUILD_KEEP_DEBUG) keep describing the build; drb_scene_wide
+ * returns the refitted nodes.  Box for box the result equals quantising the new leaf boxes on the grid of the new
+ * bounds and taking the integer union bottom-up over the unchanged links. */
+int drb_scene_refit_device(drb_scene* s, const void* objects_dev, int64_t nobjects, void* stream);
+/* Same from HOST records: copied into device scratch on the scene's own stream, then as above. */
+int drb_scene_refit(drb_scene* s, const drb_object* objects_host, int64_t nobjects);
+
 /* ---- rendering ------------------------------------------------------------------------ */
 typedef struct drb_opts {
     uint64_t seed;              /* Philox key */
