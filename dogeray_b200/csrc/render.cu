@@ -37,6 +37,7 @@
 #include <map>
 #include <mutex>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 namespace {
@@ -222,6 +223,16 @@ DRB_D float prmt_exp23(uint32_t w, uint32_t sel)
 
 constexpr int kSentinel = (int)0x80000000;     // bottom of every traversal stack: "this lane has no ray in flight"
 
+// What one traversal answers.  kClosest and kClosestSorted: the closest hit, hit()'s query (kernel.cu:468-512), with the hit
+// children besides the nearest one pushed unsorted or far-to-near (see DRB_SORTED_PUSH_FROM); a ray's result is (t, primitive
+// slot).  kAnyHit: does hit()'s test accept some primitive at t < tmax?  The ray's tmax (already clamped to 10000) rides in
+// the w component of the direction stream, starts `best`, and so is the slab test's far bound; the first accepted primitive
+// ends the ray, and the result is one byte.  The primitive test is intersect_prim started from best = tmax, so both modes
+// accept the same primitives below that bound and occluded == (closest id >= 0 && closest t < tmax) exactly: the padded
+// boxes never cull an accepted hit (§4 of DESIGN.md), and a box holding a hit at t < tmax still passes with its far bound
+// lowered to tmax.  (Once a ray accepts, best < tmax, but the ray has ended and tests no further box.)
+enum TraceMode { kClosest, kClosestSorted, kAnyHit };
+
 // Persistent traversal with per-lane dynamic ray fetch (after Aila & Laine, "Understanding the Efficiency of
 // Ray Traversal on GPUs", HPG 2009).  The reference walks its threaded tree one thread per pixel (hit(),
 // kernel.cu:468-512); incoherent bounces then leave most lanes of a warp idle while the longest ray
@@ -231,15 +242,13 @@ constexpr int kSentinel = (int)0x80000000;     // bottom of every traversal stac
 // the idle lanes claim fresh rays from the queue with ONE atomic per warp (ballot + popc + shfl), so warps
 // stay populated until the queue runs dry.  (A while-while variant measured slower on B200: with
 // one-primitive leaves, lanes that reach a leaf wait for the slowest descent.)
-#ifndef DRB_TRACE_MIN_BLOCKS
-#define DRB_TRACE_MIN_BLOCKS 8
-#endif
-template <bool kSortedPush>
-__global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(DevScene sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
-                                               uint2* __restrict__ hit, uint32_t* counters, int cur, int refill, int leaf_batch, int step_min,
-                                               const uint32_t* __restrict__ order)
+// Traces the first `count` rays of ro / rdv, handed out in the order `order` gives (nullptr: queue order); the result of a
+// ray goes to hit (closest) or occluded (any hit) at its queue position.
+template <TraceMode kMode>
+DRB_D void traverse(const DevScene& sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
+                    uint2* __restrict__ hit, uint8_t* __restrict__ occluded, uint32_t* counters, uint32_t count,
+                    int refill, int leaf_batch, int step_min, const uint32_t* __restrict__ order)
 {
-    const uint32_t count = counters[cur];
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
 
@@ -277,8 +286,12 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
                 if (k < count) {
                     const uint32_t i = order ? order[k] : k;        // queue position of the k-th ray in traversal order
                     const float4 o4 = ro[i], d4 = rdv[i];
-                    if (__float_as_uint(o4.w) == kInvalidPid || sc.nprims == 0) {
-                        hit[i] = make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
+                    bool skip;                                      // the ray has no result to search for
+                    if constexpr (kMode == kAnyHit) skip = !(d4.w > 0.0f);    // nothing is accepted at t < tmax <= 0 (t > 1e-4 / t > 0)
+                    else skip = __float_as_uint(o4.w) == kInvalidPid;
+                    if (skip || sc.nprims == 0) {
+                        if constexpr (kMode == kAnyHit) occluded[i] = 0;
+                        else hit[i] = make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
                     } else {
                         ray = i;
                         o = xyz(o4); d = xyz(d4);
@@ -301,7 +314,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
                         czz = make_float2(fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z - pz) * iz), fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z + pz) * iz));
                         snx = ix >= 0.f ? 0x7410u : 0x7432u; sny = iy >= 0.f ? 0x7410u : 0x7432u; snz = iz >= 0.f ? 0x7410u : 0x7432u;
                         sfx = snx ^ 0x22u; sfy = sny ^ 0x22u; sfz = snz ^ 0x22u;
-                        best = kTMax; bestp = -1;
+                        best = kMode == kAnyHit ? d4.w : kTMax; bestp = -1;
                         sp = s_stack + threadIdx.x; DRB_PUSH(kSentinel);
                         node = 0;
                     }
@@ -330,7 +343,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
 #undef DRB_CHILD
 #undef DRB_PLANES
             // t_near >= 0, so its bits order like unsigned integers; the two low bits carry the slot
-            if constexpr (kSortedPush) {
+            if constexpr (kMode == kClosestSorted) {
             // sort the four keys (5 compare-exchanges), push the hits far-to-near, continue with the nearest
             uint32_t a0 = min(k0, k1), a1 = max(k0, k1), a2 = min(k2, k3), a3 = max(k2, k3);
             const uint32_t s0 = min(a0, a2), t1 = max(a0, a2), t2 = min(a1, a3), s3 = max(a1, a3);
@@ -363,17 +376,24 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
         }
         // ---- postponed leaves -------------------------------------------------------------------------
         // The (long, divergent) primitive test runs for the whole warp at once when enough lanes hold a stashed
-        // leaf, or when too few lanes can still step.
+        // leaf, or when too few lanes can still step.  (Testing each leaf as soon as a lane reaches it is slower, for
+        // any hit as well: DESIGN.md §5.)
         const unsigned mpend = __ballot_sync(0xffffffffu, leaf != 0);
         if (mpend) {
             const unsigned mstep = __ballot_sync(0xffffffffu, node >= 0);
             if (__popc(mpend) >= leaf_batch || __popc(mstep) < step_min) {
-                if (leaf != 0) { intersect_prim(sc.prims, ~leaf, o, d, best, bestp); leaf = 0; }
+                if (leaf != 0) {
+                    intersect_prim(sc.prims, ~leaf, o, d, best, bestp); leaf = 0;
+                    if constexpr (kMode == kAnyHit) {
+                        if (bestp >= 0) node = kSentinel;           // an accepted primitive ends the ray, whatever the lane holds next
+                    }
+                }
             }
         }
         // ---- retire -----------------------------------------------------------------------------------
         if (node == kSentinel && leaf == 0 && ray != 0xFFFFFFFFu) {
-            hit[ray] = bestp >= 0 ? make_uint2(__float_as_uint(best), (uint32_t)bestp) : make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
+            if constexpr (kMode == kAnyHit) occluded[ray] = bestp >= 0 ? 1 : 0;
+            else hit[ray] = bestp >= 0 ? make_uint2(__float_as_uint(best), (uint32_t)bestp) : make_uint2(__float_as_uint(-1.0f), 0xFFFFFFFFu);
             ray = 0xFFFFFFFFu;
         }
     }
@@ -381,143 +401,24 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(D
 #undef DRB_POP
 }
 
-// ---- any hit ---------------------------------------------------------------------------------------
-// Occlusion query: does hit()'s test accept some primitive at t < tmax?  The traversal of k_trace<false> (persistent warps
-// with per-lane refill, packed slab test, shared-memory stack, nearest child next, the other hits pushed) with three
-// changes: the far bound of the slab test is the ray's own tmax for the whole ray (there is no shrinking `best`), the first
-// accepted primitive ends the ray, and the answer is one byte.  The primitive test is intersect_prim itself started from
-// best = tmax, so the two kernels accept the same primitives below that bound and occluded == (closest id >= 0 && closest
-// t < tmax) exactly: the padded boxes never cull an accepted hit (§4 of DESIGN.md), and a box holding a hit at t < tmax
-// still passes with its far bound lowered to tmax.  tmax (already clamped to 10000, > 0) rides in the w component of the
-// direction stream.
-// Leaves: with DRB_OCCLUDED_LEAF_NOW a lane tests each leaf as soon as it reaches it; by default it stashes the leaf and
-// the warp tests stashed leaves together, as k_trace does (DESIGN.md §5 has both measured).
-#ifndef DRB_OCCLUDED_LEAF_NOW
-#define DRB_OCCLUDED_LEAF_NOW 0
+#ifndef DRB_TRACE_MIN_BLOCKS
+#define DRB_TRACE_MIN_BLOCKS 8
 #endif
+// closest hit of the rays of queue `cur`
+template <bool kSortedPush>
+__global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(DevScene sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
+                                               uint2* __restrict__ hit, uint32_t* counters, int cur, int refill, int leaf_batch, int step_min,
+                                               const uint32_t* __restrict__ order)
+{
+    traverse<kSortedPush ? kClosestSorted : kClosest>(sc, scene_scale, ro, rdv, hit, nullptr, counters, counters[cur], refill, leaf_batch, step_min, order);
+}
+
+// any hit of a query chunk (ray count in counters[0])
 __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_occluded(DevScene sc, float scene_scale, const float4* __restrict__ ro,
                                                                                  const float4* __restrict__ rdv, uint8_t* __restrict__ occluded,
                                                                                  uint32_t* counters, int refill, int leaf_batch, int step_min)
 {
-    const uint32_t count = counters[0];
-    const unsigned lane = threadIdx.x & 31u;
-    const unsigned lt_mask = (1u << lane) - 1u;
-
-    int node = kSentinel;
-    int leaf = 0;                                   // stashed leaf (~primitive slot, always < 0), 0 = none
-    uint32_t ray = 0xFFFFFFFFu;
-    bool exhausted = false;                         // warp-uniform: the queue has been handed out completely
-    bool hit_any = false;
-    f3 o = mk3(0.f), d = mk3(0.f);
-    float2 sxx = {}, syy = {}, szz = {}, cxx = {}, cyy = {}, czz = {};
-    uint32_t snx = 0x7410u, sny = 0x7410u, snz = 0x7410u, sfx = 0x7432u, sfy = 0x7432u, sfz = 0x7432u;
-    float tmax = 0.f;
-    extern __shared__ int s_stack[];
-    int* sp = s_stack + threadIdx.x;
-#define DRB_PUSH(v) do { *sp = (v); sp += 128; } while (0)
-#define DRB_POP() (sp -= 128, *sp)
-
-    for (;;) {
-        // ---- refill idle lanes (as k_trace) -----------------------------------------------------------
-        const bool idle = (node == kSentinel && leaf == 0);
-        const unsigned midle = __ballot_sync(0xffffffffu, idle);
-        if (midle == 0xffffffffu && exhausted) break;
-        if (!exhausted && (midle == 0xffffffffu || 32 - __popc(midle) < refill)) {
-            const int leader = __ffs(midle) - 1;
-            uint32_t base = 0;
-            if ((int)lane == leader) base = atomicAdd(&counters[CNT_TICKET], (uint32_t)__popc(midle));
-            base = __shfl_sync(0xffffffffu, base, leader);
-            if (base + (uint32_t)__popc(midle) >= count) exhausted = true;
-            if (idle) {
-                const uint32_t i = base + (uint32_t)__popc(midle & lt_mask);
-                if (i < count) {
-                    const float4 o4 = ro[i], d4 = rdv[i];
-                    if (!(d4.w > 0.0f) || sc.nprims == 0) {
-                        occluded[i] = 0;                    // nothing is accepted at t < tmax <= 0 (t > 1e-4 / t > 0)
-                    } else {
-                        ray = i;
-                        o = xyz(o4); d = xyz(d4);
-                        tmax = d4.w;
-                        hit_any = false;
-                        // the per-ray constants of k_trace, operation for operation
-                        const float ix = safe_inv(d.x), iy = safe_inv(d.y), iz = safe_inv(d.z);
-                        const float pad = fminf((fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fabsf(o.z)) + scene_scale) * 1.9073486e-6f, sc.pad_cap);
-                        const float sx = sc.qscale[0] * ix, sy = sc.qscale[1] * iy, sz = sc.qscale[2] * iz;
-                        const float px = copysignf(pad, ix), py = copysignf(pad, iy), pz = copysignf(pad, iz);
-                        sxx = make_float2(sx, sx); syy = make_float2(sy, sy); szz = make_float2(sz, sz);
-                        cxx = make_float2(fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x - px) * ix), fmaf(-8388608.0f, sx, (sc.qlo[0] - o.x + px) * ix));
-                        cyy = make_float2(fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y - py) * iy), fmaf(-8388608.0f, sy, (sc.qlo[1] - o.y + py) * iy));
-                        czz = make_float2(fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z - pz) * iz), fmaf(-8388608.0f, sz, (sc.qlo[2] - o.z + pz) * iz));
-                        snx = ix >= 0.f ? 0x7410u : 0x7432u; sny = iy >= 0.f ? 0x7410u : 0x7432u; snz = iz >= 0.f ? 0x7410u : 0x7432u;
-                        sfx = snx ^ 0x22u; sfy = sny ^ 0x22u; sfz = snz ^ 0x22u;
-                        sp = s_stack + threadIdx.x; DRB_PUSH(kSentinel);
-                        node = 0;
-                    }
-                }
-            }
-        }
-        // ---- kSteps descent steps per lane between warp votes ----------------------------------------------
-#pragma unroll
-        for (int step = 0; step < kSteps; ++step) {
-        if (node >= 0) {
-            const WideNode* np = sc.wnodes + node;
-            const f8 nA = ldg256(np->bx), nB = ldg256(np->bz);
-#define DRB_PLANES(w, sn, sf, s_, c_) __ffma2_rn(make_float2(prmt_exp23(__float_as_uint(w), (sn)), prmt_exp23(__float_as_uint(w), (sf))), (s_), (c_))
-#define DRB_CHILD(c, wx, wy, wz)                                                                                              \
-            const float2 x##c = DRB_PLANES(wx, snx, sfx, sxx, cxx), y##c = DRB_PLANES(wy, sny, sfy, syy, cyy), z##c = DRB_PLANES(wz, snz, sfz, szz, czz); \
-            const float tn##c = fmaxf(fmaxf(x##c.x, y##c.x), fmaxf(z##c.x, 0.0f));                                            \
-            const float tf##c = fminf(fminf(x##c.y, y##c.y), fminf(z##c.y, tmax));                                            \
-            const uint32_t k##c = (tn##c <= tf##c) ? ((__float_as_uint(tn##c) & 0xFFFFFFFCu) | c##u) : 0xFFFFFFFFu;
-            DRB_CHILD(0, nA.lo.x, nA.hi.x, nB.lo.x)
-            DRB_CHILD(1, nA.lo.y, nA.hi.y, nB.lo.y)
-            DRB_CHILD(2, nA.lo.z, nA.hi.z, nB.lo.z)
-            DRB_CHILD(3, nA.lo.w, nA.hi.w, nB.lo.w)
-#undef DRB_CHILD
-#undef DRB_PLANES
-            const uint32_t kmin = min(min(k0, k1), min(k2, k3));
-            if (kmin == 0xFFFFFFFFu) node = DRB_POP();
-            else {
-                const int c0 = __float_as_int(nB.hi.x), c1 = __float_as_int(nB.hi.y), c2 = __float_as_int(nB.hi.z), c3 = __float_as_int(nB.hi.w);
-                if (k3 != kmin && k3 != 0xFFFFFFFFu) DRB_PUSH(c3);
-                if (k2 != kmin && k2 != 0xFFFFFFFFu) DRB_PUSH(c2);
-                if (k1 != kmin && k1 != 0xFFFFFFFFu) DRB_PUSH(c1);
-                if (k0 != kmin && k0 != 0xFFFFFFFFu) DRB_PUSH(c0);
-                node = (kmin & 2u) ? ((kmin & 1u) ? c3 : c2) : ((kmin & 1u) ? c1 : c0);
-            }
-        }
-#if DRB_OCCLUDED_LEAF_NOW
-        if (node < 0 && node != kSentinel) {
-            float b = tmax; int bp = -1;
-            intersect_prim(sc.prims, ~node, o, d, b, bp);
-            if (bp >= 0) { hit_any = true; node = kSentinel; } else node = DRB_POP();
-        }
-#else
-        if (node < 0 && node != kSentinel && leaf == 0) { leaf = node; node = DRB_POP(); }
-#endif
-        }
-#if !DRB_OCCLUDED_LEAF_NOW
-        // ---- postponed leaves: an accepted primitive ends the ray, whatever the lane holds next -------------
-        const unsigned mpend = __ballot_sync(0xffffffffu, leaf != 0);
-        if (mpend) {
-            const unsigned mstep = __ballot_sync(0xffffffffu, node >= 0);
-            if (__popc(mpend) >= leaf_batch || __popc(mstep) < step_min) {
-                if (leaf != 0) {
-                    float b = tmax; int bp = -1;
-                    intersect_prim(sc.prims, ~leaf, o, d, b, bp);
-                    leaf = 0;
-                    if (bp >= 0) { hit_any = true; node = kSentinel; }
-                }
-            }
-        }
-#endif
-        // ---- retire -----------------------------------------------------------------------------------
-        if (node == kSentinel && leaf == 0 && ray != 0xFFFFFFFFu) {
-            occluded[ray] = hit_any ? 1 : 0;
-            ray = 0xFFFFFFFFu;
-        }
-    }
-#undef DRB_PUSH
-#undef DRB_POP
+    traverse<kAnyHit>(sc, scene_scale, ro, rdv, nullptr, occluded, counters, counters[0], refill, leaf_batch, step_min, nullptr);
 }
 
 // ---- shading ---------------------------------------------------------------------------------------
@@ -953,23 +854,6 @@ __global__ void __launch_bounds__(256) k_resolve(FrameParams fp, const float4* _
     dst[0] = sum.x; dst[1] = sum.y; dst[2] = sum.z;
 }
 
-// rays of explicit (o, d) arrays -> queue 0
-__global__ void k_load_rays(const float* __restrict__ o3, const float* __restrict__ d3, uint32_t n, Queues q)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    q.ray_o[0][i] = make_float4(o3[3*i], o3[3*i+1], o3[3*i+2], __uint_as_float(i));
-    q.ray_d[0][i] = make_float4(d3[3*i], d3[3*i+1], d3[3*i+2], 0.f);
-}
-__global__ void k_store_ids(const uint2* __restrict__ hit, const int32_t* __restrict__ orig, uint32_t n, int32_t* __restrict__ ids, float* __restrict__ t)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const uint2 h = hit[i];
-    const int p = (int)h.y;
-    ids[i] = p >= 0 ? orig[p] : -1;
-    t[i] = __uint_as_float(h.x);
-}
 // one chunk of a ray query: caller's float3 arrays -> query streams (index in chunk; tmax of an occlusion query in d.w,
 // clamped to hit()'s 10000 -- a NaN stays NaN and is never occluded)
 __global__ void __launch_bounds__(256) k_load_query(const float* __restrict__ o3, const float* __restrict__ d3, const float* __restrict__ tmax,
@@ -1066,7 +950,7 @@ struct RenderBuffers {
     size_t sort_tmp_bytes = 0;
 };
 
-// Scratch of the ray-query entry points (drb_trace_device, drb_occluded_device), apart from the render's queues: a query
+// Scratch of the ray-query entry points (drb_trace_ids, drb_trace_device, drb_occluded_device), apart from the render's queues: a query
 // never reallocates or overwrites what the next frame uses.  Sized to one chunk of rays (40 B each).
 struct QueryBuffers {
     size_t capacity = 0;                // rays per chunk
@@ -1127,54 +1011,46 @@ long g_sort_min = []() { const char* e = getenv("DOGERAY_B200_SORT_MIN"); return
 struct DeviceFacts {
     std::mutex mu;
     size_t total_mem[64] = { 0 };
-    int shade_blocks[64] = { 0 };
-    std::map<std::pair<int, size_t>, int> trace_blocks;        // (device, dynamic smem) -> grid
-    size_t max_smem_set[64] = { 0 };
-    std::map<std::pair<int, size_t>, int> occluded_blocks;     // the same for k_occluded
-    size_t occluded_smem_set[64] = { 0 };
+    std::map<std::tuple<const void*, int, size_t>, int> grid;   // (kernel, device, dynamic smem) -> grid
+    std::map<std::pair<const void*, int>, size_t> smem_set;     // (kernel, device) -> dynamic smem limit set so far
 } g_facts;
 
-int occluded_shape(int device, size_t smem, int* blocks)
+// SMs x resident blocks per SM of a persistent kernel launched with `threads` per block and `smem` bytes of dynamic shared
+// memory, whose limit is raised first when it lies below `smem`
+int resident_grid(const void* kernel, int threads, int device, size_t smem, int* blocks)
 {
     std::lock_guard<std::mutex> g(g_facts.mu);
-    const int d = device & 63;
-    auto it = g_facts.occluded_blocks.find({ device, smem });
-    if (it == g_facts.occluded_blocks.end()) {
+    auto it = g_facts.grid.find({ kernel, device, smem });
+    if (it == g_facts.grid.end()) {
         int sms = 148, per_sm = 1;
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        if (smem > g_facts.occluded_smem_set[d]) {
-            DRB_CUDA(cudaFuncSetAttribute(k_occluded, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            g_facts.occluded_smem_set[d] = smem;
+        size_t& set = g_facts.smem_set[{ kernel, device }];
+        if (smem > set) {
+            DRB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            set = smem;
         }
-        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_occluded, kTraceThreads, smem));
-        it = g_facts.occluded_blocks.emplace(std::make_pair(device, smem), sms * std::max(per_sm, 1)).first;
+        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+        it = g_facts.grid.emplace(std::make_tuple(kernel, device, smem), sms * std::max(per_sm, 1)).first;
     }
     *blocks = it->second;
     return DRB_OK;
 }
 
-int launch_shape(int device, size_t trace_smem, int* trace_blocks, int* shade_blocks)
+// one grid for k_trace whichever push order the scene uses: the smaller of the two instantiations' grids
+int trace_grid(int device, size_t smem, int* blocks)
 {
-    std::lock_guard<std::mutex> g(g_facts.mu);
-    const int d = device & 63;
-    auto it = g_facts.trace_blocks.find({ device, trace_smem });
-    if (it == g_facts.trace_blocks.end() || !g_facts.shade_blocks[d]) {
-        int sms = 148, per_sm = 1;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        if (trace_smem > g_facts.max_smem_set[d]) {
-            DRB_CUDA(cudaFuncSetAttribute(k_trace<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trace_smem));
-            DRB_CUDA(cudaFuncSetAttribute(k_trace<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trace_smem));
-            g_facts.max_smem_set[d] = trace_smem;
-        }
-        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_trace<false>, kTraceThreads, trace_smem));
-        { int other = per_sm; DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&other, k_trace<true>, kTraceThreads, trace_smem)); per_sm = std::min(per_sm, other); }
-        it = g_facts.trace_blocks.emplace(std::make_pair(device, trace_smem), sms * std::max(per_sm, 1)).first;
-        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_shade, 128, 0));
-        g_facts.shade_blocks[d] = sms * std::max(per_sm, 1);
-    }
-    *trace_blocks = it->second;
-    *shade_blocks = g_facts.shade_blocks[d];
+    int sorted = 0;
+    if (int rc = resident_grid((const void*)k_trace<false>, kTraceThreads, device, smem, blocks)) return rc;
+    if (int rc = resident_grid((const void*)k_trace<true>, kTraceThreads, device, smem, &sorted)) return rc;
+    *blocks = std::min(*blocks, sorted);
     return DRB_OK;
+}
+
+// dynamic shared memory of a traversal's stack: the exact bound the collapse computed (pushes along the worst root-to-leaf
+// chain + sentinel + 1), not 3 per level, for each of the block's lanes
+size_t trace_stack_bytes(const drb_scene* s)
+{
+    return (size_t)std::max(s->stack_levels, 3) * kTraceThreads * sizeof(int);
 }
 
 size_t device_total_mem(int device)
@@ -1220,9 +1096,9 @@ int ensure_buffers(drb_scene* s, size_t slots)
     DRB_CUDA(cudaMemsetAsync(q.counters, 0, CNT_WORDS * sizeof(uint32_t), st));
     DRB_CUDA(cudaStreamSynchronize(st));             // the buffers may be used from a caller-provided stream next
     rb->capacity = slots;
-    // the exact bound the collapse computed (pushes along the worst root-to-leaf chain + sentinel + 1), not 3 per level
-    rb->trace_smem = (size_t)std::max(s->stack_levels, 3) * kTraceThreads * sizeof(int);
-    return launch_shape(s->device, rb->trace_smem, &rb->trace_blocks, &rb->shade_blocks);
+    rb->trace_smem = trace_stack_bytes(s);
+    if (int rc = trace_grid(s->device, rb->trace_smem, &rb->trace_blocks)) return rc;
+    return resident_grid((const void*)k_shade, 128, s->device, 0, &rb->shade_blocks);
 }
 
 DevScene dev_scene(const drb_scene* s)
@@ -1289,10 +1165,9 @@ int ensure_query_buffers(drb_scene* s, size_t rays)
     DRB_CUDA(drb_dev_alloc((void**)&q.counters, CNT_WORDS * sizeof(uint32_t), st));
     DRB_CUDA(cudaMemsetAsync(q.counters, 0, CNT_WORDS * sizeof(uint32_t), st));
     DRB_CUDA(cudaStreamSynchronize(st));             // the buffers are used from the caller's stream next
-    qb->trace_smem = (size_t)std::max(s->stack_levels, 3) * kTraceThreads * sizeof(int);
-    int shade_blocks = 0;
-    if (int rc = launch_shape(s->device, qb->trace_smem, &qb->trace_blocks, &shade_blocks)) return rc;
-    if (int rc = occluded_shape(s->device, qb->trace_smem, &qb->occluded_blocks)) return rc;
+    qb->trace_smem = trace_stack_bytes(s);
+    if (int rc = trace_grid(s->device, qb->trace_smem, &qb->trace_blocks)) return rc;
+    if (int rc = resident_grid((const void*)k_occluded, kTraceThreads, s->device, qb->trace_smem, &qb->occluded_blocks)) return rc;
     qb->capacity = rays;
     return DRB_OK;
 }
@@ -1802,27 +1677,17 @@ int drb_trace_ids(drb_scene* s, const float* o3, const float* d3, int64_t n, int
     if (n == 0) return DRB_OK;
     if (n >= 0x7FFFFFF0ll) { drb_set_error("too many rays"); return DRB_ERR_ARG; }
     DRB_CUDA(cudaSetDevice(s->device));
-    if (int rc = ensure_buffers(s, (size_t)n)) return rc;
-    RenderBuffers* rb = s->rb;
-    Queues q = rb->q;
     cudaStream_t stream = s->stream;
     DevBuf b_o, b_d, b_t, b_ids;
     DRB_CUDA(b_o.alloc((size_t)n * 12, stream));
     DRB_CUDA(b_d.alloc((size_t)n * 12, stream));
-    DRB_CUDA(b_t.alloc((size_t)n * 4, stream));
     DRB_CUDA(b_ids.alloc((size_t)n * 4, stream));
-    float *d_o = b_o.as<float>(), *d_d = b_d.as<float>(), *d_t = b_t.as<float>();
-    int32_t* d_ids = b_ids.as<int32_t>();
-    DRB_CUDA(cudaMemcpyAsync(d_o, o3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
-    DRB_CUDA(cudaMemcpyAsync(d_d, d3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
-    const uint32_t nn = (uint32_t)n;
-    k_load_rays<<<(nn + 255) / 256, 256, 0, stream>>>(d_o, d_d, nn, q);
-    k_prepare<<<1, 32, 0, stream>>>(q.counters, -1, 0, nn);
-    launch_trace(s, rb->trace_blocks, rb->trace_smem, stream, dev_scene(s), scene_scale(s), q, 0, nullptr);
-    k_store_ids<<<(nn + 255) / 256, 256, 0, stream>>>(q.hit, s->orig_id, nn, d_ids, d_t);
-    DRB_CUDA(cudaGetLastError());
-    DRB_CUDA(cudaMemcpyAsync(ids, d_ids, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
-    if (t) DRB_CUDA(cudaMemcpyAsync(t, d_t, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+    if (t) DRB_CUDA(b_t.alloc((size_t)n * 4, stream));
+    DRB_CUDA(cudaMemcpyAsync(b_o.p, o3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
+    DRB_CUDA(cudaMemcpyAsync(b_d.p, d3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
+    if (int rc = run_query(s, b_o.as<float>(), b_d.as<float>(), nullptr, n, b_ids.as<int32_t>(), b_t.as<float>(), nullptr, nullptr, nullptr)) return rc;
+    DRB_CUDA(cudaMemcpyAsync(ids, b_ids.p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+    if (t) DRB_CUDA(cudaMemcpyAsync(t, b_t.p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
     DRB_CUDA(cudaStreamSynchronize(stream));
     return DRB_OK;
 }

@@ -267,7 +267,10 @@ int drb_render_multi_times(float* ms, int n);
 int drb_frame_i3(drb_scene* s, const drb_settings* settings, const drb_opts* opts, int divisor, int32_t* out);
 
 /* Closest-hit object ids (index of the object line, -1 = miss) and distances for explicit rays:
- * the same query as hit() (kernel.cu:468-512).  o3/d3: n*3 floats on the host. */
+ * the same query as hit() (kernel.cu:468-512).  o3/d3: n*3 floats on the host.  Runs drb_trace_device's query on the
+ * scene's own stream and returns when the results are in ids / t.  It uses the same query buffers as drb_trace_device and
+ * drb_occluded_device (below), so it shares their rule: one call at a time per handle.  A device query enqueued on another
+ * stream must have finished before this call. */
 int drb_trace_ids(drb_scene* s, const float* o3, const float* d3, int64_t n, int32_t* ids, float* t);
 
 /* ---- ray queries on device arrays ----------------------------------------------------------
