@@ -2,9 +2,10 @@
 // `singleobject` (164 B, raygpu/kernel.cu:48-74) and `bvh` (56 B, kernel.cu:79-96) -- re-laid for
 // 128-bit loads.  See DESIGN.md "Data layout in HBM".
 #pragma once
-#include "dogeray_b200.h"
+#include "drb_internal.h"
 #include <cuda_runtime.h>
 #include <cstdint>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -82,52 +83,6 @@ struct DevTexture {
     int32_t w, h;
 };
 
-struct LbvhDebug {              // integer outputs of the build, kept for drb_scene_lbvh (DRB_BUILD_KEEP_DEBUG only)
-    uint64_t* keys = nullptr;   // n, sorted
-    int32_t* order = nullptr;   // n
-    int32_t* parent = nullptr;  // n-1
-    int32_t* left = nullptr;    // n-1
-    int32_t* right = nullptr;   // n-1
-    float4* node_min = nullptr; // n-1
-    float4* node_max = nullptr; // n-1
-};
-
-struct FinalTree {              // the hierarchy the nodes were emitted from (root = node 0), for drb_scene_tree (DRB_BUILD_KEEP_DEBUG only)
-    int32_t* left = nullptr;    // n-1
-    int32_t* right = nullptr;   // n-1
-    float4* node_min = nullptr; // n-1
-    float4* node_max = nullptr; // n-1
-};
-
-struct drb_scene {
-    int device = 0;
-    uint32_t build_flags = 0;
-    FinalTree tree;
-    drb_settings settings;
-    int64_t nobjects = 0;       // object lines
-    int64_t nprims = 0;         // renderable primitives (in the tree)
-    int64_t nnodes = 0;
-    WideNode* wnodes = nullptr; // the traversal structure
-    int64_t nwnodes = 0;
-    int wide_levels = 0;        // height of the wide tree (levels of the breadth-first collapse)
-    int* wide_level_start = nullptr; // first node of every level, wide_levels + 1 entries (the refit's bottom-up order)
-    uint32_t* refit_inv = nullptr;   // object line -> slot << 1 | sphere, or ~0u; made by the first refit
-    int stack_levels = 3;       // traversal stack entries a lane can need (exact bound from the collapse + sentinel + 1)
-    Prim* prims = nullptr;
-    ShadeRec* recs = nullptr;
-    int32_t* orig_id = nullptr; // prim slot -> object line index
-    DevTexture* textures = nullptr;
-    int ntextures = 0;
-    std::vector<void*> texture_storage;
-    LbvhDebug dbg;
-    drb_build_info info;
-    cudaStream_t stream = nullptr;
-    // render work buffers, grown on demand (render.cu)
-    struct RenderBuffers* rb = nullptr;
-    // ray-query scratch, separate from the render's queues (render.cu)
-    struct QueryBuffers* qb = nullptr;
-};
-
 #define DRB_CUDA(call)                                                                                     \
     do {                                                                                                   \
         cudaError_t e__ = (call);                                                                          \
@@ -137,16 +92,130 @@ struct drb_scene {
         }                                                                                                  \
     } while (0)
 
-void drb_render_buffers_free(drb_scene* s);
-void drb_query_buffers_free(drb_scene* s);
-// Lets kernels and copies running on device `accessor` address pool memory of device `owner` (NVLink peers); granted once
-// per pair and process.  False when the devices cannot reach each other.
-bool drb_peer_access(int owner, int accessor);
-
 // Device memory for scenes and render buffers.  Blocks come from the device's stream-ordered pool (release
 // threshold raised so nothing goes back to the driver) through an exact-size cache: a scene that is created,
 // rendered and freed every frame -- the reference's CudaStarter pattern, kernel.cu:2604-2665 -- finds every block
 // it needs in the cache and performs no allocator call at all.  Blocks must be idle (their stream synchronised)
-// when they are handed back.
+// when they are handed back.  Called only by DevArray and the cache itself.
 cudaError_t drb_dev_alloc(void** p, size_t bytes, cudaStream_t st);
 void drb_dev_free(void* p, cudaStream_t st);
+
+// The owner of one block of `count` T from the block cache, on the device that was current at alloc().  The block goes
+// back to that device's cache when the owner is reset or destroyed, freed on the stream it was allocated on, so that
+// stream must outlive the owner.  The owner does not synchronise: whoever holds it synchronises the stream (or the
+// device) first, so that the block is idle.
+template <typename T> class DevArray {
+public:
+    DevArray() = default;
+    DevArray(DevArray&& o) noexcept : p_(o.p_), dev_(o.dev_), st_(o.st_) { o.p_ = nullptr; }
+    DevArray& operator=(DevArray&& o) noexcept
+    {
+        if (this != &o) { reset(); p_ = o.p_; dev_ = o.dev_; st_ = o.st_; o.p_ = nullptr; }
+        return *this;
+    }
+    ~DevArray() { reset(); }
+
+    // releases the block held so far first; a count of 0 still yields a valid one-element block
+    int alloc(size_t count, cudaStream_t st)
+    {
+        reset();
+        void* p = nullptr;
+        DRB_CUDA(drb_dev_alloc(&p, (count ? count : 1) * sizeof(T), st));
+        cudaGetDevice(&dev_);
+        p_ = static_cast<T*>(p);
+        st_ = st;
+        return DRB_OK;
+    }
+    void reset()
+    {
+        if (!p_) return;
+        int cur = -1;
+        cudaGetDevice(&cur);
+        if (cur != dev_) cudaSetDevice(dev_);
+        drb_dev_free(p_, st_);
+        if (cur != dev_ && cur >= 0) cudaSetDevice(cur);
+        p_ = nullptr;
+    }
+    T* get() const { return p_; }
+    void* arg() { return &p_; }         // an entry of a kernel-argument array (cudaLaunchCooperativeKernel)
+
+private:
+    T* p_ = nullptr;
+    int dev_ = -1;
+    cudaStream_t st_ = nullptr;
+};
+
+// Synchronises a stream when it goes out of scope.  A call declares it after its scratch owners, so that it runs before
+// they hand their blocks back: an error can return while work is still queued on them.
+struct StreamDrain {
+    cudaStream_t st;
+    ~StreamDrain() { cudaStreamSynchronize(st); }
+};
+
+struct LbvhDebug {              // integer outputs of the build, kept for drb_scene_lbvh (DRB_BUILD_KEEP_DEBUG only)
+    DevArray<uint64_t> keys;    // n, sorted
+    DevArray<int32_t> order;    // n
+    DevArray<int32_t> parent;   // n-1
+    DevArray<int32_t> left;     // n-1
+    DevArray<int32_t> right;    // n-1
+    DevArray<float4> node_min;  // n-1
+    DevArray<float4> node_max;  // n-1
+};
+
+struct FinalTree {              // the hierarchy the nodes were emitted from (root = node 0), for drb_scene_tree (DRB_BUILD_KEEP_DEBUG only)
+    DevArray<int32_t> left;     // n-1
+    DevArray<int32_t> right;    // n-1
+    DevArray<float4> node_min;  // n-1
+    DevArray<float4> node_max;  // n-1
+};
+
+// the render's work buffers and the ray queries' scratch, defined in render.cu
+struct RenderBuffers;
+struct QueryBuffers;
+struct BuffersDelete {
+    void operator()(RenderBuffers* p) const;
+    void operator()(QueryBuffers* p) const;
+};
+
+// Every device array of a scene is owned by a member: deleting the scene (after a synchronisation, drb_scene_free)
+// returns them all.  `stream` is not owned here: the blocks are freed on it, so drb_scene_free destroys it last.
+struct drb_scene {
+    int device = 0;
+    uint32_t build_flags = 0;
+    FinalTree tree;
+    drb_settings settings;
+    int64_t nobjects = 0;       // object lines
+    int64_t nprims = 0;         // renderable primitives (in the tree)
+    int64_t nnodes = 0;
+    DevArray<WideNode> wnodes;  // the traversal structure
+    int64_t nwnodes = 0;
+    int wide_levels = 0;        // height of the wide tree (levels of the breadth-first collapse)
+    DevArray<int> wide_level_start;  // first node of every level, wide_levels + 1 entries (the refit's bottom-up order)
+    DevArray<uint32_t> refit_inv;    // object line -> slot << 1 | sphere, or ~0u; made by the first refit
+    int stack_levels = 3;       // traversal stack entries a lane can need (exact bound from the collapse + sentinel + 1)
+    DevArray<Prim> prims;
+    DevArray<ShadeRec> recs;
+    DevArray<int32_t> orig_id;  // prim slot -> object line index
+    DevArray<DevTexture> textures;
+    int ntextures = 0;
+    std::vector<DevArray<uint8_t>> texture_storage;
+    LbvhDebug dbg;
+    drb_build_info info;
+    cudaStream_t stream = nullptr;
+    // render work buffers, grown on demand (render.cu)
+    std::unique_ptr<RenderBuffers, BuffersDelete> rb;
+    // ray-query scratch, separate from the render's queues (render.cu)
+    std::unique_ptr<QueryBuffers, BuffersDelete> qb;
+};
+
+// Facts of a device, asked of the driver once per process and device (and kernel): each of these queries takes a
+// device-wide lock, and asked once per scene handle they stalled frames by tens of milliseconds whenever a monitoring
+// process polled the GPU (DESIGN.md section 8).  One cache under one mutex answers them all, for every host thread.
+// SMs of `device`, and resident blocks per SM of `kernel` at `threads` per block and `smem` bytes of dynamic shared memory
+// there (`device` current), whose limit is raised first when it lies below `smem`
+int drb_occupancy(const void* kernel, int threads, size_t smem, int device, int* sms, int* per_sm);
+// total memory of `device`, which must be current; 0 when it cannot be asked
+size_t drb_device_total_mem(int device);
+// Lets kernels and copies running on device `accessor` address pool memory of device `owner` (NVLink peers); granted once
+// per pair and process.  False when the devices cannot reach each other.
+bool drb_peer_access(int owner, int accessor);

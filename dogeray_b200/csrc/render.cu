@@ -34,10 +34,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <map>
-#include <mutex>
 #include <thread>
-#include <tuple>
 #include <vector>
 
 namespace {
@@ -940,24 +937,36 @@ __global__ void k_frame_i3(const float* __restrict__ accum, int w, int h, int fu
 // ---- host side ---------------------------------------------------------------------------------------
 struct RenderBuffers {
     size_t capacity = 0;                // path slots
-    Queues q{};
+    DevArray<float4> ray_o[2], ray_d[2], thr[2], contrib;
+    DevArray<uint2> hit;
+    DevArray<uint32_t> counters;
     int trace_blocks = 0, shade_blocks = 0;
     size_t trace_smem = 0;              // dynamic shared memory of k_trace: (tree height + 2) stack levels x 128 lanes
     // ray reordering (one sort per bounce): keys / ray indices, double-buffered, + CUB scratch
-    uint32_t* sort_keys[2] = { nullptr, nullptr };
-    uint32_t* sort_vals[2] = { nullptr, nullptr };
-    void* sort_tmp = nullptr;
+    DevArray<uint32_t> sort_keys[2], sort_vals[2];
+    DevArray<char> sort_tmp;
     size_t sort_tmp_bytes = 0;
+    Queues queues() const
+    {
+        return Queues{ { ray_o[0].get(), ray_o[1].get() }, { ray_d[0].get(), ray_d[1].get() }, { thr[0].get(), thr[1].get() }, hit.get(), contrib.get(),
+                       counters.get() };
+    }
 };
 
 // Scratch of the ray-query entry points (drb_trace_ids, drb_trace_device, drb_occluded_device), apart from the render's queues: a query
 // never reallocates or overwrites what the next frame uses.  Sized to one chunk of rays (40 B each).
 struct QueryBuffers {
     size_t capacity = 0;                // rays per chunk
-    Queues q{};                         // ray_o[0], ray_d[0], hit and counters only
+    DevArray<float4> ray_o, ray_d;
+    DevArray<uint2> hit;
+    DevArray<uint32_t> counters;
     int trace_blocks = 0, occluded_blocks = 0;
     size_t trace_smem = 0;              // stack of k_trace / k_occluded: (tree height + 2) levels x 128 lanes
+    Queues queues() const { return Queues{ { ray_o.get(), nullptr }, { ray_d.get(), nullptr }, {}, hit.get(), nullptr, counters.get() }; }
 };
+
+void BuffersDelete::operator()(RenderBuffers* p) const { delete p; }
+void BuffersDelete::operator()(QueryBuffers* p) const { delete p; }
 
 namespace {
 
@@ -1004,35 +1013,13 @@ Camera make_camera(const drb_settings& st, int W, int H, int divisor)
 // on B200 the sort costs more than the ~5 % of traversal time it saves on the 1 M-triangle workload)
 long g_sort_min = []() { const char* e = getenv("DOGERAY_B200_SORT_MIN"); return e ? atol(e) : 0L; }();
 
-// Grid sizes of the persistent kernels and the total device memory are properties of the device: they are asked
-// once per process and device (and per stack size), not once per scene handle.  Each of these driver calls takes a
-// device-wide lock; with a new handle every frame (the CudaStarter pattern) they were seen to stall a frame for
-// tens of milliseconds whenever a monitoring process polled the GPU at the same moment.
-struct DeviceFacts {
-    std::mutex mu;
-    size_t total_mem[64] = { 0 };
-    std::map<std::tuple<const void*, int, size_t>, int> grid;   // (kernel, device, dynamic smem) -> grid
-    std::map<std::pair<const void*, int>, size_t> smem_set;     // (kernel, device) -> dynamic smem limit set so far
-} g_facts;
-
 // SMs x resident blocks per SM of a persistent kernel launched with `threads` per block and `smem` bytes of dynamic shared
-// memory, whose limit is raised first when it lies below `smem`
+// memory (both asked once per process and device, drb_occupancy)
 int resident_grid(const void* kernel, int threads, int device, size_t smem, int* blocks)
 {
-    std::lock_guard<std::mutex> g(g_facts.mu);
-    auto it = g_facts.grid.find({ kernel, device, smem });
-    if (it == g_facts.grid.end()) {
-        int sms = 148, per_sm = 1;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        size_t& set = g_facts.smem_set[{ kernel, device }];
-        if (smem > set) {
-            DRB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            set = smem;
-        }
-        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-        it = g_facts.grid.emplace(std::make_tuple(kernel, device, smem), sms * std::max(per_sm, 1)).first;
-    }
-    *blocks = it->second;
+    int sms = 0, per_sm = 0;
+    if (int rc = drb_occupancy(kernel, threads, smem, device, &sms, &per_sm)) return rc;
+    *blocks = sms * std::max(per_sm, 1);
     return DRB_OK;
 }
 
@@ -1053,52 +1040,40 @@ size_t trace_stack_bytes(const drb_scene* s)
     return (size_t)std::max(s->stack_levels, 3) * kTraceThreads * sizeof(int);
 }
 
-size_t device_total_mem(int device)
-{
-    std::lock_guard<std::mutex> g(g_facts.mu);
-    size_t& t = g_facts.total_mem[device & 63];
-    if (!t) {
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) t = total_b; else cudaGetLastError();
-    }
-    return t;
-}
-
 int ensure_buffers(drb_scene* s, size_t slots)
 {
-    if (!s->rb) s->rb = new RenderBuffers();
-    RenderBuffers* rb = s->rb;
-    if (rb->capacity >= slots && rb->q.counters) return DRB_OK;
-    drb_render_buffers_free(s);
-    s->rb = rb = new RenderBuffers();
-    Queues& q = rb->q;
+    if (s->rb && s->rb->capacity >= slots) return DRB_OK;
+    cudaDeviceSynchronize();                         // renders may have run on caller streams
+    s->rb.reset(new RenderBuffers());                // the old buffers go back before the new ones are allocated
+    RenderBuffers& rb = *s->rb;
     cudaStream_t st = s->stream;
     for (int k = 0; k < 2; ++k) {
-        DRB_CUDA(drb_dev_alloc((void**)&q.ray_o[k], slots * sizeof(float4), st));
-        DRB_CUDA(drb_dev_alloc((void**)&q.ray_d[k], slots * sizeof(float4), st));
-        DRB_CUDA(drb_dev_alloc((void**)&q.thr[k], slots * sizeof(float4), st));
+        if (int rc = rb.ray_o[k].alloc(slots, st)) return rc;
+        if (int rc = rb.ray_d[k].alloc(slots, st)) return rc;
+        if (int rc = rb.thr[k].alloc(slots, st)) return rc;
     }
-    DRB_CUDA(drb_dev_alloc((void**)&q.hit, slots * sizeof(uint2), st));
-    DRB_CUDA(drb_dev_alloc((void**)&q.contrib, slots * sizeof(float4), st));
-    DRB_CUDA(drb_dev_alloc((void**)&q.counters, CNT_WORDS * sizeof(uint32_t), st));
+    if (int rc = rb.hit.alloc(slots, st)) return rc;
+    if (int rc = rb.contrib.alloc(slots, st)) return rc;
+    if (int rc = rb.counters.alloc(CNT_WORDS, st)) return rc;
     if (g_sort_min > 0) {                            // the opt-in ray reordering needs keys / indices / CUB scratch
         for (int k = 0; k < 2; ++k) {
-            DRB_CUDA(drb_dev_alloc((void**)&rb->sort_keys[k], slots * sizeof(uint32_t), st));
-            DRB_CUDA(drb_dev_alloc((void**)&rb->sort_vals[k], slots * sizeof(uint32_t), st));
+            if (int rc = rb.sort_keys[k].alloc(slots, st)) return rc;
+            if (int rc = rb.sort_vals[k].alloc(slots, st)) return rc;
         }
-        DRB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, rb->sort_tmp_bytes, rb->sort_keys[0], rb->sort_keys[1], rb->sort_vals[0], rb->sort_vals[1],
-                                                 (int)std::min<size_t>(slots, 0x7FFFFFFF), 0, 24, st));
-        DRB_CUDA(drb_dev_alloc(&rb->sort_tmp, rb->sort_tmp_bytes ? rb->sort_tmp_bytes : 16, st));
+        DRB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, rb.sort_tmp_bytes, rb.sort_keys[0].get(), rb.sort_keys[1].get(), rb.sort_vals[0].get(),
+                                                 rb.sort_vals[1].get(), (int)std::min<size_t>(slots, 0x7FFFFFFF), 0, 24, st));
+        if (int rc = rb.sort_tmp.alloc(rb.sort_tmp_bytes ? rb.sort_tmp_bytes : 16, st)) return rc;
     }
+    const Queues q = rb.queues();
     if (getenv("DOGERAY_B200_DEBUG"))
         fprintf(stderr, "[dogeray_b200] queues for %zu slots: o %p %p d %p %p thr %p %p hit %p contrib %p\n", slots, (void*)q.ray_o[0], (void*)q.ray_o[1],
                 (void*)q.ray_d[0], (void*)q.ray_d[1], (void*)q.thr[0], (void*)q.thr[1], (void*)q.hit, (void*)q.contrib);
     DRB_CUDA(cudaMemsetAsync(q.counters, 0, CNT_WORDS * sizeof(uint32_t), st));
     DRB_CUDA(cudaStreamSynchronize(st));             // the buffers may be used from a caller-provided stream next
-    rb->capacity = slots;
-    rb->trace_smem = trace_stack_bytes(s);
-    if (int rc = trace_grid(s->device, rb->trace_smem, &rb->trace_blocks)) return rc;
-    return resident_grid((const void*)k_shade, 128, s->device, 0, &rb->shade_blocks);
+    rb.capacity = slots;
+    rb.trace_smem = trace_stack_bytes(s);
+    if (int rc = trace_grid(s->device, rb.trace_smem, &rb.trace_blocks)) return rc;
+    return resident_grid((const void*)k_shade, 128, s->device, 0, &rb.shade_blocks);
 }
 
 DevScene dev_scene(const drb_scene* s)
@@ -1106,7 +1081,7 @@ DevScene dev_scene(const drb_scene* s)
     DevScene d;
     for (int a = 0; a < 3; ++a) drb_quant_grid(s->info.bounds_min[a], s->info.bounds_max[a], &d.qlo[a], &d.qscale[a]);
     d.pad_cap = 0.49f * 65527.0f * std::max(d.qscale[0], std::max(d.qscale[1], d.qscale[2]));
-    d.wnodes = s->wnodes; d.prims = s->prims; d.recs = s->recs; d.textures = s->textures;
+    d.wnodes = s->wnodes.get(); d.prims = s->prims.get(); d.recs = s->recs.get(); d.textures = s->textures.get();
     d.nprims = (int)s->nprims; d.ntextures = s->ntextures;
     return d;
 }
@@ -1154,16 +1129,15 @@ size_t g_query_chunk = []() { const char* e = getenv("DOGERAY_B200_QUERY_CHUNK")
 int ensure_query_buffers(drb_scene* s, size_t rays)
 {
     if (s->qb && s->qb->capacity >= rays) return DRB_OK;
-    drb_query_buffers_free(s);
-    s->qb = new QueryBuffers();
-    QueryBuffers* qb = s->qb;
-    Queues& q = qb->q;
+    if (s->qb) cudaDeviceSynchronize();              // queries run on caller streams
+    s->qb.reset(new QueryBuffers());                 // the old scratch goes back before the new one is allocated
+    QueryBuffers* qb = s->qb.get();
     cudaStream_t st = s->stream;
-    DRB_CUDA(drb_dev_alloc((void**)&q.ray_o[0], rays * sizeof(float4), st));
-    DRB_CUDA(drb_dev_alloc((void**)&q.ray_d[0], rays * sizeof(float4), st));
-    DRB_CUDA(drb_dev_alloc((void**)&q.hit, rays * sizeof(uint2), st));
-    DRB_CUDA(drb_dev_alloc((void**)&q.counters, CNT_WORDS * sizeof(uint32_t), st));
-    DRB_CUDA(cudaMemsetAsync(q.counters, 0, CNT_WORDS * sizeof(uint32_t), st));
+    if (int rc = qb->ray_o.alloc(rays, st)) return rc;
+    if (int rc = qb->ray_d.alloc(rays, st)) return rc;
+    if (int rc = qb->hit.alloc(rays, st)) return rc;
+    if (int rc = qb->counters.alloc(CNT_WORDS, st)) return rc;
+    DRB_CUDA(cudaMemsetAsync(qb->counters.get(), 0, CNT_WORDS * sizeof(uint32_t), st));
     DRB_CUDA(cudaStreamSynchronize(st));             // the buffers are used from the caller's stream next
     qb->trace_smem = trace_stack_bytes(s);
     if (int rc = trace_grid(s->device, qb->trace_smem, &qb->trace_blocks)) return rc;
@@ -1180,8 +1154,8 @@ int run_query(drb_scene* s, const float* o3, const float* d3, const float* tmax,
     DRB_CUDA(cudaSetDevice(s->device));
     const size_t chunk = std::min<size_t>((size_t)n, g_query_chunk);
     if (int rc = ensure_query_buffers(s, chunk)) return rc;
-    const QueryBuffers* qb = s->qb;
-    const Queues& q = qb->q;
+    const QueryBuffers* qb = s->qb.get();
+    const Queues q = qb->queues();
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     const DevScene sc = dev_scene(s);
     const float scale = scene_scale(s);
@@ -1196,7 +1170,7 @@ int run_query(drb_scene* s, const float* o3, const float* d3, const float* tmax,
                                                                                   g_refill, g_leaf_batch, g_step_min);
         } else {
             launch_trace(s, qb->trace_blocks, qb->trace_smem, st, sc, scale, q, 0, nullptr);
-            k_store_query<<<grid, 256, 0, st>>>(s->prims, q.ray_o[0], q.ray_d[0], q.hit, s->orig_id, m, ids + done, t ? t + done : nullptr,
+            k_store_query<<<grid, 256, 0, st>>>(s->prims.get(), q.ray_o[0], q.ray_d[0], q.hit, s->orig_id.get(), m, ids + done, t ? t + done : nullptr,
                                                 uv ? uv + 2 * done : nullptr);
         }
     }
@@ -1205,27 +1179,6 @@ int run_query(drb_scene* s, const float* o3, const float* d3, const float* tmax,
 }
 
 
-
-// device scratch that returns to the block cache when it goes out of scope, after its stream has drained
-struct DevBuf {
-    void* p = nullptr;
-    cudaStream_t st = nullptr;
-    int dev = -1;                       // the block cache is per device: the block goes back with its own device current
-    DevBuf() = default;
-    DevBuf(const DevBuf&) = delete;
-    DevBuf& operator=(const DevBuf&) = delete;
-    ~DevBuf()
-    {
-        if (!p) return;
-        int cur = -1;
-        cudaGetDevice(&cur);
-        if (cur != dev) cudaSetDevice(dev);
-        cudaStreamSynchronize(st); drb_dev_free(p, st);
-        if (cur != dev && cur >= 0) cudaSetDevice(cur);
-    }
-    cudaError_t alloc(size_t bytes, cudaStream_t s) { st = s; cudaGetDevice(&dev); return drb_dev_alloc(&p, bytes, s); }
-    template <typename T> T* as() const { return static_cast<T*>(p); }
-};
 
 struct EventPool {
     std::vector<cudaEvent_t> ev;
@@ -1257,7 +1210,7 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
     size_t want = o.batch_paths;
     if (!want) {
         want = (size_t)128 << 20;
-        const size_t device_mem = device_total_mem(s->device);
+        const size_t device_mem = drb_device_total_mem(s->device);
         if (device_mem) want = std::max<size_t>((size_t)(0.40 * (double)device_mem) / 120, (size_t)1 << 20);
     }
     uint32_t per_batch = 1;
@@ -1275,8 +1228,8 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
         cudaGetLastError();                              // out of memory: try half the batch
         want = slots_per_sample * (size_t)(per_batch / 2);
     }
-    RenderBuffers* rb = s->rb;
-    Queues q = rb->q;
+    const RenderBuffers* rb = s->rb.get();
+    const Queues q = rb->queues();
 
     FrameParams fp;
     fp.W = W; fp.H = H; fp.tiles_x = tiles_x; fp.tiles_y = tiles_y; fp.tile_rank = tile_rank; fp.tile_count = tile_count;
@@ -1330,11 +1283,12 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
                     const float3 lo = make_float3(s->info.bounds_min[0], s->info.bounds_min[1], s->info.bounds_min[2]);
                     auto inv = [&](int a) { const float e = s->info.bounds_max[a] - s->info.bounds_min[a]; return e > 0.f ? 1.0f / e : 0.f; };
                     k_ray_keys<<<(live + 255) / 256, 256, 0, stream>>>(q.ray_o[cur], q.ray_d[cur], live, lo, make_float3(inv(0), inv(1), inv(2)),
-                                                                       rb->sort_keys[0], rb->sort_vals[0]);
+                                                                       rb->sort_keys[0].get(), rb->sort_vals[0].get());
                     size_t tb = rb->sort_tmp_bytes;
-                    DRB_CUDA(cub::DeviceRadixSort::SortPairs(rb->sort_tmp, tb, rb->sort_keys[0], rb->sort_keys[1], rb->sort_vals[0], rb->sort_vals[1],
+                    DRB_CUDA(cub::DeviceRadixSort::SortPairs(rb->sort_tmp.get(), tb, rb->sort_keys[0].get(), rb->sort_keys[1].get(), rb->sort_vals[0].get(),
+                                                             rb->sort_vals[1].get(),
                                                              (int)live, 0, 24, stream));
-                    order = rb->sort_vals[1];
+                    order = rb->sort_vals[1].get();
                     launches += 4;
                 }
             }
@@ -1387,31 +1341,6 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
 
 } // namespace
 
-void drb_render_buffers_free(drb_scene* s)
-{
-    if (!s || !s->rb) return;
-    Queues& q = s->rb->q;
-    cudaStream_t st = s->stream;
-    cudaDeviceSynchronize();                          // renders may have run on caller streams
-    for (int k = 0; k < 2; ++k) { drb_dev_free(q.ray_o[k], st); drb_dev_free(q.ray_d[k], st); drb_dev_free(q.thr[k], st); }
-    drb_dev_free(q.hit, st); drb_dev_free(q.contrib, st); drb_dev_free(q.counters, st);
-    for (int k = 0; k < 2; ++k) { drb_dev_free(s->rb->sort_keys[k], st); drb_dev_free(s->rb->sort_vals[k], st); }
-    drb_dev_free(s->rb->sort_tmp, st);
-    delete s->rb;
-    s->rb = nullptr;
-}
-
-void drb_query_buffers_free(drb_scene* s)
-{
-    if (!s || !s->qb) return;
-    Queues& q = s->qb->q;
-    cudaStream_t st = s->stream;
-    cudaDeviceSynchronize();                          // queries run on caller streams
-    drb_dev_free(q.ray_o[0], st); drb_dev_free(q.ray_d[0], st); drb_dev_free(q.hit, st); drb_dev_free(q.counters, st);
-    delete s->qb;
-    s->qb = nullptr;
-}
-
 extern "C" {
 
 void drb_opts_default(drb_opts* o)
@@ -1435,9 +1364,10 @@ int drb_render(drb_scene* s, const drb_settings* settings, const drb_opts* opts,
     const size_t n = (size_t)settings->width * settings->height * 3;
     drb_opts o; if (opts) o = *opts; else drb_opts_default(&o);
     cudaStream_t stream = o.stream ? (cudaStream_t)o.stream : s->stream;
-    DevBuf buf;
-    DRB_CUDA(buf.alloc(n * sizeof(float), stream));
-    float* d = buf.as<float>();
+    DevArray<float> buf;
+    StreamDrain drain{ stream };                     // the image goes back to the cache idle, also when the render fails part-way
+    if (int rc = buf.alloc(n, stream)) return rc;
+    float* d = buf.get();
     // accumulate adds to the caller's values; with tile sharding the pixels of other shards must come back as they were
     if ((o.flags & DRB_FLAG_ACCUMULATE) || o.tile_count > 1) DRB_CUDA(cudaMemcpyAsync(d, accum_host, n * sizeof(float), cudaMemcpyHostToDevice, stream));
     if (int rc = render_core(s, settings, &o, settings->width, settings->height, 1, d, stats)) return rc;
@@ -1563,16 +1493,16 @@ extern "C" int drb_render_multi(drb_scene* const* scenes, int nscenes, const drb
         return rc;
     }
     DRB_CUDA(cudaSetDevice(dev0));
-    DevBuf image;                                           // THE image, on the first handle's device
-    DRB_CUDA(image.alloc(n * sizeof(float), first->stream));
-    float* d_image = image.as<float>();
+    DevArray<float> image;                                  // THE image, on the first handle's device
+    if (int rc = image.alloc(n, first->stream)) return rc;
+    float* d_image = image.get();
     const bool accumulate = (base.flags & DRB_FLAG_ACCUMULATE) != 0;
     if (accumulate) DRB_CUDA(cudaMemcpyAsync(d_image, accum_host, n * sizeof(float), cudaMemcpyHostToDevice, first->stream));
     DRB_CUDA(cudaStreamSynchronize(first->stream));        // the other devices' streams may touch it from here on
 
     std::vector<int> rcs((size_t)nscenes, DRB_OK);
     std::vector<std::string> errs((size_t)nscenes);
-    std::vector<DevBuf> parts((size_t)(by_samples ? nscenes : 0));
+    std::vector<DevArray<float>> parts((size_t)(by_samples ? nscenes : 0));
     std::atomic<uint32_t> next_shard{ 0 };
     const uint32_t nshards = dynamic ? 4u * (uint32_t)nscenes : (uint32_t)nscenes;
     const uint32_t total_samples = requested_samples(base, *settings);
@@ -1589,8 +1519,8 @@ extern "C" int drb_render_multi(drb_scene* const* scenes, int nscenes, const drb
             o.sample_count = q + ((uint32_t)k < r ? 1u : 0u);
             o.flags = (o.flags & ~DRB_FLAG_ACCUMULATE) | DRB_FLAG_EXACT_SAMPLES;
             o.tile_rank = 0; o.tile_count = 1;
-            if (parts[(size_t)k].alloc(n * sizeof(float), sc->stream) != cudaSuccess) { drb_set_error("out of device memory for a sample shard"); return fail(k, DRB_ERR_NOMEM); }
-            if (int rc = render_core(sc, settings, &o, W, H, 1, parts[(size_t)k].as<float>(), &sts[(size_t)k])) return fail(k, rc);
+            if (parts[(size_t)k].alloc(n, sc->stream) != DRB_OK) { drb_set_error("out of device memory for a sample shard"); return fail(k, DRB_ERR_NOMEM); }
+            if (int rc = render_core(sc, settings, &o, W, H, 1, parts[(size_t)k].get(), &sts[(size_t)k])) return fail(k, rc);
             return;
         }
         // tiles: claim shards (static: exactly shard k) and resolve them straight into the image on dev0
@@ -1610,13 +1540,16 @@ extern "C" int drb_render_multi(drb_scene* const* scenes, int nscenes, const drb
         work(0);
         for (auto& th : pool) th.join();
     }
+    // the image and the parts go back to the cache idle, also when a handle failed part-way
+    for (int k = 0; k < nscenes; ++k)
+        if (cudaSetDevice(scenes[k]->device) == cudaSuccess) cudaStreamSynchronize(scenes[k]->stream);
     for (int k = 0; k < nscenes; ++k)
         if (rcs[(size_t)k] != DRB_OK) { drb_set_error("drb_render_multi: scene %d: %s", k, errs[(size_t)k].c_str()); return rcs[(size_t)k]; }
     DRB_CUDA(cudaSetDevice(dev0));
     if (by_samples) {
         if (peers) {
             ShardParts sp;
-            for (int k = 0; k < nscenes; ++k) sp.p[k] = parts[(size_t)k].as<float>();
+            for (int k = 0; k < nscenes; ++k) sp.p[k] = parts[(size_t)k].get();
             k_sum_shards<<<(unsigned)((n + 255) / 256), 256, 0, first->stream>>>(d_image, sp, nscenes, n, accumulate ? 1 : 0);
             DRB_CUDA(cudaGetLastError());
             DRB_CUDA(cudaMemcpyAsync(accum_host, d_image, n * sizeof(float), cudaMemcpyDeviceToHost, first->stream));
@@ -1626,7 +1559,7 @@ extern "C" int drb_render_multi(drb_scene* const* scenes, int nscenes, const drb
             std::vector<float> tmp(n);
             for (int k = 0; k < nscenes; ++k) {
                 DRB_CUDA(cudaSetDevice(scenes[k]->device));
-                DRB_CUDA(cudaMemcpy(tmp.data(), parts[(size_t)k].as<float>(), n * sizeof(float), cudaMemcpyDeviceToHost));
+                DRB_CUDA(cudaMemcpy(tmp.data(), parts[(size_t)k].get(), n * sizeof(float), cudaMemcpyDeviceToHost));
                 if (k == 0 && !accumulate) memcpy(accum_host, tmp.data(), n * sizeof(float));
                 else for (size_t i = 0; i < n; ++i) accum_host[i] = accum_host[i] + tmp[i];
             }
@@ -1654,11 +1587,13 @@ int drb_frame_i3(drb_scene* s, const drb_settings* settings, const drb_opts* opt
     cudaStream_t stream = o.stream ? (cudaStream_t)o.stream : s->stream;
     const uint32_t spp = requested_samples(o, *settings);
     const size_t nfull = (size_t)settings->width * settings->height * 3;
-    DevBuf b_acc, b_out;
-    DRB_CUDA(b_acc.alloc((size_t)W * H * 3 * sizeof(float), stream));
-    DRB_CUDA(b_out.alloc(nfull * sizeof(int32_t), stream));
-    float* d_acc = b_acc.as<float>();
-    int32_t* d_out = b_out.as<int32_t>();
+    DevArray<float> b_acc;
+    DevArray<int32_t> b_out;
+    StreamDrain drain{ stream };
+    if (int rc = b_acc.alloc((size_t)W * H * 3, stream)) return rc;
+    if (int rc = b_out.alloc(nfull, stream)) return rc;
+    float* d_acc = b_acc.get();
+    int32_t* d_out = b_out.get();
     // entries outside the launched grid stay as the caller left them
     DRB_CUDA(cudaMemcpyAsync(d_out, out, nfull * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
     if (int rc = render_core(s, settings, &o, W, H, divisor, d_acc, nullptr)) return rc;
@@ -1678,16 +1613,18 @@ int drb_trace_ids(drb_scene* s, const float* o3, const float* d3, int64_t n, int
     if (n >= 0x7FFFFFF0ll) { drb_set_error("too many rays"); return DRB_ERR_ARG; }
     DRB_CUDA(cudaSetDevice(s->device));
     cudaStream_t stream = s->stream;
-    DevBuf b_o, b_d, b_t, b_ids;
-    DRB_CUDA(b_o.alloc((size_t)n * 12, stream));
-    DRB_CUDA(b_d.alloc((size_t)n * 12, stream));
-    DRB_CUDA(b_ids.alloc((size_t)n * 4, stream));
-    if (t) DRB_CUDA(b_t.alloc((size_t)n * 4, stream));
-    DRB_CUDA(cudaMemcpyAsync(b_o.p, o3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
-    DRB_CUDA(cudaMemcpyAsync(b_d.p, d3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
-    if (int rc = run_query(s, b_o.as<float>(), b_d.as<float>(), nullptr, n, b_ids.as<int32_t>(), b_t.as<float>(), nullptr, nullptr, nullptr)) return rc;
-    DRB_CUDA(cudaMemcpyAsync(ids, b_ids.p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
-    if (t) DRB_CUDA(cudaMemcpyAsync(t, b_t.p, (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+    DevArray<float> b_o, b_d, b_t;
+    DevArray<int32_t> b_ids;
+    StreamDrain drain{ stream };
+    if (int rc = b_o.alloc((size_t)n * 3, stream)) return rc;
+    if (int rc = b_d.alloc((size_t)n * 3, stream)) return rc;
+    if (int rc = b_ids.alloc((size_t)n, stream)) return rc;
+    if (t) { if (int rc = b_t.alloc((size_t)n, stream)) return rc; }
+    DRB_CUDA(cudaMemcpyAsync(b_o.get(), o3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
+    DRB_CUDA(cudaMemcpyAsync(b_d.get(), d3, (size_t)n * 12, cudaMemcpyHostToDevice, stream));
+    if (int rc = run_query(s, b_o.get(), b_d.get(), nullptr, n, b_ids.get(), b_t.get(), nullptr, nullptr, nullptr)) return rc;
+    DRB_CUDA(cudaMemcpyAsync(ids, b_ids.get(), (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
+    if (t) DRB_CUDA(cudaMemcpyAsync(t, b_t.get(), (size_t)n * 4, cudaMemcpyDeviceToHost, stream));
     DRB_CUDA(cudaStreamSynchronize(stream));
     return DRB_OK;
 }
@@ -1721,12 +1658,14 @@ int drb_primary_rays(drb_scene* s, const drb_settings* settings, const drb_opts*
     if (int rc = ensure_buffers(s, nslots)) return rc;
     cudaStream_t stream = s->stream;
     const size_t n = (size_t)W * H * 3;
-    DevBuf b_o, b_d;
-    DRB_CUDA(b_o.alloc(n * 4, stream));
-    DRB_CUDA(b_d.alloc(n * 4, stream));
-    float *d_o = b_o.as<float>(), *d_d = b_d.as<float>();
-    k_generate<<<(unsigned)((nslots + 255) / 256), 256, 0, stream>>>(fp, (uint32_t)nslots, s->rb->q);
-    k_store_rays<<<(unsigned)((nslots + 255) / 256), 256, 0, stream>>>(fp, (uint32_t)nslots, s->rb->q, d_o, d_d);
+    DevArray<float> b_o, b_d;
+    StreamDrain drain{ stream };
+    if (int rc = b_o.alloc(n, stream)) return rc;
+    if (int rc = b_d.alloc(n, stream)) return rc;
+    float *d_o = b_o.get(), *d_d = b_d.get();
+    const Queues q = s->rb->queues();
+    k_generate<<<(unsigned)((nslots + 255) / 256), 256, 0, stream>>>(fp, (uint32_t)nslots, q);
+    k_store_rays<<<(unsigned)((nslots + 255) / 256), 256, 0, stream>>>(fp, (uint32_t)nslots, q, d_o, d_d);
     DRB_CUDA(cudaGetLastError());
     DRB_CUDA(cudaMemcpyAsync(o3, d_o, n * 4, cudaMemcpyDeviceToHost, stream));
     DRB_CUDA(cudaMemcpyAsync(d3, d_d, n * 4, cudaMemcpyDeviceToHost, stream));

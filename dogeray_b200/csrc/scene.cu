@@ -23,8 +23,10 @@
 #include <algorithm>
 #include <chrono>
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <thread>
+#include <tuple>
 #include <unordered_map>
 
 namespace cg = cooperative_groups;
@@ -735,27 +737,6 @@ __global__ void __launch_bounds__(kBuildThreads) k_refit_wide(const int* __restr
     }
 }
 
-template <typename T> int dev_alloc(T** p, size_t count, cudaStream_t st)
-{
-    *p = nullptr;
-    if (count == 0) count = 1;
-    DRB_CUDA(drb_dev_alloc((void**)p, count * sizeof(T), st));
-    return DRB_OK;
-}
-
-struct Scratch {
-    cudaStream_t st;
-    std::vector<void*> ptrs;
-    explicit Scratch(cudaStream_t s) : st(s) {}
-    ~Scratch() { cudaStreamSynchronize(st); for (void* p : ptrs) drb_dev_free(p, st); }   // blocks must be idle when handed back
-    template <typename T> int alloc(T** p, size_t count)
-    {
-        int rc = dev_alloc(p, count, st);
-        if (rc == DRB_OK) ptrs.push_back(*p);
-        return rc;
-    }
-};
-
 } // namespace
 
 namespace {
@@ -826,15 +807,55 @@ void drb_dev_free(void* p, cudaStream_t st)
     cudaFreeAsync(p, st);
 }
 
+namespace {
+struct FactsCache {                     // the per-device facts of device_scene.cuh
+    std::mutex mu;
+    std::map<int, int> sms;
+    std::map<int, size_t> total_mem;
+    std::map<std::tuple<const void*, int, int, size_t>, int> per_sm;   // (kernel, device, threads, dynamic smem) -> blocks per SM
+    std::map<std::pair<const void*, int>, size_t> smem_set;          // (kernel, device) -> dynamic smem limit raised to so far
+    std::map<std::pair<int, int>, bool> peer;                          // (owner, accessor) -> usable
+} g_facts;
+}
+
+size_t drb_device_total_mem(int device)
+{
+    std::lock_guard<std::mutex> g(g_facts.mu);
+    size_t& t = g_facts.total_mem[device];
+    if (!t) {
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) t = total_b; else cudaGetLastError();
+    }
+    return t;
+}
+
+int drb_occupancy(const void* kernel, int threads, size_t smem, int device, int* sms, int* per_sm)
+{
+    std::lock_guard<std::mutex> g(g_facts.mu);
+    int& n = g_facts.sms[device];
+    if (!n) DRB_CUDA(cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, device));
+    auto it = g_facts.per_sm.find({ kernel, device, threads, smem });
+    if (it == g_facts.per_sm.end()) {
+        size_t& set = g_facts.smem_set[{ kernel, device }];
+        if (smem > set) {
+            DRB_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            set = smem;
+        }
+        int b = 0;
+        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, threads, smem));
+        it = g_facts.per_sm.emplace(std::make_tuple(kernel, device, threads, smem), b).first;
+    }
+    *sms = n;
+    *per_sm = it->second;
+    return DRB_OK;
+}
+
 bool drb_peer_access(int owner, int accessor)
 {
     if (owner == accessor) return true;
-    static std::mutex mu;
-    static std::unordered_map<int, bool> done;                  // owner * 4096 + accessor -> usable
-    std::lock_guard<std::mutex> g(mu);
-    const int key = owner * 4096 + accessor;
-    auto it = done.find(key);
-    if (it != done.end()) return it->second;
+    std::lock_guard<std::mutex> g(g_facts.mu);
+    auto it = g_facts.peer.find({ owner, accessor });
+    if (it != g_facts.peer.end()) return it->second;
     bool ok = false;
     int can = 0;
     if (cudaDeviceCanAccessPeer(&can, accessor, owner) == cudaSuccess && can) {
@@ -854,7 +875,7 @@ bool drb_peer_access(int owner, int accessor)
         cudaSetDevice(cur);
     }
     cudaGetLastError();
-    done[key] = ok;
+    g_facts.peer[{ owner, accessor }] = ok;
     return ok;
 }
 
@@ -910,21 +931,13 @@ struct EventTrio {
     int create() { for (auto& x : e) DRB_CUDA(cudaEventCreate(&x)); return DRB_OK; }
 };
 
-// co-resident grid of a cooperative build kernel, asked once per process and device
+// co-resident grid of a cooperative build kernel, at most max_per_sm blocks per SM: a grid barrier costs more the more
+// blocks take part
 int coop_grid(int device, const void* kernel, int want_blocks, int max_per_sm, int* blocks)
 {
-    static std::mutex mu;
-    static std::unordered_map<uint64_t, int> cache;
-    std::lock_guard<std::mutex> g(mu);
-    const uint64_t key = ((uint64_t)(uintptr_t)kernel << 8) ^ (uint64_t)(device & 0xFF);
-    auto it = cache.find(key);
-    if (it == cache.end()) {
-        int sms = 148, per_sm = 1;
-        DRB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-        DRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kBuildThreads, 0));
-        it = cache.emplace(key, sms * std::max(std::min(per_sm, max_per_sm), 1)).first;      // a grid barrier costs more the more blocks take part
-    }
-    *blocks = std::max(1, std::min(it->second, want_blocks));
+    int sms = 0, per_sm = 0;
+    if (int rc = drb_occupancy(kernel, kBuildThreads, 0, device, &sms, &per_sm)) return rc;
+    *blocks = std::max(1, std::min(sms * std::max(std::min(per_sm, max_per_sm), 1), want_blocks));
     return DRB_OK;
 }
 
@@ -938,8 +951,20 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
     cudaStream_t st = s->stream;
     StageClock clk;
     struct PrintOnExit { StageClock& c; ~PrintOnExit() { c.mark("scratch-free"); c.print("build_tree"); } };
-    Scratch tmp(st);
-    PrintOnExit print_on_exit{ clk };                         // destroyed before tmp: "scratch-free" is then ~0; see drb_scene_create's own clock
+    // scratch of the build, declared before `drain` so that the stream has drained when it goes back to the cache
+    DevArray<drb_object> up;
+    DevArray<int> d_flag, d_slot, d_bounds, d_levels, leaf_parent, visits, d_height, cid[2], nn, pl, pr, wq[2], wcounts, wneed, idx_u, orig_u;
+    DevArray<float4> bmin_u, bmax_u, lmin, lmax, cmn[2], cmx[2], pmin, pmax;
+    DevArray<unsigned long long> fl, btot, wtot;
+    DevArray<uint64_t> keys_u;
+    DevArray<BuildCtl> d_ctl;
+    DevArray<Prim> prims_u;
+    DevArray<ShadeRec> recs_u;
+    DevArray<int4> wslots;
+    DevArray<char> d_scan, d_sort;
+    LbvhDebug dbg; FinalTree tree;                          // moved into the scene with DRB_BUILD_KEEP_DEBUG
+    StreamDrain drain{ st };
+    PrintOnExit print_on_exit{ clk };                         // destroyed before the scratch: "scratch-free" is then ~0; see drb_scene_create's own clock
     EventTrio ev;
     if (int rc = ev.create()) return rc;
     DRB_CUDA(cudaEventRecord(ev.e[0], st));
@@ -949,19 +974,17 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
     const bool lbvh_only = (s->build_flags & DRB_BUILD_LBVH_ONLY) != 0;
     const int nprims = (int)drb_host_scene_num_renderable(hs);
     const drb_object* d_objs = objs_dev;
-    int* d_flag = nullptr; int* d_slot = nullptr; int* d_bounds = nullptr; BuildCtl* d_ctl = nullptr; int* d_levels = nullptr;
     if (!d_objs) {
-        drb_object* up = nullptr;
-        if (int rc = tmp.alloc(&up, (size_t)nobj)) return rc;
-        if (nobj) DRB_CUDA(cudaMemcpyAsync(up, hs->objects.data(), (size_t)nobj * sizeof(drb_object), cudaMemcpyHostToDevice, st));
-        d_objs = up;
+        if (int rc = up.alloc((size_t)nobj, st)) return rc;
+        if (nobj) DRB_CUDA(cudaMemcpyAsync(up.get(), hs->objects.data(), (size_t)nobj * sizeof(drb_object), cudaMemcpyHostToDevice, st));
+        d_objs = up.get();
     }
-    if (int rc = tmp.alloc(&d_flag, (size_t)nobj + 1)) return rc;
-    if (int rc = tmp.alloc(&d_slot, (size_t)nobj + 1)) return rc;
-    if (int rc = tmp.alloc(&d_bounds, 8)) return rc;
-    if (int rc = tmp.alloc(&d_ctl, 1)) return rc;
-    if (int rc = tmp.alloc(&d_levels, (size_t)kMaxWideLevels + 1)) return rc;
-    DRB_CUDA(cudaMemsetAsync(d_ctl, 0, sizeof(BuildCtl), st));
+    if (int rc = d_flag.alloc((size_t)nobj + 1, st)) return rc;
+    if (int rc = d_slot.alloc((size_t)nobj + 1, st)) return rc;
+    if (int rc = d_bounds.alloc(8, st)) return rc;
+    if (int rc = d_ctl.alloc(1, st)) return rc;
+    if (int rc = d_levels.alloc((size_t)kMaxWideLevels + 1, st)) return rc;
+    DRB_CUDA(cudaMemsetAsync(d_ctl.get(), 0, sizeof(BuildCtl), st));
     DRB_CUDA(cudaEventRecord(ev.e[1], st));
     clk.mark("upload-enqueue");
 
@@ -972,133 +995,123 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
     memset(&s->info, 0, sizeof s->info);
     s->info.nprims = nprims; s->info.nnodes = s->nnodes;
 
-    if (int rc = dev_alloc(&s->prims, (size_t)nprims, st)) return rc;
-    if (int rc = dev_alloc(&s->recs, (size_t)nprims, st)) return rc;
-    if (int rc = dev_alloc(&s->orig_id, (size_t)nprims, st)) return rc;
+    if (int rc = s->prims.alloc((size_t)nprims, st)) return rc;
+    if (int rc = s->recs.alloc((size_t)nprims, st)) return rc;
+    if (int rc = s->orig_id.alloc((size_t)nprims, st)) return rc;
     const size_t nint = nprims > 1 ? (size_t)nprims - 1 : 1;
     // the integer outputs of the build stay resident only on request (drb_scene_lbvh / drb_scene_tree); otherwise they
     // are scratch: ~100 B per primitive that rendering never reads
-    auto side = [&](auto** p, size_t count) -> int { return keep ? dev_alloc(p, count, st) : tmp.alloc(p, count); };
-    LbvhDebug dbg; FinalTree tree;
-    if (int rc = side(&dbg.keys, (size_t)nprims)) return rc;
-    if (int rc = side(&dbg.order, (size_t)nprims)) return rc;
+    if (int rc = dbg.keys.alloc((size_t)nprims, st)) return rc;
+    if (int rc = dbg.order.alloc((size_t)nprims, st)) return rc;
     if (keep || lbvh_only) {
-        if (int rc = side(&dbg.parent, nint)) return rc;
-        if (int rc = side(&dbg.left, nint)) return rc;
-        if (int rc = side(&dbg.right, nint)) return rc;
-        if (int rc = side(&dbg.node_min, nint)) return rc;
-        if (int rc = side(&dbg.node_max, nint)) return rc;
+        if (int rc = dbg.parent.alloc(nint, st)) return rc;
+        if (int rc = dbg.left.alloc(nint, st)) return rc;
+        if (int rc = dbg.right.alloc(nint, st)) return rc;
+        if (int rc = dbg.node_min.alloc(nint, st)) return rc;
+        if (int rc = dbg.node_max.alloc(nint, st)) return rc;
     }
-    if (int rc = side(&tree.left, nint)) return rc;
-    if (int rc = side(&tree.right, nint)) return rc;
-    if (int rc = side(&tree.node_min, nint)) return rc;
-    if (int rc = side(&tree.node_max, nint)) return rc;
-    if (keep) { s->dbg = dbg; s->tree = tree; }
+    if (int rc = tree.left.alloc(nint, st)) return rc;
+    if (int rc = tree.right.alloc(nint, st)) return rc;
+    if (int rc = tree.node_min.alloc(nint, st)) return rc;
+    if (int rc = tree.node_max.alloc(nint, st)) return rc;
 
     BuildCtl ctl; memset(&ctl, 0, sizeof ctl);
     int hb[6] = { 0, 0, 0, 0, 0, 0 };
     if (nprims > 0) {
-        Prim* prims_u; ShadeRec* recs_u; int32_t* orig_u; float4 *bmin_u, *bmax_u, *lmin, *lmax;
-        uint64_t* keys_u; int32_t* idx_u;
-        if (int rc = tmp.alloc(&prims_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&recs_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&orig_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&bmin_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&bmax_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&lmin, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&lmax, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&keys_u, (size_t)nprims)) return rc;
-        if (int rc = tmp.alloc(&idx_u, (size_t)nprims)) return rc;
+        if (int rc = prims_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = recs_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = orig_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = bmin_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = bmax_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = lmin.alloc((size_t)nprims, st)) return rc;
+        if (int rc = lmax.alloc((size_t)nprims, st)) return rc;
+        if (int rc = keys_u.alloc((size_t)nprims, st)) return rc;
+        if (int rc = idx_u.alloc((size_t)nprims, st)) return rc;
 
-        k_flag<<<(unsigned)((nobj + T - 1) / T), T, 0, st>>>(d_objs, nobj, d_flag);
+        k_flag<<<(unsigned)((nobj + T - 1) / T), T, 0, st>>>(d_objs, nobj, d_flag.get());
         size_t scan_bytes = 0;
-        DRB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_flag, d_slot, (int)nobj, st));
-        void* d_scan = nullptr;
-        if (int rc = tmp.alloc((char**)&d_scan, scan_bytes)) return rc;
-        DRB_CUDA(cub::DeviceScan::ExclusiveSum(d_scan, scan_bytes, d_flag, d_slot, (int)nobj, st));
-        k_init_bounds<<<1, 32, 0, st>>>(d_bounds);
-        k_pack<<<(unsigned)((nobj + T - 1) / T), T, 0, st>>>(d_objs, nobj, d_flag, d_slot, nprims, prims_u, recs_u, orig_u, bmin_u, bmax_u, d_bounds, &d_ctl->packed);
-        k_keys<<<(nprims + T - 1) / T, T, 0, st>>>(bmin_u, bmax_u, nprims, d_bounds, keys_u, idx_u);
+        DRB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, d_flag.get(), d_slot.get(), (int)nobj, st));
+        if (int rc = d_scan.alloc(scan_bytes, st)) return rc;
+        DRB_CUDA(cub::DeviceScan::ExclusiveSum(d_scan.get(), scan_bytes, d_flag.get(), d_slot.get(), (int)nobj, st));
+        k_init_bounds<<<1, 32, 0, st>>>(d_bounds.get());
+        k_pack<<<(unsigned)((nobj + T - 1) / T), T, 0, st>>>(d_objs, nobj, d_flag.get(), d_slot.get(), nprims, prims_u.get(), recs_u.get(), orig_u.get(),
+                                                             bmin_u.get(), bmax_u.get(), d_bounds.get(), &d_ctl.get()->packed);
+        k_keys<<<(nprims + T - 1) / T, T, 0, st>>>(bmin_u.get(), bmax_u.get(), nprims, d_bounds.get(), keys_u.get(), idx_u.get());
         size_t sort_bytes = 0;
-        DRB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys_u, dbg.keys, idx_u, dbg.order, nprims, 0, 63, st));
-        void* d_sort = nullptr;
-        if (int rc = tmp.alloc((char**)&d_sort, sort_bytes)) return rc;
-        DRB_CUDA(cub::DeviceRadixSort::SortPairs(d_sort, sort_bytes, keys_u, dbg.keys, idx_u, dbg.order, nprims, 0, 63, st));
+        DRB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, keys_u.get(), dbg.keys.get(), idx_u.get(), dbg.order.get(), nprims, 0, 63, st));
+        if (int rc = d_sort.alloc(sort_bytes, st)) return rc;
+        DRB_CUDA(cub::DeviceRadixSort::SortPairs(d_sort.get(), sort_bytes, keys_u.get(), dbg.keys.get(), idx_u.get(), dbg.order.get(), nprims, 0, 63, st));
         {
             const long long threads = (long long)nprims * 8;
-            k_gather<<<(unsigned)((threads + T - 1) / T), T, 0, st>>>(dbg.order, nprims, prims_u, recs_u, orig_u, bmin_u, bmax_u,
-                                                                      s->prims, s->recs, s->orig_id, lmin, lmax);
+            k_gather<<<(unsigned)((threads + T - 1) / T), T, 0, st>>>(dbg.order.get(), nprims, prims_u.get(), recs_u.get(), orig_u.get(), bmin_u.get(),
+                                                                      bmax_u.get(), s->prims.get(), s->recs.get(), s->orig_id.get(), lmin.get(), lmax.get());
         }
-        if (int rc = dev_alloc(&s->wnodes, nint, st)) return rc;
+        if (int rc = s->wnodes.alloc(nint, st)) return rc;
         if (nprims > 1) {
             if (keep || lbvh_only) {
                 // the LBVH of north_star: Karras hierarchy + bottom-up refit (the traversal tree only with DRB_BUILD_LBVH_ONLY)
-                int32_t* leaf_parent; int* visits; int* d_height;
-                if (int rc = tmp.alloc(&leaf_parent, (size_t)nprims)) return rc;
-                if (int rc = tmp.alloc(&visits, nint)) return rc;
-                if (int rc = tmp.alloc(&d_height, 1)) return rc;
-                DRB_CUDA(cudaMemsetAsync(visits, 0, nint * sizeof(int), st));
-                DRB_CUDA(cudaMemsetAsync(d_height, 0, sizeof(int), st));
-                k_karras<<<(nprims - 1 + T - 1) / T, T, 0, st>>>(dbg.keys, nprims, dbg.left, dbg.right, dbg.parent, leaf_parent);
-                k_refit<<<(nprims + T - 1) / T, T, 0, st>>>(nprims, lmin, lmax, dbg.left, dbg.right, dbg.parent, leaf_parent, visits,
-                                                           dbg.node_min, dbg.node_max, d_height);
+                if (int rc = leaf_parent.alloc((size_t)nprims, st)) return rc;
+                if (int rc = visits.alloc(nint, st)) return rc;
+                if (int rc = d_height.alloc(1, st)) return rc;
+                DRB_CUDA(cudaMemsetAsync(visits.get(), 0, nint * sizeof(int), st));
+                DRB_CUDA(cudaMemsetAsync(d_height.get(), 0, sizeof(int), st));
+                k_karras<<<(nprims - 1 + T - 1) / T, T, 0, st>>>(dbg.keys.get(), nprims, dbg.left.get(), dbg.right.get(), dbg.parent.get(), leaf_parent.get());
+                k_refit<<<(nprims + T - 1) / T, T, 0, st>>>(nprims, lmin.get(), lmax.get(), dbg.left.get(), dbg.right.get(), dbg.parent.get(), leaf_parent.get(),
+                                                           visits.get(), dbg.node_min.get(), dbg.node_max.get(), d_height.get());
             }
             if (lbvh_only) {
-                DRB_CUDA(cudaMemcpyAsync(tree.left, dbg.left, nint * 4, cudaMemcpyDeviceToDevice, st));
-                DRB_CUDA(cudaMemcpyAsync(tree.right, dbg.right, nint * 4, cudaMemcpyDeviceToDevice, st));
-                DRB_CUDA(cudaMemcpyAsync(tree.node_min, dbg.node_min, nint * 16, cudaMemcpyDeviceToDevice, st));
-                DRB_CUDA(cudaMemcpyAsync(tree.node_max, dbg.node_max, nint * 16, cudaMemcpyDeviceToDevice, st));
+                DRB_CUDA(cudaMemcpyAsync(tree.left.get(), dbg.left.get(), nint * 4, cudaMemcpyDeviceToDevice, st));
+                DRB_CUDA(cudaMemcpyAsync(tree.right.get(), dbg.right.get(), nint * 4, cudaMemcpyDeviceToDevice, st));
+                DRB_CUDA(cudaMemcpyAsync(tree.node_min.get(), dbg.node_min.get(), nint * 16, cudaMemcpyDeviceToDevice, st));
+                DRB_CUDA(cudaMemcpyAsync(tree.node_max.get(), dbg.node_max.get(), nint * 16, cudaMemcpyDeviceToDevice, st));
             } else {
                 // SAH-guided rebuild over the same sorted leaves
-                int32_t* cid[2]; float4* cmn[2]; float4* cmx[2]; int32_t* nn; unsigned long long *fl, *btot;
-                int32_t *pl, *pr; float4 *pmin, *pmax;
                 for (int k = 0; k < 2; ++k) {
-                    if (int rc = tmp.alloc(&cid[k], (size_t)nprims)) return rc;
-                    if (int rc = tmp.alloc(&cmn[k], (size_t)nprims)) return rc;
-                    if (int rc = tmp.alloc(&cmx[k], (size_t)nprims)) return rc;
+                    if (int rc = cid[k].alloc((size_t)nprims, st)) return rc;
+                    if (int rc = cmn[k].alloc((size_t)nprims, st)) return rc;
+                    if (int rc = cmx[k].alloc((size_t)nprims, st)) return rc;
                 }
-                if (int rc = tmp.alloc(&nn, (size_t)nprims)) return rc;
-                if (int rc = tmp.alloc(&fl, (size_t)nprims)) return rc;
-                if (int rc = tmp.alloc(&pl, nint)) return rc;
-                if (int rc = tmp.alloc(&pr, nint)) return rc;
-                if (int rc = tmp.alloc(&pmin, nint)) return rc;
-                if (int rc = tmp.alloc(&pmax, nint)) return rc;
+                if (int rc = nn.alloc((size_t)nprims, st)) return rc;
+                if (int rc = fl.alloc((size_t)nprims, st)) return rc;
+                if (int rc = pl.alloc(nint, st)) return rc;
+                if (int rc = pr.alloc(nint, st)) return rc;
+                if (int rc = pmin.alloc(nint, st)) return rc;
+                if (int rc = pmax.alloc(nint, st)) return rc;
                 int blocks = 1;
                 if (int rc = coop_grid(s->device, (const void*)k_ploc_all, (nprims + kBuildThreads - 1) / kBuildThreads, 2, &blocks)) return rc;
-                if (int rc = tmp.alloc(&btot, (size_t)blocks)) return rc;
+                if (int rc = btot.alloc((size_t)blocks, st)) return rc;
                 int n0 = nprims;
-                const float4* c_lmin = lmin; const float4* c_lmax = lmax;
-                void* args[] = { &n0, &c_lmin, &c_lmax, &cid[0], &cid[1], &cmn[0], &cmn[1], &cmx[0], &cmx[1], &nn, &fl, &btot, &pl, &pr, &pmin, &pmax, &d_ctl };
+                void* args[] = { &n0, lmin.arg(), lmax.arg(), cid[0].arg(), cid[1].arg(), cmn[0].arg(), cmn[1].arg(), cmx[0].arg(), cmx[1].arg(), nn.arg(),
+                                 fl.arg(), btot.arg(), pl.arg(), pr.arg(), pmin.arg(), pmax.arg(), d_ctl.arg() };
                 DRB_CUDA(cudaLaunchCooperativeKernel((const void*)k_ploc_all, dim3(blocks), dim3(kBuildThreads), args, 0, st));
-                k_relabel<<<(nprims - 1 + T - 1) / T, T, 0, st>>>(nprims, pl, pr, pmin, pmax, tree.left, tree.right, tree.node_min, tree.node_max);
+                k_relabel<<<(nprims - 1 + T - 1) / T, T, 0, st>>>(nprims, pl.get(), pr.get(), pmin.get(), pmax.get(), tree.left.get(), tree.right.get(),
+                                                                 tree.node_min.get(), tree.node_max.get());
             }
             // ---- four-wide collapse of the final tree (tree.*, root 0)
-            int32_t* wq[2]; int4* wslots; int *wcounts, *wneed; unsigned long long* wtot;
-            if (int rc = tmp.alloc(&wq[0], (size_t)nprims)) return rc;
-            if (int rc = tmp.alloc(&wq[1], (size_t)nprims)) return rc;
-            if (int rc = tmp.alloc(&wslots, (size_t)nprims)) return rc;
-            if (int rc = tmp.alloc(&wcounts, (size_t)nprims)) return rc;
-            if (int rc = tmp.alloc(&wneed, nint)) return rc;
+            if (int rc = wq[0].alloc((size_t)nprims, st)) return rc;
+            if (int rc = wq[1].alloc((size_t)nprims, st)) return rc;
+            if (int rc = wslots.alloc((size_t)nprims, st)) return rc;
+            if (int rc = wcounts.alloc((size_t)nprims, st)) return rc;
+            if (int rc = wneed.alloc(nint, st)) return rc;
             int blocks = 1;
             if (int rc = coop_grid(s->device, (const void*)k_wide_all, (nprims / 2 + kBuildThreads - 1) / kBuildThreads, 1, &blocks)) return rc;
-            if (int rc = tmp.alloc(&wtot, (size_t)blocks)) return rc;
-            const int32_t* c_left = tree.left; const int32_t* c_right = tree.right; const float4* c_nmin = tree.node_min; const float4* c_nmax = tree.node_max;
-            const float4* c_lmin = lmin; const float4* c_lmax = lmax; const int* c_bounds = d_bounds;
+            if (int rc = wtot.alloc((size_t)blocks, st)) return rc;
             int max_nodes = (int)nint;
-            void* args[] = { &c_left, &c_right, &c_nmin, &c_nmax, &c_lmin, &c_lmax, &c_bounds, &max_nodes, &wq[0], &wq[1], &wslots, &wcounts, &wtot,
-                             &s->wnodes, &wneed, &d_levels, &d_ctl };
+            void* args[] = { tree.left.arg(), tree.right.arg(), tree.node_min.arg(), tree.node_max.arg(), lmin.arg(), lmax.arg(), d_bounds.arg(), &max_nodes,
+                             wq[0].arg(), wq[1].arg(), wslots.arg(), wcounts.arg(), wtot.arg(), s->wnodes.arg(), wneed.arg(), d_levels.arg(), d_ctl.arg() };
             DRB_CUDA(cudaLaunchCooperativeKernel((const void*)k_wide_all, dim3(blocks), dim3(kBuildThreads), args, 0, st));
         } else {
-            k_wide_single<<<1, 1, 0, st>>>(lmin, lmax, d_bounds, s->wnodes, d_levels);
+            k_wide_single<<<1, 1, 0, st>>>(lmin.get(), lmax.get(), d_bounds.get(), s->wnodes.get(), d_levels.get());
         }
-        DRB_CUDA(cudaMemcpyAsync(hb, d_bounds, sizeof hb, cudaMemcpyDeviceToHost, st));
-        DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl, sizeof ctl, cudaMemcpyDeviceToHost, st));
+        DRB_CUDA(cudaMemcpyAsync(hb, d_bounds.get(), sizeof hb, cudaMemcpyDeviceToHost, st));
+        DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl.get(), sizeof ctl, cudaMemcpyDeviceToHost, st));
     }
     DRB_CUDA(cudaEventRecord(ev.e[2], st));
     clk.mark("build-enqueue");
     DRB_CUDA(cudaStreamSynchronize(st));                     // the one synchronisation of the build
     clk.mark("sync");
     DRB_CUDA(cudaGetLastError());
+    if (keep) { s->dbg = std::move(dbg); s->tree = std::move(tree); }
     if (nprims > 0) {
         if (ctl.packed != nprims) { drb_set_error("the device packed %d renderable objects, the host scene counted %d", ctl.packed, nprims); return DRB_ERR_ARG; }
         if (ctl.error == 1) { drb_set_error("hierarchy rebuild made no progress (%d clusters left after %d rounds)", ctl.ploc_n, ctl.rounds); return DRB_ERR_CUDA; }
@@ -1108,8 +1121,8 @@ int build_tree(drb_scene* s, const drb_host_scene* hs, const drb_object* objs_de
         else { s->nwnodes = 1; s->wide_levels = 1; s->stack_levels = 3; s->info.max_depth = 1; }
         s->info.rebuild_iterations = ctl.rounds;
         s->info.nwide = s->nwnodes; s->info.wide_levels = s->wide_levels; s->info.stack_levels = s->stack_levels;
-        if (int rc = dev_alloc(&s->wide_level_start, (size_t)s->wide_levels + 1, st)) return rc;
-        DRB_CUDA(cudaMemcpyAsync(s->wide_level_start, d_levels, ((size_t)s->wide_levels + 1) * sizeof(int), cudaMemcpyDeviceToDevice, st));
+        if (int rc = s->wide_level_start.alloc((size_t)s->wide_levels + 1, st)) return rc;
+        DRB_CUDA(cudaMemcpyAsync(s->wide_level_start.get(), d_levels.get(), ((size_t)s->wide_levels + 1) * sizeof(int), cudaMemcpyDeviceToDevice, st));
     }
     float ms = 0;
     cudaEventElapsedTime(&ms, ev.e[0], ev.e[1]); s->info.upload_ms = ms;
@@ -1138,15 +1151,15 @@ int upload_textures(drb_scene* s, const drb_host_scene* hs)
             if (used[(size_t)i]) return rc;             // a texture the scene names must load
             continue;                                   // the reference loads every .ppm it finds; unused ones may be anything
         }
-        void* d = nullptr;
-        DRB_CUDA(drb_dev_alloc(&d, img.rgba.size(), s->stream));
-        s->texture_storage.push_back(d);
+        s->texture_storage.emplace_back();
+        if ((rc = s->texture_storage.back().alloc(img.rgba.size(), s->stream)) != DRB_OK) return rc;
+        uint8_t* d = s->texture_storage.back().get();
         DRB_CUDA(cudaMemcpyAsync(d, img.rgba.data(), img.rgba.size(), cudaMemcpyHostToDevice, s->stream));
         DRB_CUDA(cudaStreamSynchronize(s->stream));      // img goes out of scope
         table[(size_t)i] = DevTexture{ (const uchar4*)d, img.w, img.h };
     }
-    if (int rc = dev_alloc(&s->textures, table.size(), s->stream)) return rc;
-    DRB_CUDA(cudaMemcpyAsync(s->textures, table.data(), table.size() * sizeof(DevTexture), cudaMemcpyHostToDevice, s->stream));
+    if (int rc = s->textures.alloc(table.size(), s->stream)) return rc;
+    DRB_CUDA(cudaMemcpyAsync(s->textures.get(), table.data(), table.size() * sizeof(DevTexture), cudaMemcpyHostToDevice, s->stream));
     DRB_CUDA(cudaStreamSynchronize(s->stream));
     drb_clear_error();
     return DRB_OK;
@@ -1160,31 +1173,26 @@ int refit_tree(drb_scene* s, const drb_object* d_objs, cudaStream_t st)
     const int64_t nobj = s->nobjects;
     const int nprims = (int)s->nprims;
     const int T = 256;
-    Scratch tmp(st);
-    RefitCtl* d_ctl = nullptr; float4* lmin = nullptr; float4* lmax = nullptr;
-    if (int rc = tmp.alloc(&d_ctl, 1)) return rc;
-    if (int rc = tmp.alloc(&lmin, (size_t)nprims)) return rc;
-    if (int rc = tmp.alloc(&lmax, (size_t)nprims)) return rc;
-    if (!s->refit_inv) {
-        if (int rc = dev_alloc(&s->refit_inv, (size_t)nobj, st)) return rc;
-        DRB_CUDA(cudaMemsetAsync(s->refit_inv, 0xFF, (size_t)nobj * sizeof(uint32_t), st));
-        if (nprims > 0) k_refit_inverse<<<(nprims + T - 1) / T, T, 0, st>>>(s->orig_id, s->prims, nprims, s->refit_inv);
-    }
+    DevArray<RefitCtl> d_ctl;
+    DevArray<float4> lmin, lmax;
+    StreamDrain drain{ st };                                 // the scratch goes back to the cache idle, whichever return is taken
+    if (int rc = d_ctl.alloc(1, st)) return rc;
+    if (int rc = lmin.alloc((size_t)nprims, st)) return rc;
+    if (int rc = lmax.alloc((size_t)nprims, st)) return rc;
     const unsigned grid_lines = (unsigned)((nobj + T - 1) / T);
-    k_refit_init<<<1, 32, 0, st>>>(d_ctl);
-    k_refit_check<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv, lmin, lmax, d_ctl);
+    k_refit_init<<<1, 32, 0, st>>>(d_ctl.get());
+    k_refit_check<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv.get(), lmin.get(), lmax.get(), d_ctl.get());
     if (nprims > 0) {
-        k_refit_pack<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv, d_ctl, s->prims, s->recs);
+        k_refit_pack<<<grid_lines, T, 0, st>>>(d_objs, nobj, s->refit_inv.get(), d_ctl.get(), s->prims.get(), s->recs.get());
         int blocks = 1;
         if (int rc = coop_grid(s->device, (const void*)k_refit_wide, (int)((s->nwnodes + kBuildThreads - 1) / kBuildThreads), 2, &blocks)) return rc;
-        const int* c_levels = s->wide_level_start; int levels = s->wide_levels;
-        const float4* c_lmin = lmin; const float4* c_lmax = lmax; const RefitCtl* c_ctl = d_ctl;
-        void* args[] = { &c_levels, &levels, &c_lmin, &c_lmax, &c_ctl, &s->wnodes };
+        int levels = s->wide_levels;
+        void* args[] = { s->wide_level_start.arg(), &levels, lmin.arg(), lmax.arg(), d_ctl.arg(), s->wnodes.arg() };
         DRB_CUDA(cudaLaunchCooperativeKernel((const void*)k_refit_wide, dim3(blocks), dim3(kBuildThreads), args, 0, st));
     }
     DRB_CUDA(cudaGetLastError());
     RefitCtl ctl;
-    DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl, sizeof ctl, cudaMemcpyDeviceToHost, st));
+    DRB_CUDA(cudaMemcpyAsync(&ctl, d_ctl.get(), sizeof ctl, cudaMemcpyDeviceToHost, st));
     DRB_CUDA(cudaStreamSynchronize(st));                     // the one synchronisation of the refit
     if (ctl.bad != ~0ull) {
         const long long line = (long long)(ctl.bad >> 2);
@@ -1196,6 +1204,17 @@ int refit_tree(drb_scene* s, const drb_object* d_objs, cudaStream_t st)
     }
     if (nprims > 0)
         for (int a = 0; a < 3; ++a) { s->info.bounds_min[a] = ordered_to_float(ctl.bounds[a]); s->info.bounds_max[a] = ordered_to_float(ctl.bounds[3 + a]); }
+    return DRB_OK;
+}
+
+// The line -> slot map, made by the first refit on the scene's own stream: the stream it is freed on when the scene is.
+int ensure_refit_inverse(drb_scene* s)
+{
+    if (s->refit_inv.get()) return DRB_OK;
+    const int nprims = (int)s->nprims, T = 256;
+    if (int rc = s->refit_inv.alloc((size_t)s->nobjects, s->stream)) return rc;
+    DRB_CUDA(cudaMemsetAsync(s->refit_inv.get(), 0xFF, (size_t)s->nobjects * sizeof(uint32_t), s->stream));
+    if (nprims > 0) k_refit_inverse<<<(nprims + T - 1) / T, T, 0, s->stream>>>(s->orig_id.get(), s->prims.get(), nprims, s->refit_inv.get());
     return DRB_OK;
 }
 
@@ -1229,18 +1248,10 @@ void drb_scene_free(drb_scene* s)
 {
     if (!s) return;
     cudaSetDevice(s->device);
-    drb_render_buffers_free(s);
-    drb_query_buffers_free(s);
+    cudaDeviceSynchronize();                                 // renders and queries may have run on caller streams
     cudaStream_t st = s->stream;
-    if (st) cudaStreamSynchronize(st);
-    for (void* p : { (void*)s->prims, (void*)s->recs, (void*)s->orig_id, (void*)s->textures, (void*)s->dbg.keys,
-                     (void*)s->dbg.order, (void*)s->dbg.parent, (void*)s->dbg.left, (void*)s->dbg.right, (void*)s->dbg.node_min,
-                     (void*)s->dbg.node_max, (void*)s->tree.left, (void*)s->tree.right, (void*)s->tree.node_min, (void*)s->tree.node_max, (void*)s->wnodes,
-                     (void*)s->wide_level_start, (void*)s->refit_inv })
-        if (p) drb_dev_free(p, st);
-    for (void* p : s->texture_storage) drb_dev_free(p, st);
-    if (st) cudaStreamDestroy(st);
-    delete s;
+    delete s;                                                // every array goes back to the cache, some freed on the stream ...
+    if (st) cudaStreamDestroy(st);                           // ... which therefore goes last
 }
 
 int drb_scene_create(const drb_host_scene* hs, int device, drb_scene** out) { return drb_scene_create_from_device(hs, device, 0u, nullptr, nullptr, out); }
@@ -1316,7 +1327,7 @@ int drb_scene_create_multi(const drb_host_scene* hs, const int* devices, int nde
     auto trace = [&](const char* fmt, int a, int b) { if (debug) { fprintf(stderr, "[dogeray_b200] create_multi: "); fprintf(stderr, fmt, a, b); fputc('\n', stderr); fflush(stderr); } };
     // share k = object lines [k * chunk, (k + 1) * chunk): uploaded by device k, pulled by all the others
     const size_t chunk = (nobj + (size_t)ndevices - 1) / (size_t)ndevices;
-    struct Side { drb_object* buf = nullptr; cudaStream_t st = nullptr; cudaEvent_t uploaded = nullptr, pulled = nullptr; int rc = DRB_OK; std::string err; };
+    struct Side { DevArray<drb_object> buf; cudaStream_t st = nullptr; cudaEvent_t uploaded = nullptr, pulled = nullptr; int rc = DRB_OK; std::string err; };
     std::vector<Side> side((size_t)ndevices);
     auto share = [&](int k, size_t* lo, size_t* hi) { *lo = std::min(nobj, (size_t)k * chunk); *hi = std::min(nobj, *lo + chunk); };
     // phase 1 (sequential, cheap): buffers, streams, events, and each device's own share on its way
@@ -1327,9 +1338,9 @@ int drb_scene_create_multi(const drb_host_scene* hs, const int* devices, int nde
         if (retain_pool(devices[k]) != DRB_OK) { sd.rc = DRB_ERR_CUDA; sd.err = drb_last_error(); break; }
         if (cudaStreamCreateWithFlags(&sd.st, cudaStreamNonBlocking) != cudaSuccess) { bad("cudaStreamCreate"); break; }
         if (cudaEventCreateWithFlags(&sd.uploaded, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&sd.pulled, cudaEventDisableTiming) != cudaSuccess) { bad("cudaEventCreate"); break; }
-        if (drb_dev_alloc((void**)&sd.buf, std::max<size_t>(nobj, 1) * sizeof(drb_object), sd.st) != cudaSuccess) { bad("device memory for the object lines"); break; }
+        if (sd.buf.alloc(nobj, sd.st) != DRB_OK) { bad("device memory for the object lines"); break; }
         size_t lo, hi; share(k, &lo, &hi);
-        if (hi > lo && cudaMemcpyAsync(sd.buf + lo, hs->objects.data() + lo, (hi - lo) * sizeof(drb_object), cudaMemcpyHostToDevice, sd.st) != cudaSuccess) { bad("upload"); break; }
+        if (hi > lo && cudaMemcpyAsync(sd.buf.get() + lo, hs->objects.data() + lo, (hi - lo) * sizeof(drb_object), cudaMemcpyHostToDevice, sd.st) != cudaSuccess) { bad("upload"); break; }
         if (cudaEventRecord(sd.uploaded, sd.st) != cudaSuccess) { bad("cudaEventRecord"); break; }
         trace("share %d uploading on device %d", k, devices[k]);
     }
@@ -1350,14 +1361,14 @@ int drb_scene_create_multi(const drb_host_scene* hs, const int* devices, int nde
                 if (hi <= lo) continue;
                 if (cudaStreamWaitEvent(sd.st, side[(size_t)j].uploaded, 0) != cudaSuccess) return bad("cudaStreamWaitEvent");
                 const cudaError_t ce = devices[j] == devices[k]
-                    ? cudaMemcpyAsync(sd.buf + lo, side[(size_t)j].buf + lo, (hi - lo) * sizeof(drb_object), cudaMemcpyDeviceToDevice, sd.st)
-                    : cudaMemcpyPeerAsync(sd.buf + lo, devices[k], side[(size_t)j].buf + lo, devices[j], (hi - lo) * sizeof(drb_object), sd.st);
+                    ? cudaMemcpyAsync(sd.buf.get() + lo, side[(size_t)j].buf.get() + lo, (hi - lo) * sizeof(drb_object), cudaMemcpyDeviceToDevice, sd.st)
+                    : cudaMemcpyPeerAsync(sd.buf.get() + lo, devices[k], side[(size_t)j].buf.get() + lo, devices[j], (hi - lo) * sizeof(drb_object), sd.st);
                 if (ce != cudaSuccess) return bad("peer copy");
                 trace("pulled share %d into %d", j, k);
             }
             if (cudaEventRecord(sd.pulled, sd.st) != cudaSuccess) return bad("cudaEventRecord");
             trace("building scene %d on device %d", k, devices[k]);
-            sd.rc = drb_scene_create_from_device(hs, devices[k], build_flags, sd.buf, sd.st, &out[k]);
+            sd.rc = drb_scene_create_from_device(hs, devices[k], build_flags, sd.buf.get(), sd.st, &out[k]);
             if (sd.rc != DRB_OK) sd.err = drb_last_error();
             trace("scene %d: rc %d", k, sd.rc);
         };
@@ -1373,7 +1384,7 @@ int drb_scene_create_multi(const drb_host_scene* hs, const int* devices, int nde
     for (int k = 0; k < ndevices; ++k) {
         Side& sd = side[(size_t)k];
         if (cudaSetDevice(devices[k]) != cudaSuccess) { cudaGetLastError(); continue; }
-        if (sd.buf) drb_dev_free(sd.buf, sd.st);
+        sd.buf.reset();                                             // before its stream goes
         if (sd.uploaded) cudaEventDestroy(sd.uploaded);
         if (sd.pulled) cudaEventDestroy(sd.pulled);
         if (sd.st) cudaStreamDestroy(sd.st);
@@ -1421,6 +1432,7 @@ int drb_scene_refit_device(drb_scene* s, const void* objects_dev, int64_t nobjec
     if (int rc = refit_args(s, objects_dev, nobjects)) return rc;
     if (nobjects == 0) return DRB_OK;
     DRB_CUDA(cudaSetDevice(s->device));
+    if (int rc = ensure_refit_inverse(s)) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     if (st != s->stream) {
         // the refit runs on the caller's stream, after what is already enqueued on the scene's own
@@ -1439,11 +1451,11 @@ int drb_scene_refit(drb_scene* s, const drb_object* objects_host, int64_t nobjec
     if (int rc = refit_args(s, objects_host, nobjects)) return rc;
     if (nobjects == 0) return DRB_OK;
     DRB_CUDA(cudaSetDevice(s->device));
-    Scratch up(s->stream);
-    drb_object* d = nullptr;
-    if (int rc = up.alloc(&d, (size_t)nobjects)) return rc;
-    DRB_CUDA(cudaMemcpyAsync(d, objects_host, (size_t)nobjects * sizeof(drb_object), cudaMemcpyHostToDevice, s->stream));
-    return refit_tree(s, d, s->stream);
+    if (int rc = ensure_refit_inverse(s)) return rc;
+    DevArray<drb_object> d;                                  // idle once refit_tree returns: it drains the same stream
+    if (int rc = d.alloc((size_t)nobjects, s->stream)) return rc;
+    DRB_CUDA(cudaMemcpyAsync(d.get(), objects_host, (size_t)nobjects * sizeof(drb_object), cudaMemcpyHostToDevice, s->stream));
+    return refit_tree(s, d.get(), s->stream);
 }
 
 int drb_scene_lbvh(const drb_scene* s, uint64_t* keys, int32_t* order, int32_t* parent, int32_t* left, int32_t* right,
@@ -1453,19 +1465,19 @@ int drb_scene_lbvh(const drb_scene* s, uint64_t* keys, int32_t* order, int32_t* 
     if (!(s->build_flags & DRB_BUILD_KEEP_DEBUG)) { drb_set_error("drb_scene_lbvh: the scene was not created with DRB_BUILD_KEEP_DEBUG"); return DRB_ERR_UNSUPPORTED; }
     DRB_CUDA(cudaSetDevice(s->device));
     const size_t n = (size_t)s->nprims, ni = n > 1 ? n - 1 : 0;
-    if (keys && n) DRB_CUDA(cudaMemcpy(keys, s->dbg.keys, n * 8, cudaMemcpyDeviceToHost));
-    if (order && n) DRB_CUDA(cudaMemcpy(order, s->dbg.order, n * 4, cudaMemcpyDeviceToHost));
-    if (parent && ni) DRB_CUDA(cudaMemcpy(parent, s->dbg.parent, ni * 4, cudaMemcpyDeviceToHost));
-    if (left && ni) DRB_CUDA(cudaMemcpy(left, s->dbg.left, ni * 4, cudaMemcpyDeviceToHost));
-    if (right && ni) DRB_CUDA(cudaMemcpy(right, s->dbg.right, ni * 4, cudaMemcpyDeviceToHost));
+    if (keys && n) DRB_CUDA(cudaMemcpy(keys, s->dbg.keys.get(), n * 8, cudaMemcpyDeviceToHost));
+    if (order && n) DRB_CUDA(cudaMemcpy(order, s->dbg.order.get(), n * 4, cudaMemcpyDeviceToHost));
+    if (parent && ni) DRB_CUDA(cudaMemcpy(parent, s->dbg.parent.get(), ni * 4, cudaMemcpyDeviceToHost));
+    if (left && ni) DRB_CUDA(cudaMemcpy(left, s->dbg.left.get(), ni * 4, cudaMemcpyDeviceToHost));
+    if (right && ni) DRB_CUDA(cudaMemcpy(right, s->dbg.right.get(), ni * 4, cudaMemcpyDeviceToHost));
     if ((node_min || node_max) && ni) {
         std::vector<float4> tmp(ni);
         if (node_min) {
-            DRB_CUDA(cudaMemcpy(tmp.data(), s->dbg.node_min, ni * 16, cudaMemcpyDeviceToHost));
+            DRB_CUDA(cudaMemcpy(tmp.data(), s->dbg.node_min.get(), ni * 16, cudaMemcpyDeviceToHost));
             for (size_t i = 0; i < ni; ++i) { node_min[3*i] = tmp[i].x; node_min[3*i+1] = tmp[i].y; node_min[3*i+2] = tmp[i].z; }
         }
         if (node_max) {
-            DRB_CUDA(cudaMemcpy(tmp.data(), s->dbg.node_max, ni * 16, cudaMemcpyDeviceToHost));
+            DRB_CUDA(cudaMemcpy(tmp.data(), s->dbg.node_max.get(), ni * 16, cudaMemcpyDeviceToHost));
             for (size_t i = 0; i < ni; ++i) { node_max[3*i] = tmp[i].x; node_max[3*i+1] = tmp[i].y; node_max[3*i+2] = tmp[i].z; }
         }
     }
@@ -1479,7 +1491,7 @@ int drb_scene_wide(const drb_scene* s, int32_t* child, uint32_t* boxes)
     const size_t n = (size_t)s->nwnodes;
     if (!n) return DRB_OK;
     std::vector<WideNode> tmp(n);
-    DRB_CUDA(cudaMemcpy(tmp.data(), s->wnodes, n * sizeof(WideNode), cudaMemcpyDeviceToHost));
+    DRB_CUDA(cudaMemcpy(tmp.data(), s->wnodes.get(), n * sizeof(WideNode), cudaMemcpyDeviceToHost));
     for (size_t i = 0; i < n; ++i)
         for (int k = 0; k < 4; ++k) {
             if (child) child[4 * i + k] = tmp[i].child[k];
@@ -1494,16 +1506,16 @@ int drb_scene_tree(const drb_scene* s, int32_t* left, int32_t* right, float* nod
     if (!(s->build_flags & DRB_BUILD_KEEP_DEBUG)) { drb_set_error("drb_scene_tree: the scene was not created with DRB_BUILD_KEEP_DEBUG"); return DRB_ERR_UNSUPPORTED; }
     DRB_CUDA(cudaSetDevice(s->device));
     const size_t n = (size_t)s->nprims, ni = n > 1 ? n - 1 : 0;
-    if (left && ni) DRB_CUDA(cudaMemcpy(left, s->tree.left, ni * 4, cudaMemcpyDeviceToHost));
-    if (right && ni) DRB_CUDA(cudaMemcpy(right, s->tree.right, ni * 4, cudaMemcpyDeviceToHost));
+    if (left && ni) DRB_CUDA(cudaMemcpy(left, s->tree.left.get(), ni * 4, cudaMemcpyDeviceToHost));
+    if (right && ni) DRB_CUDA(cudaMemcpy(right, s->tree.right.get(), ni * 4, cudaMemcpyDeviceToHost));
     if ((node_min || node_max) && ni) {
         std::vector<float4> tmp(ni);
         if (node_min) {
-            DRB_CUDA(cudaMemcpy(tmp.data(), s->tree.node_min, ni * 16, cudaMemcpyDeviceToHost));
+            DRB_CUDA(cudaMemcpy(tmp.data(), s->tree.node_min.get(), ni * 16, cudaMemcpyDeviceToHost));
             for (size_t i = 0; i < ni; ++i) { node_min[3*i] = tmp[i].x; node_min[3*i+1] = tmp[i].y; node_min[3*i+2] = tmp[i].z; }
         }
         if (node_max) {
-            DRB_CUDA(cudaMemcpy(tmp.data(), s->tree.node_max, ni * 16, cudaMemcpyDeviceToHost));
+            DRB_CUDA(cudaMemcpy(tmp.data(), s->tree.node_max.get(), ni * 16, cudaMemcpyDeviceToHost));
             for (size_t i = 0; i < ni; ++i) { node_max[3*i] = tmp[i].x; node_max[3*i+1] = tmp[i].y; node_max[3*i+2] = tmp[i].z; }
         }
     }
