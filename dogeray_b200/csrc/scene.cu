@@ -293,8 +293,12 @@ __global__ void k_refit(int n, const float4* __restrict__ lmin, const float4* __
 // of it visits ~1.5x more nodes than a SAH-quality tree.  Starting from the same sorted leaves, every
 // cluster looks `radius` positions left and right for the neighbour whose union box has the smallest
 // surface area; mutually nearest pairs merge into a new node, the survivors are compacted in order, and
-// the process repeats until one cluster is left.  All steps are deterministic (ties go to the lower
-// position; node ids come from a prefix sum, not from atomics), so oracle/lbvh_host.c reproduces the
+// the process repeats until one cluster is left.  Equal areas go to the nearer position, then to the
+// smaller i ^ j: both are keys the two ends of a pair share, and for one cluster i they name one
+// neighbour.  So every cluster minimises (area, |i - j|, i ^ j) over its window, the least pair of the
+// whole array is mutual, and every round merges.  A run of identical boxes pairs (2k, 2k+1) and halves
+// each round; a tie to the lower position made it a chain, one merge per round.  All steps are
+// deterministic (node ids come from a prefix sum, not from atomics), so oracle/lbvh_host.c reproduces the
 // topology bit for bit.
 #ifndef DRB_PLOC_RADIUS
 #define DRB_PLOC_RADIUS 16
@@ -384,7 +388,8 @@ __global__ void __launch_bounds__(kBuildThreads) k_ploc_all(int n0, const float4
             for (int j = j0; j <= j1; ++j) {
                 if (j == i) continue;
                 const float a = union_half_area(lo, hi, cmin[j], cmax[j]);
-                if (a < best) { best = a; bj = j; }
+                const int d = abs(i - j), bd = abs(i - bj);
+                if (a < best || (a == best && (d < bd || (d == bd && (i ^ j) < (i ^ bj))))) { best = a; bj = j; }
             }
             if (bj < 0) bj = (i ^ 1) < n ? (i ^ 1) : i - 1;        // non-finite boxes: pair neighbours so the loop still ends
             nn[i] = bj;

@@ -136,7 +136,8 @@ int lbvh_host_build(const float* bmin, const float* bmax, int n, uint64_t* keys,
 
 /* ---- host mirror of the SAH-guided rebuild (k_ploc_* in dogeray_b200/csrc/scene.cu) ----------------
  * lmin/lmax: n*3 leaf boxes in SORTED order.  Outputs in the final labelling (root = node 0): left/right
- * [n-1] with leaves as ~sorted_position, node_min/node_max [(n-1)*3].  Returns the tree height. */
+ * [n-1] with leaves as ~sorted_position, node_min/node_max [(n-1)*3].  Returns the tree height; *rounds gets the
+ * number of clustering rounds (drb_build_info.rebuild_iterations of the device build). */
 static float union_half_area(const float* alo, const float* ahi, const float* blo, const float* bhi)
 {
     float ex = fmaxf(ahi[0], bhi[0]) - fminf(alo[0], blo[0]);
@@ -145,8 +146,10 @@ static float union_half_area(const float* alo, const float* ahi, const float* bl
     return ex * ey + ey * ez + ez * ex;
 }
 
-int ploc_host_build(const float* lmin, const float* lmax, int n, int radius, int32_t* left, int32_t* right, float* node_min, float* node_max)
+int ploc_host_build(const float* lmin, const float* lmax, int n, int radius, int32_t* left, int32_t* right, float* node_min, float* node_max,
+                    int* rounds)
 {
+    *rounds = 0;
     if (n <= 1) return n;
     size_t N = (size_t)n;
     int32_t* cid[2]; float* cmn[2]; float* cmx[2]; int* chg[2];
@@ -163,12 +166,14 @@ int ploc_host_build(const float* lmin, const float* lmax, int n, int radius, int
             for (int j = j0; j <= j1; j++) {
                 if (j == i) continue;
                 float a = union_half_area(cmn[cur] + 3 * i, cmx[cur] + 3 * i, cmn[cur] + 3 * j, cmx[cur] + 3 * j);
-                if (a < best) { best = a; bj = j; }
+                const int d = abs(i - j), bd = abs(i - bj);
+                if (a < best || (a == best && (d < bd || (d == bd && (i ^ j) < (i ^ bj))))) { best = a; bj = j; }
             }
             if (bj < 0) bj = (i ^ 1) < m ? (i ^ 1) : i - 1;
             nn[i] = bj;
         }
         int pos = 0, merges = 0, nx = cur ^ 1;
+        ++*rounds;
         for (int i = 0; i < m; i++) {
             int j = nn[i];
             int mutual = j >= 0 && j < m && nn[j] == i;

@@ -35,7 +35,7 @@ def _load():
     L.orc_philox_word.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]; L.orc_philox_word.restype = C.c_uint32
     L.lbvh_host_build.argtypes = [C.c_void_p] * 2 + [C.c_int] + [C.c_void_p] * 8
     L.lbvh_host_build.restype = C.c_int
-    L.ploc_host_build.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 4
+    L.ploc_host_build.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 5
     L.ploc_host_build.restype = C.c_int
     L.wide_host_build.argtypes = [C.c_void_p] * 6 + [C.c_int] + [C.c_void_p] * 4
     L.wide_host_build.restype = C.c_int
@@ -139,14 +139,16 @@ def lbvh_host(bmin: np.ndarray, bmax: np.ndarray):
 
 
 def ploc_host(lmin_sorted: np.ndarray, lmax_sorted: np.ndarray, radius: int = 16):
-    """Host mirror of the SAH-guided rebuild over sorted leaf boxes: dict(left, right, node_min, node_max, height)."""
+    """Host mirror of the SAH-guided rebuild over sorted leaf boxes: dict(left, right, node_min, node_max, height, rounds)."""
     L = _load()
     lmin = np.ascontiguousarray(lmin_sorted, np.float32); lmax = np.ascontiguousarray(lmax_sorted, np.float32)
     n = len(lmin); ni = max(n - 1, 0)
     left = np.zeros(ni, np.int32); right = np.zeros(ni, np.int32)
     nmin = np.zeros((ni, 3), np.float32); nmax = np.zeros((ni, 3), np.float32)
-    h = L.ploc_host_build(lmin.ctypes.data, lmax.ctypes.data, n, radius, left.ctypes.data, right.ctypes.data, nmin.ctypes.data, nmax.ctypes.data)
-    return dict(left=left, right=right, node_min=nmin, node_max=nmax, height=h)
+    rounds = C.c_int(0)
+    h = L.ploc_host_build(lmin.ctypes.data, lmax.ctypes.data, n, radius, left.ctypes.data, right.ctypes.data, nmin.ctypes.data, nmax.ctypes.data,
+                          C.byref(rounds))
+    return dict(left=left, right=right, node_min=nmin, node_max=nmax, height=h, rounds=rounds.value)
 
 
 def wide_host(left, right, node_min, node_max, lmin_sorted, lmax_sorted, scene_bounds):
