@@ -25,8 +25,6 @@
 #include "philox.cuh"
 #include "vec.cuh"
 
-#include <cub/device/device_radix_sort.cuh>
-
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -239,12 +237,12 @@ enum TraceMode { kClosest, kClosestSorted, kAnyHit };
 // the idle lanes claim fresh rays from the queue with ONE atomic per warp (ballot + popc + shfl), so warps
 // stay populated until the queue runs dry.  (A while-while variant measured slower on B200: with
 // one-primitive leaves, lanes that reach a leaf wait for the slowest descent.)
-// Traces the first `count` rays of ro / rdv, handed out in the order `order` gives (nullptr: queue order); the result of a
-// ray goes to hit (closest) or occluded (any hit) at its queue position.
+// Traces the first `count` rays of ro / rdv, taken in queue order; the result of a ray goes to hit (closest) or occluded
+// (any hit) at its queue position.
 template <TraceMode kMode>
 DRB_D void traverse(const DevScene& sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
                     uint2* __restrict__ hit, uint8_t* __restrict__ occluded, uint32_t* counters, uint32_t count,
-                    int refill, int leaf_batch, int step_min, const uint32_t* __restrict__ order)
+                    int refill, int leaf_batch, int step_min)
 {
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -279,9 +277,8 @@ DRB_D void traverse(const DevScene& sc, float scene_scale, const float4* __restr
             base = __shfl_sync(0xffffffffu, base, leader);
             if (base + (uint32_t)__popc(midle) >= count) exhausted = true;
             if (idle) {
-                const uint32_t k = base + (uint32_t)__popc(midle & lt_mask);
-                if (k < count) {
-                    const uint32_t i = order ? order[k] : k;        // queue position of the k-th ray in traversal order
+                const uint32_t i = base + (uint32_t)__popc(midle & lt_mask);
+                if (i < count) {
                     const float4 o4 = ro[i], d4 = rdv[i];
                     bool skip;                                      // the ray has no result to search for
                     if constexpr (kMode == kAnyHit) skip = !(d4.w > 0.0f);    // nothing is accepted at t < tmax <= 0 (t > 1e-4 / t > 0)
@@ -404,10 +401,9 @@ DRB_D void traverse(const DevScene& sc, float scene_scale, const float4* __restr
 // closest hit of the rays of queue `cur`
 template <bool kSortedPush>
 __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_trace(DevScene sc, float scene_scale, const float4* __restrict__ ro, const float4* __restrict__ rdv,
-                                               uint2* __restrict__ hit, uint32_t* counters, int cur, int refill, int leaf_batch, int step_min,
-                                               const uint32_t* __restrict__ order)
+                                               uint2* __restrict__ hit, uint32_t* counters, int cur, int refill, int leaf_batch, int step_min)
 {
-    traverse<kSortedPush ? kClosestSorted : kClosest>(sc, scene_scale, ro, rdv, hit, nullptr, counters, counters[cur], refill, leaf_batch, step_min, order);
+    traverse<kSortedPush ? kClosestSorted : kClosest>(sc, scene_scale, ro, rdv, hit, nullptr, counters, counters[cur], refill, leaf_batch, step_min);
 }
 
 // any hit of a query chunk (ray count in counters[0])
@@ -415,7 +411,7 @@ __global__ void __launch_bounds__(kTraceThreads, DRB_TRACE_MIN_BLOCKS) k_occlude
                                                                                  const float4* __restrict__ rdv, uint8_t* __restrict__ occluded,
                                                                                  uint32_t* counters, int refill, int leaf_batch, int step_min)
 {
-    traverse<kAnyHit>(sc, scene_scale, ro, rdv, nullptr, occluded, counters, counters[0], refill, leaf_batch, step_min, nullptr);
+    traverse<kAnyHit>(sc, scene_scale, ro, rdv, nullptr, occluded, counters, counters[0], refill, leaf_batch, step_min);
 }
 
 // ---- shading ---------------------------------------------------------------------------------------
@@ -792,33 +788,6 @@ __global__ void __launch_bounds__(128, DRB_SHADE_MIN_BLOCKS) k_shade(DevScene sc
     if (lane == 0 && local_rays) atomicAdd(reinterpret_cast<unsigned long long*>(&counters[CNT_RAYS]), (unsigned long long)local_rays);
 }
 
-// Sort key of a queued ray: direction octant (3 bits) above the 21-bit Morton code of the origin's cell in a
-// 128^3 grid over the scene bounds.  Rays that start close together and head the same way end up in the
-// same warp: they touch the same nodes (fewer distinct lines per load = fewer L1 wavefronts) and leave the
-// tree at similar times (fewer idle lanes).  Purely a scheduling order: results do not depend on it.
-__global__ void __launch_bounds__(256) k_ray_keys(const float4* __restrict__ ro, const float4* __restrict__ rdv, uint32_t count,
-                                                   float3 lo, float3 inv_ext, uint32_t* __restrict__ keys, uint32_t* __restrict__ vals)
-{
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= count) return;
-    const float4 o = ro[i], d = rdv[i];
-    auto cell = [](float v, float l, float s) -> uint32_t {
-        const float x = fminf(fmaxf((v - l) * s * 128.0f, 0.0f), 127.0f);
-        return (uint32_t)x;
-    };
-    auto spread7 = [](uint32_t v) -> uint32_t {                 // 7 bits -> every third bit
-        v = (v | (v << 16)) & 0x030000FFu;
-        v = (v | (v << 8)) & 0x0300F00Fu;
-        v = (v | (v << 4)) & 0x030C30C3u;
-        v = (v | (v << 2)) & 0x09249249u;
-        return v;
-    };
-    const uint32_t m = (spread7(cell(o.x, lo.x, inv_ext.x)) << 2) | (spread7(cell(o.y, lo.y, inv_ext.y)) << 1) | spread7(cell(o.z, lo.z, inv_ext.z));
-    const uint32_t oct = (d.x < 0.f ? 1u : 0u) | (d.y < 0.f ? 2u : 0u) | (d.z < 0.f ? 4u : 0u);
-    keys[i] = (oct << 21) | m;
-    vals[i] = i;
-}
-
 // counters for the next bounce: clear the queue that k_shade is about to fill and the trace ticket
 __global__ void k_prepare(uint32_t* counters, int clear_queue, int set_queue, uint32_t set_value)
 {
@@ -942,10 +911,6 @@ struct RenderBuffers {
     DevArray<uint32_t> counters;
     int trace_blocks = 0, shade_blocks = 0;
     size_t trace_smem = 0;              // dynamic shared memory of k_trace: (tree height + 2) stack levels x 128 lanes
-    // ray reordering (one sort per bounce): keys / ray indices, double-buffered, + CUB scratch
-    DevArray<uint32_t> sort_keys[2], sort_vals[2];
-    DevArray<char> sort_tmp;
-    size_t sort_tmp_bytes = 0;
     Queues queues() const
     {
         return Queues{ { ray_o[0].get(), ray_o[1].get() }, { ray_d[0].get(), ray_d[1].get() }, { thr[0].get(), thr[1].get() }, hit.get(), contrib.get(),
@@ -1009,10 +974,6 @@ Camera make_camera(const drb_settings& st, int W, int H, int divisor)
     return c;
 }
 
-// reorder a bounce's rays before tracing when the queue holds at least this many (0 = never, the default:
-// on B200 the sort costs more than the ~5 % of traversal time it saves on the 1 M-triangle workload)
-long g_sort_min = []() { const char* e = getenv("DOGERAY_B200_SORT_MIN"); return e ? atol(e) : 0L; }();
-
 // SMs x resident blocks per SM of a persistent kernel launched with `threads` per block and `smem` bytes of dynamic shared
 // memory (both asked once per process and device, drb_occupancy)
 int resident_grid(const void* kernel, int threads, int device, size_t smem, int* blocks)
@@ -1055,15 +1016,6 @@ int ensure_buffers(drb_scene* s, size_t slots)
     if (int rc = rb.hit.alloc(slots, st)) return rc;
     if (int rc = rb.contrib.alloc(slots, st)) return rc;
     if (int rc = rb.counters.alloc(CNT_WORDS, st)) return rc;
-    if (g_sort_min > 0) {                            // the opt-in ray reordering needs keys / indices / CUB scratch
-        for (int k = 0; k < 2; ++k) {
-            if (int rc = rb.sort_keys[k].alloc(slots, st)) return rc;
-            if (int rc = rb.sort_vals[k].alloc(slots, st)) return rc;
-        }
-        DRB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, rb.sort_tmp_bytes, rb.sort_keys[0].get(), rb.sort_keys[1].get(), rb.sort_vals[0].get(),
-                                                 rb.sort_vals[1].get(), (int)std::min<size_t>(slots, 0x7FFFFFFF), 0, 24, st));
-        if (int rc = rb.sort_tmp.alloc(rb.sort_tmp_bytes ? rb.sort_tmp_bytes : 16, st)) return rc;
-    }
     const Queues q = rb.queues();
     if (getenv("DOGERAY_B200_DEBUG"))
         fprintf(stderr, "[dogeray_b200] queues for %zu slots: o %p %p d %p %p thr %p %p hit %p contrib %p\n", slots, (void*)q.ray_o[0], (void*)q.ray_o[1],
@@ -1116,11 +1068,10 @@ int g_leaf_batch = []() { const char* e = getenv("DOGERAY_B200_LEAF_BATCH"); int
 int g_step_min = []() { const char* e = getenv("DOGERAY_B200_STEP_MIN"); int v = e ? atoi(e) : 20; return v < 1 ? 1 : v; }();
 
 // the closest-hit kernel for this scene: large scenes push the other hit children far-to-near (see DRB_SORTED_PUSH_FROM)
-void launch_trace(const drb_scene* s, int blocks, size_t smem, cudaStream_t stream, const DevScene& sc, float scale, const Queues& q, int cur,
-                  const uint32_t* order)
+void launch_trace(const drb_scene* s, int blocks, size_t smem, cudaStream_t stream, const DevScene& sc, float scale, const Queues& q, int cur)
 {
     auto kernel = s->nprims >= (int64_t)DRB_SORTED_PUSH_FROM ? k_trace<true> : k_trace<false>;
-    kernel<<<blocks, kTraceThreads, smem, stream>>>(sc, scale, q.ray_o[cur], q.ray_d[cur], q.hit, q.counters, cur, g_refill, g_leaf_batch, g_step_min, order);
+    kernel<<<blocks, kTraceThreads, smem, stream>>>(sc, scale, q.ray_o[cur], q.ray_d[cur], q.hit, q.counters, cur, g_refill, g_leaf_batch, g_step_min);
 }
 
 // rays per chunk of a ray query (DOGERAY_B200_QUERY_CHUNK, default 64 Mi: 2.6 GB of query scratch)
@@ -1169,7 +1120,7 @@ int run_query(drb_scene* s, const float* o3, const float* d3, const float* tmax,
             k_occluded<<<qb->occluded_blocks, kTraceThreads, qb->trace_smem, st>>>(sc, scale, q.ray_o[0], q.ray_d[0], occluded + done, q.counters,
                                                                                   g_refill, g_leaf_batch, g_step_min);
         } else {
-            launch_trace(s, qb->trace_blocks, qb->trace_smem, st, sc, scale, q, 0, nullptr);
+            launch_trace(s, qb->trace_blocks, qb->trace_smem, st, sc, scale, q, 0);
             k_store_query<<<grid, 256, 0, st>>>(s->prims.get(), q.ray_o[0], q.ray_d[0], q.hit, s->orig_id.get(), m, ids + done, t ? t + done : nullptr,
                                                 uv ? uv + 2 * done : nullptr);
         }
@@ -1271,29 +1222,15 @@ int render_core(drb_scene* s, const drb_settings* st, const drb_opts* opts, int 
         int cur = 0;
         uint32_t live = nslots;
         for (int b = 0; b < st->max_depth; ++b) {
-            const uint32_t* order = nullptr;
             // The queue size ends the batch early and sizes the shade grid.  Reading it back drains the stream, so it is read
-            // every fourth bounce only (queues never grow from one bounce to the next: the last value read is an upper bound);
-            // the opt-in reordering needs it every bounce.
-            if (b > 0 && (g_sort_min > 0 || (b & 3) == 0)) {
+            // every fourth bounce only (queues never grow from one bounce to the next: the last value read is an upper bound).
+            if (b > 0 && (b & 3) == 0) {
                 DRB_CUDA(cudaMemcpyAsync(&live, q.counters + cur, sizeof live, cudaMemcpyDeviceToHost, stream));
                 DRB_CUDA(cudaStreamSynchronize(stream));
                 if (live == 0) break;
-                if (g_sort_min > 0 && (long)live >= g_sort_min) {
-                    const float3 lo = make_float3(s->info.bounds_min[0], s->info.bounds_min[1], s->info.bounds_min[2]);
-                    auto inv = [&](int a) { const float e = s->info.bounds_max[a] - s->info.bounds_min[a]; return e > 0.f ? 1.0f / e : 0.f; };
-                    k_ray_keys<<<(live + 255) / 256, 256, 0, stream>>>(q.ray_o[cur], q.ray_d[cur], live, lo, make_float3(inv(0), inv(1), inv(2)),
-                                                                       rb->sort_keys[0].get(), rb->sort_vals[0].get());
-                    size_t tb = rb->sort_tmp_bytes;
-                    DRB_CUDA(cub::DeviceRadixSort::SortPairs(rb->sort_tmp.get(), tb, rb->sort_keys[0].get(), rb->sort_keys[1].get(), rb->sort_vals[0].get(),
-                                                             rb->sort_vals[1].get(),
-                                                             (int)live, 0, 24, stream));
-                    order = rb->sort_vals[1].get();
-                    launches += 4;
-                }
             }
             if (stats) { auto e0 = pool.get(), e1 = pool.get(); trace_ev.push_back({ e0, e1 }); DRB_CUDA(cudaEventRecord(e0, stream)); }
-            launch_trace(s, rb->trace_blocks, rb->trace_smem, stream, sc, fp.scene_scale, q, cur, order);
+            launch_trace(s, rb->trace_blocks, rb->trace_smem, stream, sc, fp.scene_scale, q, cur);
             if (stats) DRB_CUDA(cudaEventRecord(trace_ev.back().second, stream));
             k_shade<<<std::min<uint32_t>((uint32_t)rb->shade_blocks, (live + 4u * kShadeRays - 1u) / (4u * kShadeRays)), 128, 0, stream>>>(
                 sc, fp, q.ray_o[cur], q.ray_d[cur], q.thr[cur], q.hit, q.ray_o[cur ^ 1], q.ray_d[cur ^ 1], q.thr[cur ^ 1], q.contrib, q.counters, cur,
